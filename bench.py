@@ -6,6 +6,7 @@ batches (BASELINE.json configs[1]), one process per GPU.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps K --warmup W      # the reference algorithm on the host CPU cores
+    python bench.py --steps K --warmup W --dump-outputs bench_outputs   # also write the last timed step's outputs (.npy)
 
 One "step" = forward (vision x2, text x2, fusion over 4B pairs, VQ-KD tokenizer, heads) + backward + gradient
 all-reduce + clip + AdamW on B pairs per GPU.  `value` is timed with the batches already resident in HBM; `e2e` repeats
@@ -32,6 +33,10 @@ GFLOP_PER_PAIR = 445.3
 FUSION_GFLOP_PER_PAIR = 4 * 12 * 3.46
 METRIC = "image-text pairs/sec/step"
 UNIT = "pairs/s"
+# 33 steps of the default workload (B = 96) take ~2.1 s on a B200 at 62-64 ms / step
+WARMUP_MIN_STEPS = 33
+# --dump-outputs: size of the fixed, seeded sample of the fp32 master weights written after the dumped step (16 MB)
+DUMP_PARAM_SAMPLES = 1 << 22
 
 
 def peaks():
@@ -137,6 +142,18 @@ def make_host_batch(B, L, M, vocab, res, seed):
         ids_masked[b, pos] = vocab - 1
     out = dict(image=image, text_ids=ids, text_atts=atts, text_ids_masked=ids_masked, masked_pos=masked_pos, masked_ids=masked_ids)
     return {k: v.pin_memory() for k, v in out.items()}
+
+
+LOSS_NAMES = ("loss_itc", "loss_itm", "loss_mlm", "loss_mim")
+
+
+def step_outputs(loss, losses, norm, master):
+    """What one training step hands its caller, as host float32 arrays: the loss, its four terms, the clipped gradient norm
+    and the updated weights (a fixed, seeded sample of the flat fp32 master buffer)."""
+    g = torch.Generator().manual_seed(0)
+    idx = torch.randint(0, master.numel(), (min(DUMP_PARAM_SAMPLES, master.numel()),), generator=g).sort().values
+    out = dict(loss=loss, **losses, grad_norm=norm, params_sample=master[idx.to(master.device)])
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
 
 
 def _eager_legs(dev, B, steps, out):
@@ -255,8 +272,8 @@ def run_ours(args):
                       masked_ids=b["masked_ids"], ret_mim_loss=True, data_source="image")
         loss = out["loss_itc"] + out["loss_itm"] + out["loss_mlm"] + out["loss_mim"]
         acc.backward_step(loss, opt)
-        acc.optimizer_step(opt, wrapped)
-        return loss.detach(), out
+        norm = acc.optimizer_step(opt, wrapped)
+        return loss.detach(), out, norm
 
     def barrier():
         torch.cuda.synchronize()
@@ -265,28 +282,19 @@ def run_ours(args):
             torch.cuda.synchronize()
 
     resident = [to_dev(hb) for hb in host]
-    t_warm = time.perf_counter()
     i = 0
-    # W warm-up steps, and at least ~2 s of them: a GPU coming out of idle needs about a second under load before its
-    # clocks and power state settle (first-loop timings varied by 15 % with 3 warm-up steps of 85 ms)
-    # The number of steps must be the SAME on every rank (each step contains collectives): the first W steps are timed
-    # locally, the number of extra steps is agreed with a MAX all-reduce.
-    n_warm = args.warmup
+    # W warm-up steps, and at least WARMUP_MIN_STEPS: a GPU coming out of idle needs about a second under load before its
+    # clocks and power state settle (first-loop timings varied by 15 % with 3 warm-up steps of 85 ms).  A fixed count, not
+    # a time budget: every warm-up step updates the weights, so a count that followed the clock would make what the timed
+    # steps compute depend on how fast the build is.
+    n_warm = max(args.warmup, WARMUP_MIN_STEPS)
     while i < n_warm:
-        loss, out = step(resident[i % n_pool])
+        loss, out, _ = step(resident[i % n_pool])
         if i == 0:
             arena = reserve_arena(factor=1.5)  # no cudaMalloc inside the timed regions (see accelerator.reserve_arena)
-            t_warm = time.perf_counter()       # the 2 s start after the one-off initialisation of the first step
         if i % 4 == 3:
             torch.cuda.synchronize()
         i += 1
-        if i == args.warmup:
-            torch.cuda.synchronize()
-            per = max((time.perf_counter() - t_warm) / max(args.warmup - 1, 1), 1e-3)
-            extra = torch.tensor([min(40, max(0, int((2.0 - (time.perf_counter() - t_warm)) / per) + 1))], device=dev)
-            if world > 1:
-                dist.all_reduce(extra, op=dist.ReduceOp.MAX)
-            n_warm = args.warmup + int(extra)
     warm_steps = i
     barrier()
     clocks = ClockSampler(local) if rank == 0 else None
@@ -327,7 +335,7 @@ def run_ours(args):
     last = {}
 
     def resident_step(i):
-        last["loss"], last["out"] = step(resident[i % n_pool])
+        last["loss"], last["out"], last["norm"] = step(resident[i % n_pool])
 
     # End-to-end loop: every step's inputs come from pinned host memory and its loss is read back.  The copy of step i+1 is
     # issued on a side stream while step i computes (what a prefetching loader does); both copies and the read-back are
@@ -353,12 +361,15 @@ def run_ours(args):
         s = i & 1
         torch.cuda.current_stream().wait_event(ready[s])
         stage(i + 1)
-        loss, _ = step(slots[s])
+        loss, _, _ = step(slots[s])
         consumed[s].record(torch.cuda.current_stream())
         last["host_loss"] = float(loss.detach())  # D2H read of the step's result
 
     pairs_all = B * world
     ms_step, launches = timed(resident_step, "resident")
+    dumped = None
+    if args.dump_outputs and not args.graph:
+        dumped = step_outputs(last["loss"], {k: last["out"][k] for k in LOSS_NAMES}, last["norm"], model.flat.P)
     ms_e2e, _ = timed(e2e_step, "e2e")
     graph_info = None
     if args.graph:   # the same step replayed as ONE CUDA graph (xfm_b200/graph.py)
@@ -367,11 +378,13 @@ def run_ours(args):
         def loss_fn(m, b):
             out = m(b["image"], b["text_ids"], b["text_atts"], text_ids_masked=b["text_ids_masked"], masked_pos=b["masked_pos"],
                     masked_ids=b["masked_ids"], ret_mim_loss=True, data_source="image")
-            return out["loss_itc"] + out["loss_itm"] + out["loss_mlm"] + out["loss_mim"]
+            return (out["loss_itc"] + out["loss_itm"] + out["loss_mlm"] + out["loss_mim"],) + tuple(out[k] for k in LOSS_NAMES)
         gs = GraphedStep(wrapped, opt, acc, loss_fn, resident[0], warmup=3, uses_mim_masks=True)
         for i in range(3):
             gs(resident[i % n_pool])
         ms_g, _ = timed(lambda i: gs(resident[i % n_pool]), "graph_resident")
+        if args.dump_outputs:   # gs.outputs = (loss, its four terms, gradient norm), overwritten by the next replay
+            dumped = step_outputs(gs.outputs[0], dict(zip(LOSS_NAMES, gs.outputs[1:5])), gs.outputs[5], model.flat.P)
 
         g_staged = {"next": None}
 
@@ -489,6 +502,10 @@ def run_ours(args):
     if rank == 0:
         if world == 1 and not args.no_cpu:
             line["cpu_baseline"] = cpu_baseline(args, quick=True)
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for k, v in dumped.items():
+                np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
         print(json.dumps(line), file=out_stream, flush=True)
     if world > 1:
         # leave without running destructors: tearing down a process group while captured graphs / side streams still
@@ -741,7 +758,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-eager", action="store_true", help="skip the gpu_eager_baseline leg (eager PyTorch on the same GPU)")
     ap.add_argument("--overlap", default="auto", help="accelerator OVERLAP_ALLREDUCE: auto | true | false")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="pretrain config: write what the last step of the headline timed loop returned (loss, its four "
+                         "terms, gradient norm, a seeded sample of the updated fp32 weights) as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "pretrain"):
+        ap.error("--dump-outputs is implemented for the pre-training step (--impl ours --config pretrain)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.overlap = {"true": True, "false": False}.get(str(args.overlap).lower(), "auto")
     args.batch_given = args.batch is not None

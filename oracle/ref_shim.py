@@ -1,9 +1,9 @@
-"""Import the UNMODIFIED reference (/root/reference) in this container.  TEST INFRASTRUCTURE ONLY.
+"""Import the UNMODIFIED reference (the XFM checkout named by XFM_REFERENCE_ROOT).  TEST INFRASTRUCTURE ONLY.
 
 The reference pins transformers==4.12.5 / timm==0.4.12; this image has transformers 5.x and no timm.
 The shim (SURVEY.md Appendix A) provides the handful of helpers the reference imports from those
-packages; no reference source is copied or edited.  Only `tools/make_golden.py` (run in the build
-container, where /root/reference exists) uses this module; nothing on the GPU box may import it.
+packages; no reference source is copied or edited.  Only `tools/make_golden.py` and tests/ref_probe.py use
+this module, and only where XFM_REFERENCE_ROOT names a checkout of the reference; the package never imports it.
 """
 import importlib.machinery
 import json
@@ -16,7 +16,7 @@ import types
 import torch
 import torch.nn as nn
 
-REF_ROOT = os.environ.get("XFM_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("XFM_REFERENCE_ROOT", "")
 
 
 def _mod(name, **attrs):

@@ -1,5 +1,5 @@
-"""Helper for tests/test_feed_cpu.py — run as a SUBPROCESS (it registers import stubs), only where the reference tree exists
-(the build container; never on the GPU box).  Differential check on fresh random cases, beyond the committed fixture: the
+"""Helper for tests/test_feed_cpu.py — run as a SUBPROCESS (it registers import stubs), only where XFM_REFERENCE_ROOT names a
+checkout of the original XFM sources.  Differential check on fresh random cases, beyond the committed fixture: the
 reference's TextMaskingGenerator / preprocess / get_image_attns / RandomAugment sampling and xfm_b200.feed, same seeds.
 Prints one JSON object."""
 import contextlib

@@ -1,5 +1,5 @@
-"""Helper for tests/test_boundary_cpu.py — run as a SUBPROCESS (it rebinds `models` in sys.modules), only where the
-reference tree exists (/root/reference, i.e. the build container; never on the GPU box).  Prints one JSON object.
+"""Helper for tests/test_boundary_cpu.py — run as a SUBPROCESS (it rebinds `models` in sys.modules), only where
+XFM_REFERENCE_ROOT names a checkout of the original XFM sources.  Prints one JSON object.
 
     python tests/ref_probe.py loaders    constructor-time checkpoint import: reference XFM(load_*_params=True) vs xfm_b200
     python tests/ref_probe.py subclass   the reference's OWN models/model_pretrain.py, model_retrieval.py and model_nlvr.py
@@ -16,7 +16,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = os.environ.get("XFM_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("XFM_REFERENCE_ROOT", "")
 
 from oracle import ref_shim  # noqa: E402
 from oracle import xfm_oracle as O  # noqa: E402

@@ -5,8 +5,8 @@
     unchanged: the Pretrain.py:413-417 construction sequence, forward_multimodal's call pattern, temp.clamp_, the
     optimizer / accelerator set-up;
   * relative-position table resampling (models/beit2.py:611-652) properties.
-The two reference-dependent checks run tests/ref_probe.py in a subprocess and are skipped where /root/reference is absent
-(the GPU box)."""
+The two reference-dependent checks run tests/ref_probe.py in a subprocess and are skipped unless XFM_REFERENCE_ROOT names a
+checkout of the original XFM sources."""
 import json
 import os
 import subprocess
@@ -16,8 +16,9 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+REF = os.environ.get("XFM_REFERENCE_ROOT", "")
+needs_ref = pytest.mark.skipif(not os.path.isdir(REF),
+                               reason="XFM_REFERENCE_ROOT does not name a checkout of the original XFM sources")
 
 
 def _probe(mode):

@@ -412,7 +412,8 @@ def test_randaugment_sampling_and_table_operations_match_reference(golden):
         feed.channel_table(img[:, :, 0], "Rotate")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present")
+@pytest.mark.skipif(not os.path.isdir(os.environ.get("XFM_REFERENCE_ROOT", "")),
+                    reason="XFM_REFERENCE_ROOT does not name a checkout of the original XFM sources")
 def test_live_differential_against_the_reference_loader_code():
     """Beyond the committed fixture: tests/feed_probe.py imports the reference's dataset package in a subprocess and compares
     it with xfm_b200.feed on fresh random configurations and seeds (600 masker / preprocess cases over random mask

@@ -2,7 +2,7 @@
   * the oracle restatement of transformers-4.12.5 AdamW + clip_grad_norm_ (oracle/optim_oracle.py) against torch's own Adam /
     clip_grad_norm_;
   * FlatAdamW's parameter-group membership for every parameter of the XFM layout against optim.py's rules — through the
-    reference's own create_optimizer when /root/reference is present, else the restated rule;
+    reference's own create_optimizer where XFM_REFERENCE_ROOT names a checkout of it, else the restated rule;
   * FlatAdamW is a torch.optim.Optimizer: scheduler.py's LambdaLR drives its param_groups and the values reach the
     hyper-parameter block the kernel reads."""
 import importlib.util
@@ -15,7 +15,7 @@ import torch
 from oracle import optim_oracle as OO
 from oracle import xfm_oracle as O
 
-REF = "/root/reference"
+REF = os.environ.get("XFM_REFERENCE_ROOT", "")
 
 
 def test_oracle_adamw_against_torch_adam_and_clip():
@@ -85,7 +85,7 @@ def test_group_membership_matches_optim_py_rules():
     assert not any(n.startswith("vqkd.") for n in have)  # frozen tokenizer
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="XFM_REFERENCE_ROOT does not name a checkout of the original XFM sources")
 def test_group_membership_through_the_reference_create_optimizer(monkeypatch):
     """optim.py:4-50 itself, with transformers.optimization.AdamW (removed in transformers 5) replaced by a recorder."""
     import types

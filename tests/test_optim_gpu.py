@@ -164,6 +164,11 @@ def test_nlvr_heads_are_updated_by_the_flat_optimizer():
             super().__init__(config, **kw)
             self.cls_head = build_mlp(input_dim=self.text_width * 2, output_dim=2)
             self.init_params = ["cls_head." + n for n, _ in self.cls_head.named_parameters()]
+            # nn.Linear's default init draws from the global RNG, whose state depends on the tests that ran before this
+            # one; the name-keyed values of the mirror's head make the three steps the same wherever the test runs
+            with torch.no_grad():
+                for n, p in self.cls_head.named_parameters():
+                    p.copy_(O.make_tensor("cls_head." + n, tuple(p.shape), 0))
         forward = XFMForNLVR.forward
 
     cfg = O.tiny_config()

@@ -1,9 +1,10 @@
-"""Generate tests/golden/feed.json by running the UNMODIFIED reference loader code (/root/reference/dataset/pretrain_dataset.py:
-TextMaskingGenerator, ImageTextJsonDataset.preprocess / collate_fn, TextJsonDataset.preprocess, RegionTextJsonDataset.__iter__ /
-get_image_attns / collate_fn) on seeded inputs with the stub tokenizer of tests/feed_stub.py.  Runs in the build container only
-(the reference tree is not on the GPU box); the fixture it writes is what tests/test_feed_cpu.py checks xfm_b200.feed against.
+"""Generate tests/golden/feed.json by running the UNMODIFIED reference loader code (dataset/pretrain_dataset.py of the original
+XFM sources: TextMaskingGenerator, ImageTextJsonDataset.preprocess / collate_fn, TextJsonDataset.preprocess,
+RegionTextJsonDataset.__iter__ / get_image_attns / collate_fn) on seeded inputs with the stub tokenizer of tests/feed_stub.py.
+Needs a checkout of those sources, named by XFM_REFERENCE_ROOT; the fixture it writes is what tests/test_feed_cpu.py checks
+xfm_b200.feed against.
 
-    python tools/make_golden_feed.py
+    XFM_REFERENCE_ROOT=<XFM checkout> python tools/make_golden_feed.py
 """
 import base64
 import contextlib
@@ -18,7 +19,7 @@ import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-REF_ROOT = "/root/reference"
+REF_ROOT = os.environ.get("XFM_REFERENCE_ROOT", "")
 ABSENT = {"pycocotools", "pycocoevalcap", "skimage", "matplotlib", "ruamel", "h5py", "cv2", "ftfy", "timm"}
 
 
