@@ -76,7 +76,9 @@ typedef struct xfm_gemm_params {
   int32_t M, N, K;
   int32_t a_mn_major, b_mn_major;
   int32_t c_dtype;    /* 0 = bf16, 1 = f32 */
-  int32_t split_k;    /* >= 1; > 1 requires c_dtype == 1 and accumulate == 1 (atomic f32 adds) */
+  int32_t split_k;    /* >= 1; > 1 requires c_dtype == 1 and accumulate == 1 (atomic f32 adds), and no bias, residual,
+                         aux_out or act: every K slice applies the epilogue to its partial sum, so only col_scale,
+                         row_group_scale and dropout (linear, same factor in every slice) may be combined with it */
   int32_t accumulate; /* 0: C = v, 1: C += v (f32 only) */
   int32_t act;        /* 0 none, 1 gelu, 2 dgelu(aux_in), 3 tanh */
   int32_t res_dtype;  /* 0 = bf16, 1 = f32 */

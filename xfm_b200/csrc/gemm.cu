@@ -1153,6 +1153,13 @@ int gemm_bf16(const xfm_gemm_params* p, cudaStream_t stream) {
     set_error("gemm: split_k > 1 needs accumulate = 1 (caller zeroes or owns C)");
     return XFM_ERR_BAD_ARG;
   }
+  // Every K slice runs the whole epilogue on its partial sum.  Only the steps linear in the accumulator with the same
+  // factor in every slice (col_scale, row_group_scale, dropout) distribute over the slices; bias, residual, aux_out and
+  // the activations would be applied once per slice.
+  if (split_k > 1 && (p->bias || p->residual || p->aux_out || p->act != 0)) {
+    set_error("gemm: split_k > 1 allows no bias, residual, aux_out or act (each K slice applies the epilogue)");
+    return XFM_ERR_BAD_ARG;
+  }
   if (p->act == 2 && !p->aux_in) {
     set_error("gemm: act=2 (dgelu) needs aux_in");
     return XFM_ERR_BAD_ARG;

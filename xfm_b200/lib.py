@@ -112,6 +112,8 @@ def gemm(a, b, *, a_t=False, b_t=False, out=None, out_dtype=torch.bfloat16, bias
 
     a: bf16 [M,K] (or [K,M] with a_t=True: the stored tensor is the transpose, "MN-major").
     b: bf16 [N,K] (or [K,N] with b_t=True).
+    split_k > 1 needs an f32 `out` with accumulate=True and rejects bias, residual, aux_out and act != 0: every K slice
+    applies the epilogue to its partial sum, so only col_scale, row_group_scale and dropout may be combined with it.
     """
     assert a.dtype == torch.bfloat16 and b.dtype == torch.bfloat16
     assert a.dim() == 2 and b.dim() == 2 and a.stride(1) == 1 and b.stride(1) == 1
