@@ -133,9 +133,9 @@ typedef struct xfm_attn_params {
   const float* rel_table;
   int32_t rel_window;
   int32_t allow_tc;
-  /* Forward scratch for samples processed in blocks of 192 keys (Lq = Lk = 577, 384 px): bf16 [3, B*Lq, H*64] block-normalised
-   * partial outputs and f32 [3, B, H, Lq] block lse, merged into out / lse by a last kernel.  Without them the 577-token
-   * forward runs on the mma.sync kernel. */
+  /* Forward scratch for rows processed in key blocks (577 keys at 384 px: 3 blocks; 901 at 480 px: 5): bf16 [nb, B*Lq, H*64]
+   * block-normalised partial outputs and f32 [nb, B, H, Lq] block lse, merged into out / lse by a last kernel, with nb from
+   * xfm_attention_fwd_parts.  Without them these forwards run on the mma.sync kernel. */
   void* part_out;
   float* part_lse;
   float* rel_dtable; /* backward: gradient of rel_table, accumulated (+=) by the tcgen05 dQ kernel; when null or when the
@@ -144,6 +144,9 @@ typedef struct xfm_attn_params {
 
 int xfm_attention_fwd(const xfm_attn_params* p, void* stream);
 int xfm_attention_bwd(const xfm_attn_params* p, void* stream);
+/* Number of key blocks nb whose partial results the forward of *p would write to part_out / part_lse if they were given
+ * (0: the path xfm_attention_fwd chooses needs no scratch).  Host-only, needs no device; part_out / part_lse are ignored. */
+int xfm_attention_fwd_parts(const xfm_attn_params* p);
 
 /* ------------------------------------------------------------------------------------------------
  * K6 — LayerNorm (torch layer_norm at beit2.py:201-205,458; xroberta.py:135,303,384,1328; xfm.py:118).

@@ -91,6 +91,7 @@ const char* xfm_last_error(void) { return g_err; }
 int xfm_gemm_bf16(const xfm_gemm_params* p, void* stream) { return gemm_bf16(p, ST); }
 int xfm_attention_fwd(const xfm_attn_params* p, void* stream) { return attention_fwd(p, ST); }
 int xfm_attention_bwd(const xfm_attn_params* p, void* stream) { return attention_bwd(p, ST); }
+int xfm_attention_fwd_parts(const xfm_attn_params* p) { return attention_fwd_parts(p); }
 
 int xfm_layernorm_fwd(const void* x, int x_dtype, const float* w, const float* b, void* y, int y_dtype, float* y2_f32,
                       float* stats, int M, int D, float eps, void* stream) {

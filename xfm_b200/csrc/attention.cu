@@ -213,24 +213,33 @@ XFM_DEVINL float logit2(const AttnArgs& a, float raw, float addend, int key) {
 // ================================================================================================ forward
 // WARPS x 16 query rows per CTA (4 or 8 warps): K / V of the whole sample are shared-memory resident, so at N = 577 (164 KB)
 // only one CTA fits an SM and the warp count per CTA is the SM's occupancy.
-template <int WARPS>
+// STREAM (rows whose K / V do not fit shared memory, e.g. 901 keys at 480 px): K / V pass through shared memory in chunks of
+// KV_CHUNK keys.  The 64-key blocks, and therefore every operation and its order, are the resident kernel's.
+constexpr int KV_CHUNK = 128;
+template <int WARPS, bool STREAM>
 __global__ void __launch_bounds__(WARPS * 32)
 attn_fwd_kernel(const AttnArgs a) {
   constexpr int RT = WARPS * 16;
   extern __shared__ __align__(128) uint8_t smem[];
   const int LkP = (a.Lk + AT_TILE - 1) / AT_TILE * AT_TILE;
+  const int KR = STREAM ? KV_CHUNK : LkP;   // key rows held in shared memory
   uint8_t* sQ = smem;
   uint8_t* sK = sQ + RT * ROW_BYTES;
-  uint8_t* sV = sK + LkP * ROW_BYTES;
+  uint8_t* sV = sK + KR * ROW_BYTES;
   const int q0 = blockIdx.x * RT, h = blockIdx.y, b = blockIdx.z;
   const int kvb = a.kv_index ? a.kv_index[b] : b;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const bf16* kg = a.k + (int64_t)kvb * a.Lk * a.k_stride + h * HD;
+  const bf16* vg = a.v + (int64_t)kvb * a.Lk * a.v_stride + h * HD;
   load_tile(sQ, a.q + ((int64_t)b * a.Lq + q0) * a.q_stride + h * HD, a.q_stride, min(RT, a.Lq - q0), RT);
-  load_tile(sK, a.k + (int64_t)kvb * a.Lk * a.k_stride + h * HD, a.k_stride, a.Lk, LkP);
-  load_tile(sV, a.v + (int64_t)kvb * a.Lk * a.v_stride + h * HD, a.v_stride, a.Lk, LkP);
+  if (!STREAM) {
+    load_tile(sK, kg, a.k_stride, a.Lk, LkP);
+    load_tile(sV, vg, a.v_stride, a.Lk, LkP);
+  }
   cp_async_wait_all();
   __syncthreads();
-  if (q0 + warp * 16 >= a.Lq) return;  // warp-uniform; no later block-wide barrier
+  const bool live = q0 + warp * 16 < a.Lq;   // warp-uniform
+  if (!STREAM && !live) return;              // no later block-wide barrier
   const uint32_t aQ = smem_u32(sQ), aK = smem_u32(sK), aV = smem_u32(sV);
   uint32_t qf[4][4];
   load_a_frags(aQ, warp * 16, lane, qf);
@@ -243,14 +252,23 @@ attn_fwd_kernel(const AttnArgs a) {
   const float inv_keep = a.dropout_p > 0.f ? 1.0f / (1.0f - a.dropout_p) : 1.0f;
   const uint32_t seed_mix = drop_seed_mix(a.seed + *a.salt), thr = drop_threshold(a.dropout_p);
   const uint64_t dp0 = drop_row_pair_base(a, b, h, r0), dp1 = drop_row_pair_base(a, b, h, r1);
-  for (int kb = 0; kb < LkP; kb += AT_TILE) {
+  for (int chunk0 = 0; chunk0 < LkP; chunk0 += KR) {
+  if (STREAM) {   // the whole CTA: the previous chunk is consumed, then the next one lands
+    __syncthreads();
+    load_tile(sK, kg + (int64_t)chunk0 * a.k_stride, a.k_stride, min(KR, a.Lk - chunk0), KR);
+    load_tile(sV, vg + (int64_t)chunk0 * a.v_stride, a.v_stride, min(KR, a.Lk - chunk0), KR);
+    cp_async_wait_all();
+    __syncthreads();
+    if (!live) continue;
+  }
+  for (int kb = chunk0; kb < min(chunk0 + KR, LkP); kb += AT_TILE) {
     float s[8][4];
 #pragma unroll
     for (int i = 0; i < 8; ++i) s[i][0] = s[i][1] = s[i][2] = s[i][3] = 0.f;
     float bb[8][4];
     load_addend_rows(a, b, h, r0, r1, kb, t, bb);
     const int lim = a.Lk - kb;   // valid keys in this block
-    mma_rows_nt(s, qf, aK, kb, lane, lim);
+    mma_rows_nt(s, qf, aK, kb - chunk0, lane, lim);
     float mx0 = -INFINITY, mx1 = -INFINITY;
 #pragma unroll
     for (int nt = 0; nt < 8; ++nt) {
@@ -295,8 +313,10 @@ attn_fwd_kernel(const AttnArgs a) {
     }
     uint32_t pf[4][4];
     c_to_a_frags(s, pf);
-    mma_rows_kd(o, pf, aV, kb, lane, lim);
+    mma_rows_kd(o, pf, aV, kb - chunk0, lane, lim);
   }
+  }
+  if (!live) return;
   l0 = quad_sum(l0);
   l1 = quad_sum(l1);
   const float i0 = 1.0f / l0, i1 = 1.0f / l1;
@@ -339,28 +359,34 @@ __global__ void attn_delta_kernel(const bf16* __restrict__ dout, int64_t do_stri
   }
 }
 
-// Kernel A: dQ (+ optional bf16 dS dump).  Same tiling as the forward.
-template <int WARPS>
+// Kernel A: dQ (+ optional bf16 dS dump).  Same tiling as the forward; STREAM: K / V in chunks, as there.
+template <int WARPS, bool STREAM>
 __global__ void __launch_bounds__(WARPS * 32)
 attn_bwd_dq_kernel(const AttnArgs a) {
   constexpr int RT = WARPS * 16;
   extern __shared__ __align__(128) uint8_t smem[];
   const int LkP = (a.Lk + AT_TILE - 1) / AT_TILE * AT_TILE;
+  const int KR = STREAM ? KV_CHUNK : LkP;
   uint8_t* sQ = smem;
   uint8_t* sdO = sQ + RT * ROW_BYTES;
   uint8_t* sK = sdO + RT * ROW_BYTES;
-  uint8_t* sV = sK + LkP * ROW_BYTES;
+  uint8_t* sV = sK + KR * ROW_BYTES;
   const int q0 = blockIdx.x * RT, h = blockIdx.y, b = blockIdx.z;
   const int kvb = a.kv_index ? a.kv_index[b] : b;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nq = min(RT, a.Lq - q0);
+  const bf16* kg = a.k + (int64_t)kvb * a.Lk * a.k_stride + h * HD;
+  const bf16* vg = a.v + (int64_t)kvb * a.Lk * a.v_stride + h * HD;
   load_tile(sQ, a.q + ((int64_t)b * a.Lq + q0) * a.q_stride + h * HD, a.q_stride, nq, RT);
   load_tile(sdO, a.dout + ((int64_t)b * a.Lq + q0) * a.do_stride + h * HD, a.do_stride, nq, RT);
-  load_tile(sK, a.k + (int64_t)kvb * a.Lk * a.k_stride + h * HD, a.k_stride, a.Lk, LkP);
-  load_tile(sV, a.v + (int64_t)kvb * a.Lk * a.v_stride + h * HD, a.v_stride, a.Lk, LkP);
+  if (!STREAM) {
+    load_tile(sK, kg, a.k_stride, a.Lk, LkP);
+    load_tile(sV, vg, a.v_stride, a.Lk, LkP);
+  }
   cp_async_wait_all();
   __syncthreads();
-  if (q0 + warp * 16 >= a.Lq) return;
+  const bool live = q0 + warp * 16 < a.Lq;
+  if (!STREAM && !live) return;
   const uint32_t aQ = smem_u32(sQ), adO = smem_u32(sdO), aK = smem_u32(sK), aV = smem_u32(sV);
   uint32_t qf[4][4], dof[4][4];
   load_a_frags(aQ, warp * 16, lane, qf);
@@ -376,7 +402,16 @@ attn_bwd_dq_kernel(const AttnArgs a) {
   float dq[8][4];
 #pragma unroll
   for (int i = 0; i < 8; ++i) dq[i][0] = dq[i][1] = dq[i][2] = dq[i][3] = 0.f;
-  for (int kb = 0; kb < LkP; kb += AT_TILE) {
+  for (int chunk0 = 0; chunk0 < LkP; chunk0 += KR) {
+  if (STREAM) {
+    __syncthreads();
+    load_tile(sK, kg + (int64_t)chunk0 * a.k_stride, a.k_stride, min(KR, a.Lk - chunk0), KR);
+    load_tile(sV, vg + (int64_t)chunk0 * a.v_stride, a.v_stride, min(KR, a.Lk - chunk0), KR);
+    cp_async_wait_all();
+    __syncthreads();
+    if (!live) continue;
+  }
+  for (int kb = chunk0; kb < min(chunk0 + KR, LkP); kb += AT_TILE) {
     float s[8][4], dp[8][4];
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -386,8 +421,8 @@ attn_bwd_dq_kernel(const AttnArgs a) {
     float bb[8][4];
     load_addend_rows(a, b, h, r0, r1, kb, t, bb);
     const int lim = a.Lk - kb;
-    mma_rows_nt(s, qf, aK, kb, lane, lim);    // S  = Q K^T
-    mma_rows_nt(dp, dof, aV, kb, lane, lim);  // dP = dO V^T
+    mma_rows_nt(s, qf, aK, kb - chunk0, lane, lim);    // S  = Q K^T
+    mma_rows_nt(dp, dof, aV, kb - chunk0, lane, lim);  // dP = dO V^T
 #pragma unroll
     for (int nt = 0; nt < 8; ++nt) {
       if (nt * 8 >= lim) continue;   // all-padding key group: dS stays 0 (ds_dump beyond Lk is pre-zeroed by the caller)
@@ -417,8 +452,10 @@ attn_bwd_dq_kernel(const AttnArgs a) {
     }
     uint32_t dsf[4][4];
     c_to_a_frags(s, dsf);
-    mma_rows_kd(dq, dsf, aK, kb, lane, lim);  // dQ += dS K
+    mma_rows_kd(dq, dsf, aK, kb - chunk0, lane, lim);  // dQ += dS K
   }
+  }
+  if (!live) return;
 #pragma unroll
   for (int nt = 0; nt < 8; ++nt) {
     const int col = h * HD + nt * 8 + 2 * t;
@@ -431,18 +468,20 @@ attn_bwd_dq_kernel(const AttnArgs a) {
 
 // Kernel B: dK, dV for one 64-key tile of one (K/V batch row, head); loops over every referencing sample and over
 // that sample's queries in blocks of 64.  Works on the transposed problem: rows = keys, columns = queries.
-template <int WARPS>
+// STREAM: a sample's Q / dO (and lse / delta) pass through shared memory in chunks of KV_CHUNK queries.
+template <int WARPS, bool STREAM>
 __global__ void __launch_bounds__(WARPS * 32)
 attn_bwd_dkv_kernel(const AttnArgs a) {
   constexpr int RT = WARPS * 16;
   extern __shared__ __align__(128) uint8_t smem[];
   const int LqP = (a.Lq + AT_TILE - 1) / AT_TILE * AT_TILE;
+  const int QR = STREAM ? KV_CHUNK : LqP;   // query rows held in shared memory
   uint8_t* sK = smem;
   uint8_t* sV = sK + RT * ROW_BYTES;
   uint8_t* sQ = sV + RT * ROW_BYTES;
-  uint8_t* sdO = sQ + LqP * ROW_BYTES;
-  float* sLse = (float*)(sdO + LqP * ROW_BYTES);
-  float* sDelta = sLse + LqP;
+  uint8_t* sdO = sQ + QR * ROW_BYTES;
+  float* sLse = (float*)(sdO + QR * ROW_BYTES);
+  float* sDelta = sLse + QR;
   const int k0 = blockIdx.x * RT, h = blockIdx.y, kvb = blockIdx.z;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nk = min(RT, a.Lk - k0);
@@ -460,26 +499,30 @@ attn_bwd_dkv_kernel(const AttnArgs a) {
     dv[i][0] = dv[i][1] = dv[i][2] = dv[i][3] = 0.f;
   }
   uint32_t kf[4][4], vf[4][4];
+  bool frags = false;
   const int s_begin = a.kv_samples ? a.kv_offsets[kvb] : kvb;
   const int s_end = a.kv_samples ? a.kv_offsets[kvb + 1] : kvb + 1;
   for (int si = s_begin; si < s_end; ++si) {
     const int b = a.kv_samples ? a.kv_samples[si] : si;
-    __syncthreads();  // previous sample's tiles fully consumed (also orders the K/V tile loads on the first pass)
-    load_tile(sQ, a.q + (int64_t)b * a.Lq * a.q_stride + h * HD, a.q_stride, a.Lq, LqP);
-    load_tile(sdO, a.dout + (int64_t)b * a.Lq * a.do_stride + h * HD, a.do_stride, a.Lq, LqP);
     const int64_t st = ((int64_t)b * a.H + h) * a.Lq;
-    for (int i = threadIdx.x; i < LqP; i += blockDim.x) {
-      sLse[i] = i < a.Lq ? a.lse[st + i] : 0.f;
-      sDelta[i] = i < a.Lq ? a.delta[st + i] : 0.f;
+    for (int chunk0 = 0; chunk0 < LqP; chunk0 += QR) {
+    const int nq = min(QR, a.Lq - chunk0);
+    __syncthreads();  // previous sample's (chunk's) tiles fully consumed (also orders the K/V tile loads on the first pass)
+    load_tile(sQ, a.q + ((int64_t)b * a.Lq + chunk0) * a.q_stride + h * HD, a.q_stride, nq, QR);
+    load_tile(sdO, a.dout + ((int64_t)b * a.Lq + chunk0) * a.do_stride + h * HD, a.do_stride, nq, QR);
+    for (int i = threadIdx.x; i < QR; i += blockDim.x) {
+      sLse[i] = i < nq ? a.lse[st + chunk0 + i] : 0.f;
+      sDelta[i] = i < nq ? a.delta[st + chunk0 + i] : 0.f;
     }
     cp_async_wait_all();
     __syncthreads();
     if (!warp_active) continue;
-    if (si == s_begin) {
+    if (!frags) {
       load_a_frags(aK, warp * 16, lane, kf);
       load_a_frags(aV, warp * 16, lane, vf);
+      frags = true;
     }
-    for (int qb = 0; qb < LqP; qb += AT_TILE) {
+    for (int qb = chunk0; qb < min(chunk0 + QR, LqP); qb += AT_TILE) {
       float s[8][4], dp[8][4];
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
@@ -489,8 +532,8 @@ attn_bwd_dkv_kernel(const AttnArgs a) {
       float bb[8][4];
       load_addend_cols(a, b, h, key0, key1, qb, t, bb);
       const int lim = a.Lq - qb;   // valid queries in this block
-      mma_rows_nt(s, kf, aQ, qb, lane, lim);    // S^T  = K Q^T
-      mma_rows_nt(dp, vf, adO, qb, lane, lim);  // dP^T = V dO^T
+      mma_rows_nt(s, kf, aQ, qb - chunk0, lane, lim);    // S^T  = K Q^T
+      mma_rows_nt(dp, vf, adO, qb - chunk0, lane, lim);  // dP^T = V dO^T
       float pd[8][4];
 #pragma unroll
       for (int nt = 0; nt < 8; ++nt) {
@@ -504,18 +547,19 @@ attn_bwd_dkv_kernel(const AttnArgs a) {
           const int key = (e < 2) ? key0 : key1;
           const int qi = qb + nt * 8 + 2 * t + (e & 1);
           float p = 0.f;
-          if (qi < a.Lq && key < a.Lk) p = __expf(s[nt][e] * a.scale + bb[nt][e] - sLse[qi]);
+          if (qi < a.Lq && key < a.Lk) p = __expf(s[nt][e] * a.scale + bb[nt][e] - sLse[qi - chunk0]);
           float keep = 1.f;
           if (a.dropout_p > 0.f) keep = (qi < a.Lq && key < a.Lk && drop_keep(a, b, h, qi, key)) ? inv_keep : 0.f;
           pd[nt][e] = p * keep;
-          s[nt][e] = p * (dp[nt][e] * keep - sDelta[min(qi, LqP - 1)]);
+          s[nt][e] = p * (dp[nt][e] * keep - sDelta[min(qi - chunk0, QR - 1)]);
         }
       }
       uint32_t pf[4][4], dsf[4][4];
       c_to_a_frags(pd, pf);
       c_to_a_frags(s, dsf);
-      mma_rows_kd(dv, pf, adO, qb, lane, lim);  // dV += P^T dO
-      mma_rows_kd(dk, dsf, aQ, qb, lane, lim);  // dK += dS^T Q
+      mma_rows_kd(dv, pf, adO, qb - chunk0, lane, lim);  // dV += P^T dO
+      mma_rows_kd(dk, dsf, aQ, qb - chunk0, lane, lim);  // dK += dS^T Q
+    }
     }
   }
   if (!warp_active) return;
@@ -569,6 +613,30 @@ static void fill_args(const xfm_attn_params* p, AttnArgs& a) {
   a.Bkv = p->Bkv > 0 ? p->Bkv : p->B;
 }
 
+// The resident kernels hold a whole row of K / V (or Q / dO) in shared memory; past this, the streaming variants run.
+constexpr size_t RESIDENT_SMEM_MAX = 220 * 1024;
+
+template <int WARPS, bool STREAM>
+static int launch_attn_fwd(const AttnArgs& a, size_t smem, cudaStream_t s) {
+  cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<WARPS, STREAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  const dim3 grid((a.Lq + WARPS * 16 - 1) / (WARPS * 16), a.H, a.B);
+  attn_fwd_kernel<WARPS, STREAM><<<grid, WARPS * 32, smem, s>>>(a);
+  count_launch();
+  return (int)cudaGetLastError();
+}
+
+int attention_fwd_parts(const xfm_attn_params* p) {
+  if (!p || !p->allow_tc || attn_check(p)) return 0;
+  xfm_attn_params q = *p;   // as if the scratch were given: does the chosen tcgen05 path run in key blocks?
+  static float dummy;
+  q.part_out = &dummy;
+  q.part_lse = &dummy;
+  if (!vit_attention_tc_supported(&q) && !cross_attention_tc_supported(&q)) return 0;
+  const int nb = KeyBlocks::nb(q.Lk);
+  return nb > 1 ? nb : 0;
+}
+
 int attention_fwd(const xfm_attn_params* p, cudaStream_t s) {
   if (attn_check(p)) return XFM_ERR_BAD_ARG;
   if (p->allow_tc && vit_attention_tc_supported(p)) return vit_attention_fwd_tc(p, s);
@@ -580,16 +648,29 @@ int attention_fwd(const xfm_attn_params* p, cudaStream_t s) {
   const bool big = a.Lq > 256;   // 8 warps (128 query rows) per CTA when the resident K / V leave room for one CTA per SM only
   const int rt = big ? 128 : 64;
   const size_t smem = (size_t)(rt + 2 * LkP) * ROW_BYTES;
-  if (smem > 220 * 1024) {
-    set_error("attention: Lk=%d needs %zu bytes of shared memory (max 220 KB; K/V streaming not built yet)", a.Lk, smem);
-    return XFM_ERR_BAD_ARG;
+  if (smem > RESIDENT_SMEM_MAX) {
+    const size_t smem_s = (size_t)(rt + 2 * KV_CHUNK) * ROW_BYTES;
+    return big ? launch_attn_fwd<8, true>(a, smem_s, s) : launch_attn_fwd<4, true>(a, smem_s, s);
   }
-  cudaError_t e = big ? cudaFuncSetAttribute(attn_fwd_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                      : cudaFuncSetAttribute(attn_fwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  return big ? launch_attn_fwd<8, false>(a, smem, s) : launch_attn_fwd<4, false>(a, smem, s);
+}
+
+template <int WARPS, bool STREAM>
+static int launch_attn_bwd_dq(const AttnArgs& a, size_t smem, cudaStream_t s) {
+  cudaError_t e = cudaFuncSetAttribute(attn_bwd_dq_kernel<WARPS, STREAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  const dim3 grid((a.Lq + rt - 1) / rt, a.H, a.B);
-  if (big) attn_fwd_kernel<8><<<grid, 256, smem, s>>>(a);
-  else attn_fwd_kernel<4><<<grid, 128, smem, s>>>(a);
+  const dim3 grid((a.Lq + WARPS * 16 - 1) / (WARPS * 16), a.H, a.B);
+  attn_bwd_dq_kernel<WARPS, STREAM><<<grid, WARPS * 32, smem, s>>>(a);
+  count_launch();
+  return (int)cudaGetLastError();
+}
+
+template <int WARPS, bool STREAM>
+static int launch_attn_bwd_dkv(const AttnArgs& a, size_t smem, cudaStream_t s) {
+  cudaError_t e = cudaFuncSetAttribute(attn_bwd_dkv_kernel<WARPS, STREAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  const dim3 grid((a.Lk + WARPS * 16 - 1) / (WARPS * 16), a.H, a.Bkv);
+  attn_bwd_dkv_kernel<WARPS, STREAM><<<grid, WARPS * 32, smem, s>>>(a);
   count_launch();
   return (int)cudaGetLastError();
 }
@@ -624,24 +705,19 @@ int attention_bwd(const xfm_attn_params* p, cudaStream_t s) {
   const int rq = big_q ? 128 : 64, rk = big_k ? 128 : 64;
   const size_t smem_a = (size_t)(2 * rq + 2 * LkP) * ROW_BYTES;
   const size_t smem_b = (size_t)(2 * rk + 2 * LqP) * ROW_BYTES + 2 * LqP * sizeof(float);
-  if (smem_a > 220 * 1024 || smem_b > 220 * 1024) {
-    set_error("attention_bwd: sequence too long for the shared-memory resident kernels");
-    return XFM_ERR_BAD_ARG;
+  int rc;
+  if (smem_a > RESIDENT_SMEM_MAX) {
+    const size_t sm = (size_t)(2 * rq + 2 * KV_CHUNK) * ROW_BYTES;
+    rc = big_q ? launch_attn_bwd_dq<8, true>(a, sm, s) : launch_attn_bwd_dq<4, true>(a, sm, s);
+  } else {
+    rc = big_q ? launch_attn_bwd_dq<8, false>(a, smem_a, s) : launch_attn_bwd_dq<4, false>(a, smem_a, s);
   }
-  cudaError_t e = big_q ? cudaFuncSetAttribute(attn_bwd_dq_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a)
-                        : cudaFuncSetAttribute(attn_bwd_dq_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a);
-  if (e != cudaSuccess) return (int)e;
-  e = big_k ? cudaFuncSetAttribute(attn_bwd_dkv_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b)
-            : cudaFuncSetAttribute(attn_bwd_dkv_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b);
-  if (e != cudaSuccess) return (int)e;
-  const dim3 ga((a.Lq + rq - 1) / rq, a.H, a.B), gb((a.Lk + rk - 1) / rk, a.H, a.Bkv);
-  if (big_q) attn_bwd_dq_kernel<8><<<ga, 256, smem_a, s>>>(a);
-  else attn_bwd_dq_kernel<4><<<ga, 128, smem_a, s>>>(a);
-  count_launch();
-  if (big_k) attn_bwd_dkv_kernel<8><<<gb, 256, smem_b, s>>>(a);
-  else attn_bwd_dkv_kernel<4><<<gb, 128, smem_b, s>>>(a);
-  count_launch();
-  return (int)cudaGetLastError();
+  if (rc) return rc;
+  if (smem_b > RESIDENT_SMEM_MAX) {
+    const size_t sm = (size_t)(2 * rk + 2 * KV_CHUNK) * ROW_BYTES + 2 * KV_CHUNK * sizeof(float);
+    return big_k ? launch_attn_bwd_dkv<8, true>(a, sm, s) : launch_attn_bwd_dkv<4, true>(a, sm, s);
+  }
+  return big_k ? launch_attn_bwd_dkv<8, false>(a, smem_b, s) : launch_attn_bwd_dkv<4, false>(a, smem_b, s);
 }
 
 }  // namespace xfm

@@ -56,17 +56,18 @@ struct VitCfg {
   static_assert(2 * LPAD + 64 <= 512, "scores of two tiles + one output tile must fit TMEM");
 };
 // Forward configuration.  Up to 208 keys: an item is one (sample, head) with all its query tiles (== VitCfg).  More (384 px,
-// W = 24, L = 577): one launch per block of 192 keys writes a block-normalised partial output and the block's lse; the
+// W = 24, L = 577; 480 px, W = 30, L = 901): one launch per key block (KeyBlocks) writes a block-normalised partial output
+// and the block's lse; the
 // partials are merged afterwards (merge_parts_kernel).  An item is then a PAIR of query tiles of a (sample, head), a CTA
 // stays on one head (one copy of the bias table, loaded once), and the K / V block is re-loaded per item (L2 hits).
 template <int W>
 struct VitFwdCfg {
   static constexpr int L = W * W + 1;
-  static constexpr bool BLOCKED = L > 208;
-  static constexpr int KBS = BLOCKED ? 192 : L;
-  static constexpr int NB = BLOCKED ? (L - 1) / 192 : 1;
-  static constexpr int LAST = L - (NB - 1) * KBS;
-  static constexpr int LPAD = BLOCKED ? 208 : (L + 15) / 16 * 16;
+  static constexpr int NB = KeyBlocks::nb(L);
+  static constexpr bool BLOCKED = NB > 1;
+  static constexpr int KBS = KeyBlocks::kbs(L);
+  static constexpr int LAST = KeyBlocks::last(L);
+  static constexpr int LPAD = KeyBlocks::lpad(L);
   static constexpr int NT = BLOCKED ? 2 : (L + 127) / 128;          // query tiles per item
   static constexpr int NTP = BLOCKED ? ((L + 127) / 128 + 1) / 2 : 1;  // items per (sample, head)
   static constexpr int NKB = (LPAD + 63) / 64;
@@ -82,6 +83,8 @@ struct VitFwdCfg {
   static_assert(LAST <= LPAD && 2 * LPAD + 64 <= 512, "scores of two tiles + one output tile must fit TMEM");
   static_assert(SMEM_BYTES <= 232448, "shared memory");
 };
+static_assert(VitFwdCfg<24>::NB == 3 && VitFwdCfg<24>::LAST == 193 && VitFwdCfg<24>::LPAD == 208, "384 px: 192 / 192 / 193");
+static_assert(VitFwdCfg<30>::NB == 5 && VitFwdCfg<30>::LAST == 133 && VitFwdCfg<30>::LPAD == 192, "480 px: 4 x 192 + 133");
 // column part of the relative-position index (beit2.py:104-108) of key j >= 1
 template <int W>
 XFM_DEVINL constexpr int rel_off(int j) {
@@ -956,31 +959,41 @@ vit_attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gr
 // kernels, therefore runs once per (query, key) pair instead of once in a dQ kernel and again in a dK/dV kernel.  The outputs
 // re-use the TMEM columns of S / dP; the second query tile of a (sample, head) adds its dK / dV to the first tile's rows in
 // global memory (same thread, same rows: no synchronisation needed).
-// Samples with more than 208 keys (384 px: W = 24, L = 577) are processed one KEY BLOCK of 192 keys per launch (the last
-// block takes the remainder, 193): the backward needs no online softmax — P = 2^(S - lse) with the forward's lse — so a
+// Samples with more than 208 keys (384 px: W = 24, L = 577; 480 px: W = 30, L = 901) are processed one KEY BLOCK per launch
+// (KeyBlocks: 192 / 192 / 193 keys at 577, 4 x 192 + 133 at 901; scores beyond a block's keys are masked): the backward needs no online softmax — P = 2^(S - lse) with the forward's lse — so a
 // key block is just a narrower K / V operand, an offset into the relative-position index, per-block dK / dV rows, and dQ
 // accumulated across the launches (block 0 stores, later blocks TMA-reduce-add; launches of one stream run in order).
 template <int W>
 struct VitFusedCfg {
   static constexpr int L = W * W + 1;
-  static constexpr bool BLOCKED = L > 208;
-  static constexpr int KBS = BLOCKED ? 192 : L;                    // keys per block
-  static constexpr int NB = BLOCKED ? (L - 1) / 192 : 1;           // key blocks = launches
-  static constexpr int LAST = L - (NB - 1) * KBS;                  // keys of the last block
-  static constexpr int LPAD = BLOCKED ? 208 : (L + 15) / 16 * 16;  // score columns in TMEM / operand rows in shared memory
+  static constexpr int NB = KeyBlocks::nb(L);                      // key blocks = launches
+  static constexpr bool BLOCKED = NB > 1;
+  static constexpr int KBS = KeyBlocks::kbs(L);                    // keys per block
+  static constexpr int LAST = KeyBlocks::last(L);                  // keys of the last block
+  static constexpr int LPAD = KeyBlocks::lpad(L);                  // score columns in TMEM / operand rows in shared memory
   static constexpr int NT = (L + 127) / 128;
   static constexpr int T = (2 * W - 1) * (2 * W - 1) + 3;
   static constexpr int OFFMAX = (W - 1) * (2 * W - 1) + (W - 1);
-  static constexpr int TAB_FLOATS = (OFFMAX + 1 + T + 7) & ~7;
   static constexpr int KV_BYTES = LPAD * 128;
   static constexpr int NM = (LPAD + 127) / 128;                    // 128-key M tiles of dK / dV
   static constexpr int PD_BYTES = 2 * NM * 16384;                  // P / dS operand: whole 64-key blocks for every M tile
-  static constexpr int SMEM = 2 * 16384 + 2 * KV_BYTES + 2 * PD_BYTES + TAB_FLOATS * 4 + 128;
+  static constexpr int SMEM_NO_TAB = 2 * 16384 + 2 * KV_BYTES + 2 * PD_BYTES + 128;
+  // The bias table is staged as [OFFMAX+1 copies of table[T-3]] ++ [table], so that the CLS query row reads its constant
+  // through the same address arithmetic as every other row.  Where that prefix does not fit (W = 30: 6 964 bytes over the
+  // limit with it) only the table is staged and row 0 selects its constant instead; the values stay the exact fp32 entries.
+  static constexpr bool ROW0_PREFIX = SMEM_NO_TAB + ((OFFMAX + 1 + T + 7) & ~7) * 4 <= 232448;
+  static constexpr int PREFIX = ROW0_PREFIX ? OFFMAX + 1 : 0;      // table[i] is tab[PREFIX + i]
+  static constexpr int TAB_FLOATS = (PREFIX + T + 7) & ~7;
+  static constexpr int SMEM = SMEM_NO_TAB + TAB_FLOATS * 4;
   static constexpr int TM_DQ = 0, TM_DK = 64, TM_DV = 64 + 64 * NM, TM_END = 64 + 128 * NM;
   static constexpr int UNITS = TM_END / 32;                        // 32-column drain units, split between the warpgroups
   static_assert(LAST <= LPAD && 2 * LPAD <= 512 && TM_END <= 512, "TMEM");
   static_assert(SMEM <= 232448, "shared memory");
 };
+static_assert(VitFusedCfg<24>::NB == 3 && VitFusedCfg<24>::LAST == 193 && VitFusedCfg<24>::LPAD == 208 &&
+              VitFusedCfg<24>::ROW0_PREFIX && VitFusedCfg<14>::ROW0_PREFIX, "384 / 224 px backward: unchanged geometry");
+static_assert(VitFusedCfg<30>::NB == 5 && VitFusedCfg<30>::LAST == 133 && VitFusedCfg<30>::LPAD == 192 &&
+              !VitFusedCfg<30>::ROW0_PREFIX, "480 px backward");
 
 template <int W, int KB, bool PROF>
 __global__ void __launch_bounds__(TCF_THREADS, 1)
@@ -1002,7 +1015,7 @@ vit_attn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __
   uint8_t* sV = sK + Cfg::KV_BYTES;
   uint8_t* sdS = sV + Cfg::KV_BYTES;
   uint8_t* sP = sdS + Cfg::PD_BYTES;
-  float* tab = (float*)(sP + Cfg::PD_BYTES);    // [OFFMAX+1 copies of table[T-3]] ++ [table], log2 domain
+  float* tab = (float*)(sP + Cfg::PD_BYTES);    // [PREFIX copies of table[T-3]] ++ [table], log2 domain
   uint64_t* bars = (uint64_t*)(tab + Cfg::TAB_FLOATS);
   uint64_t *kv_full = bars, *kv_empty = bars + 1, *qdo_full = bars + 2, *qdo_empty = bars + 3, *sd_full = bars + 4,
            *ds_full = bars + 5, *out_full = bars + 6, *out_empty = bars + 7;
@@ -1130,20 +1143,23 @@ vit_attn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __
       if (h != cur_h) {
         named_bar_sync(1, 512);
         for (int i = wgt; i < Cfg::T; i += 512)
-          tab[Cfg::OFFMAX + 1 + i] = a.table ? __ldg(a.table + (int64_t)i * a.H + h) * 1.4426950408889634f : 0.f;
+          tab[Cfg::PREFIX + i] = a.table ? __ldg(a.table + (int64_t)i * a.H + h) * 1.4426950408889634f : 0.f;
         const float row0 = a.table ? __ldg(a.table + (int64_t)(Cfg::T - 3) * a.H + h) * 1.4426950408889634f : 0.f;
-        for (int i = wgt; i <= Cfg::OFFMAX; i += 512) tab[i] = row0;
+        for (int i = wgt; i < Cfg::PREFIX; i += 512) tab[i] = row0;
         named_bar_sync(1, 512);
         cur_h = h;
       }
       const int qc = qi < L ? qi : L - 1;
       const bool row_ok = qi < L;
       const bool wv = __any_sync(0xffffffffu, row_ok);
-      const int rb_off = qc >= 1 ? Cfg::OFFMAX + 1 + (((qc - 1) / W) + W - 1) * (2 * W - 1) + ((qc - 1) % W) + W - 1
-                                 : Cfg::OFFMAX;
+      // row 0 without the prefix: any base keeps the (discarded) gather inside the table
+      const int rb_off = qc >= 1 ? Cfg::PREFIX + (((qc - 1) / W) + W - 1) * (2 * W - 1) + ((qc - 1) % W) + W - 1
+                                 : (Cfg::ROW0_PREFIX ? Cfg::OFFMAX : Cfg::PREFIX + Cfg::OFFMAX);
       const float* rb = tab + rb_off;
-      const int c0_idx = Cfg::OFFMAX + 1 + (qc >= 1 ? Cfg::T - 2 : Cfg::T - 1);
+      const int c0_idx = Cfg::PREFIX + (qc >= 1 ? Cfg::T - 2 : Cfg::T - 1);
       const float bias_c0 = tab[c0_idx];
+      const bool cls_row = !Cfg::ROW0_PREFIX && qc == 0;
+      const float bias_r0 = tab[Cfg::PREFIX + Cfg::T - 3];
       const int64_t st_row = ((int64_t)b * a.H + h) * L + qc;
       const float lse2 = __ldg(a.lse + st_row) * 1.4426950408889634f;
       const float dl = __ldg(a.delta + st_row);
@@ -1181,7 +1197,7 @@ vit_attn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __
 #pragma unroll
           for (int e = 0; e < 8; ++e) {
             const int j = col8 + e;              // key inside the block; K0 + j inside the sample
-            const float bias2 = K0 + j == 0 ? bias_c0 : *(rb - rel_off<W>(K0 + j));
+            const float bias2 = K0 + j == 0 ? bias_c0 : (cls_row ? bias_r0 : *(rb - rel_off<W>(K0 + j)));
             float p = ex2_approx(fmaf(__uint_as_float(vs[g8 * 8 + e]), scale2, bias2) - lse2);
             if (j >= KLEN || !row_ok) p = 0.f;
             pp[e] = p;
@@ -1327,17 +1343,18 @@ static int encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, uin
 }
 
 // window sides with an instantiated kernel: 14 (224 px / 16), 12 and 7 (test sizes), 4 (tiny parity model); the fused
-// backward also 24 (384 px / 16: three key blocks per sample)
+// backward, and the forward given the key-block scratch, also 24 (384 px / 16: three key blocks per sample) and 30
+// (480 px / 16: five key blocks)
 static int window_for(int L, bool bwd = false) {
-  const int ws[] = {14, 12, 7, 4, 24};
-  for (int i = 0; i < (bwd ? 5 : 4); ++i)
+  const int ws[] = {14, 12, 7, 4, 24, 30};
+  for (int i = 0; i < (bwd ? 6 : 4); ++i)
     if (ws[i] * ws[i] + 1 == L) return ws[i];
   return 0;
 }
 
 bool vit_attention_tc_supported(const xfm_attn_params* p, bool bwd) {
-  const int w = window_for(p->Lk, bwd || (p->part_out && p->part_lse));   // forward at 24: needs the key-block scratch
-  if (w == 24 && p->rel_dtable) return false;   // key-blocked shape: fused kernel only (table gradient from the dS dump)
+  const int w = window_for(p->Lk, bwd || (p->part_out && p->part_lse));   // forward at 24 / 30: needs the key-block scratch
+  if (w * w + 1 > 208 && p->rel_dtable) return false;   // key-blocked shape: fused kernel only (table gradient from the dS dump)
   return p->head_dim == TC_HD && p->Lq == p->Lk && w > 0 && !p->kmask && !p->kv_index &&
          (!p->bias || p->rel_table) && !(p->dropout_p > 0.f) && (p->Bkv == 0 || p->Bkv == p->B) &&
          (p->rel_table == nullptr || p->rel_window == w) &&
@@ -1385,11 +1402,12 @@ __global__ void merge_parts_kernel(const bf16* __restrict__ part_out, const floa
 
 int launch_merge_parts(int nb, const void* part_out, const float* part_lse, void* out, int64_t o_stride, float* lse, int B, int H,
                        int L, cudaStream_t s) {
-  if (nb != 3 || H * 8 > 1024) {
+  if ((nb != 3 && nb != 5) || H * 8 > 1024) {
     set_error("merge of key-block partials: %d blocks / %d heads not instantiated", nb, H);
     return XFM_ERR_BAD_ARG;
   }
-  merge_parts_kernel<3><<<(unsigned)(B * L), H * 8, 0, s>>>((const bf16*)part_out, part_lse, (bf16*)out, o_stride, lse, B, H, L);
+  if (nb == 3) merge_parts_kernel<3><<<(unsigned)(B * L), H * 8, 0, s>>>((const bf16*)part_out, part_lse, (bf16*)out, o_stride, lse, B, H, L);
+  else merge_parts_kernel<5><<<(unsigned)(B * L), H * 8, 0, s>>>((const bf16*)part_out, part_lse, (bf16*)out, o_stride, lse, B, H, L);
   count_launch();
   return (int)cudaGetLastError();
 }
@@ -1592,6 +1610,7 @@ int vit_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s) {
     return XFM_ERR_BAD_ARG;
   }
   switch (window_for(p->Lk, true)) {
+    case 30: return launch_vit_bwd_fused<30>(p, s);
     case 24: return launch_vit_bwd_fused<24>(p, s);
     case 14: return launch_vit_bwd<14>(p, s);
     case 12: return launch_vit_bwd<12>(p, s);
@@ -1604,6 +1623,7 @@ int vit_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s) {
 
 int vit_attention_fwd_tc(const xfm_attn_params* p, cudaStream_t s) {
   switch (window_for(p->Lk, true)) {
+    case 30: return launch_vit_fwd<30>(p, s);
     case 24: return launch_vit_fwd<24>(p, s);
     case 14: return launch_vit_fwd<14>(p, s);
     case 12: return launch_vit_fwd<12>(p, s);

@@ -41,13 +41,13 @@ struct XCfg {
   static constexpr int PER_TILE = (GMAX + 1) / 2;            // sample slots per 128-row query tile
   static_assert(PER_TILE * LQS <= 128, "slots of one tile must fit 128 rows");
   static_assert((LQS * 128) % 1024 == 0, "a sample's rows must start on a swizzle-atom boundary (LQS multiple of 8)");
-  // more than 208 keys (384 px: 577): one launch per block of 192 keys, partial results merged afterwards (forward) — see
-  // attention_tc.cu::VitFwdCfg
-  static constexpr bool BLOCKED = LK > 208;
-  static constexpr int KBS = BLOCKED ? 192 : LK;
-  static constexpr int NB = BLOCKED ? (LK - 1) / 192 : 1;
-  static constexpr int LAST = LK - (NB - 1) * KBS;
-  static constexpr int LPAD = BLOCKED ? 208 : (LK + 15) / 16 * 16;
+  // more than 208 keys (384 px: 577, 480 px: 901): one launch per key block (KeyBlocks), partial results merged afterwards
+  // (forward) — see attention_tc.cu::VitFwdCfg
+  static constexpr int NB = KeyBlocks::nb(LK);
+  static constexpr bool BLOCKED = NB > 1;
+  static constexpr int KBS = KeyBlocks::kbs(LK);
+  static constexpr int LAST = KeyBlocks::last(LK);
+  static constexpr int LPAD = KeyBlocks::lpad(LK);
   static_assert(LAST <= LPAD && (NB == 1 || KBS % 2 == 0), "key blocks");
   static constexpr int NKB = (LPAD + 63) / 64;
   static constexpr int Q_BYTES = 2 * 128 * 128;
@@ -849,13 +849,13 @@ template <int LQS, int LK>
 struct XFusedCfg {
   static constexpr int GMAX = 3;
   static_assert(GMAX * LQS <= 128, "three samples per query tile");
-  // Images with more than 208 tokens (384 px: 577) are processed one block of 192 keys per launch, like the ViT backward
+  // Images with more than 208 tokens (384 px: 577, 480 px: 901) are processed one key block per launch, like the ViT backward
   // (attention_tc.cu::VitFusedCfg): P = 2^(S - lse) needs no online softmax; dQ accumulates across the launches.
-  static constexpr bool BLOCKED = LK > 208;
-  static constexpr int KBS = BLOCKED ? 192 : LK;
-  static constexpr int NB = BLOCKED ? (LK - 1) / 192 : 1;
-  static constexpr int LAST = LK - (NB - 1) * KBS;
-  static constexpr int LPAD = BLOCKED ? 208 : (LK + 15) / 16 * 16;
+  static constexpr int NB = KeyBlocks::nb(LK);
+  static constexpr bool BLOCKED = NB > 1;
+  static constexpr int KBS = KeyBlocks::kbs(LK);
+  static constexpr int LAST = KeyBlocks::last(LK);
+  static constexpr int LPAD = KeyBlocks::lpad(LK);
   static constexpr int NM = (LPAD + 127) / 128;
   static constexpr int KV_BYTES = LPAD * 128;
   static constexpr int PD_BYTES = 2 * NM * 16384;
@@ -865,6 +865,8 @@ struct XFusedCfg {
   static_assert(LAST <= LPAD && (NB == 1 || KBS % 2 == 0) && 2 * LPAD <= 512 && TM_END <= 512, "TMEM / dropout pairs");
   static_assert(SMEM <= 232448, "shared memory");
 };
+static_assert(XFusedCfg<40, 577>::NB == 3 && XFusedCfg<40, 577>::LAST == 193 && XFusedCfg<40, 577>::LPAD == 208, "384 px");
+static_assert(XFusedCfg<40, 901>::NB == 5 && XFusedCfg<40, 901>::LAST == 133 && XFusedCfg<40, 901>::LPAD == 192, "480 px");
 
 template <int LQS, int LK, int KB>
 __global__ void __launch_bounds__(XTF_THREADS, 1)
@@ -1210,9 +1212,11 @@ static int xt_encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, 
   return 0;
 }
 
-// Instantiated shape: 40 text tokens attending to 197 image tokens (BASELINE configs[1]), up to 6 samples per chunk.
+// Instantiated shapes: 40 text tokens attending to 197 image tokens (BASELINE configs[1]), up to 6 samples per chunk; and
+// to 577 / 901 image tokens (384 / 480 px) in key blocks: the forward needs the part scratch, the backward has no dS dump.
 bool cross_attention_tc_supported(const xfm_attn_params* p, bool bwd) {
-  return p->head_dim == XT_HD && p->Lq == 40 && (p->Lk == 197 || (p->Lk == 577 && (bwd ? !p->ds_dump : (p->part_out && p->part_lse)))) && !p->kmask && !p->bias && p->kv_offsets && p->kv_samples &&
+  const bool blocked = p->Lk == 577 || p->Lk == 901;
+  return p->head_dim == XT_HD && p->Lq == 40 && (p->Lk == 197 || (blocked && (bwd ? !p->ds_dump : (p->part_out && p->part_lse)))) && !p->kmask && !p->bias && p->kv_offsets && p->kv_samples &&
          p->Bkv > 0 && ((uintptr_t)p->q & 15) == 0 && ((uintptr_t)p->k & 15) == 0 && ((uintptr_t)p->v & 15) == 0 &&
          ((p->q_stride | p->k_stride | p->v_stride | p->o_stride) & 7) == 0;
 }
@@ -1273,7 +1277,11 @@ static int xt_launch_fwd(const xfm_attn_params* p, cudaStream_t s) {
 }
 
 int cross_attention_fwd_tc(const xfm_attn_params* p, cudaStream_t s) {
-  return p->Lk == 577 ? xt_launch_fwd<40, 577, 6>(p, s) : xt_launch_fwd<40, 197, 6>(p, s);
+  switch (p->Lk) {
+    case 577: return xt_launch_fwd<40, 577, 6>(p, s);
+    case 901: return xt_launch_fwd<40, 901, 6>(p, s);
+  }
+  return xt_launch_fwd<40, 197, 6>(p, s);
 }
 
 // Fused backward, one launch per key block.
@@ -1329,7 +1337,13 @@ int cross_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s) {
     set_error("cross attention bwd: operands must be 16-byte aligned with row strides that are multiples of 8");
     return XFM_ERR_BAD_ARG;
   }
-  if (!p->ds_dump) return p->Lk == 577 ? xt_launch_fused<LQS, 577>(p, s) : xt_launch_fused<LQS, LK>(p, s);   // one fused kernel
+  if (!p->ds_dump) {   // one fused kernel
+    switch (p->Lk) {
+      case 577: return xt_launch_fused<LQS, 577>(p, s);
+      case 901: return xt_launch_fused<LQS, 901>(p, s);
+    }
+    return xt_launch_fused<LQS, LK>(p, s);
+  }
   XAttnArgs a;
   xt_fill(p, a);
   const uint64_t cols = (uint64_t)a.H * XT_HD;

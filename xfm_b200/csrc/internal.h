@@ -30,6 +30,24 @@ int vit_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s);
 // out / lse from nb key-block partials (bf16 [nb, B*L, H*64], f32 [nb, B, H, L]); attention_tc.cu
 int launch_merge_parts(int nb, const void* part_out, const float* part_lse, void* out, int64_t o_stride, float* lse, int B, int H,
                        int L, cudaStream_t s);
+// Key blocks of the tcgen05 attention kernels (attention_tc.cu, attention_xtc.cu).  Up to 208 keys are one block.  Longer rows
+// are split into blocks of 192 keys (one launch each); a remainder of at most 16 keys joins the last block, a longer one is a
+// block of its own.  577 keys (384 px) -> 192 / 192 / 193, 901 keys (480 px) -> 4 x 192 + 133.
+struct KeyBlocks {
+  static constexpr int KBS_MAX = 192;
+  static constexpr int nb(int L) { return L <= 208 ? 1 : (L % KBS_MAX <= 16 ? L / KBS_MAX : L / KBS_MAX + 1); }
+  static constexpr int kbs(int L) { return L <= 208 ? L : KBS_MAX; }                  // keys of every block but the last
+  static constexpr int last(int L) { return L - (nb(L) - 1) * kbs(L); }             // keys of the last block
+  static constexpr int lpad(int L) {                                                 // score columns: round16(widest block)
+    return ((kbs(L) > last(L) ? kbs(L) : last(L)) + 15) / 16 * 16;
+  }
+};
+static_assert(KeyBlocks::nb(577) == 3 && KeyBlocks::last(577) == 193 && KeyBlocks::lpad(577) == 208, "384 px key blocks");
+static_assert(KeyBlocks::nb(901) == 5 && KeyBlocks::last(901) == 133 && KeyBlocks::lpad(901) == 192, "480 px key blocks");
+static_assert(KeyBlocks::nb(197) == 1 && KeyBlocks::lpad(197) == 208, "224 px: one block");
+// Partial-result blocks the forward of *p needs in part_out / part_lse when they are given (0: none; the chosen path writes
+// out / lse directly).  Host-only: evaluates the same dispatch as attention_fwd.
+int attention_fwd_parts(const xfm_attn_params* p);
 bool cross_attention_tc_supported(const xfm_attn_params* p, bool bwd = false);
 int cross_attention_fwd_tc(const xfm_attn_params* p, cudaStream_t s);
 int cross_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s);

@@ -238,21 +238,15 @@ def attention_fwd(q, k, v, B, H, Lq, Lk, scale, *, Bkv=None, bias=None, kmask=No
         assert rel_table.dtype == torch.float32 and rel_table.is_contiguous() and rel_table.shape[1] == H
         assert rel_table.shape[0] == (2 * rel_window - 1) ** 2 + 3
         p.rel_table, p.rel_window = rel_table.data_ptr(), rel_window
-    parts = None
-    if (allow_tc and Lq == Lk == 577 and kmask is None and kv_index is None and dropout_p == 0.0
-            and (bias is None or rel_table is not None)):
-        # 384 px self-attention on tcgen05: one launch per block of 192 keys + a merge; scratch for the partial results
-        parts = (torch.empty((3, B * Lq, H * 64), dtype=torch.bfloat16, device=q.device),
-                 torch.empty((3, B, H, Lq), dtype=torch.float32, device=q.device))
-        p.part_out, p.part_lse = parts[0].data_ptr(), parts[1].data_ptr()
-    if allow_tc and Lq == 40 and Lk == 577 and kv_samples is not None and kmask is None and bias is None:   # cross-attention, 384 px
-        parts = (torch.empty((3, B * Lq, H * 64), dtype=torch.bfloat16, device=q.device),
-                 torch.empty((3, B, H, Lq), dtype=torch.float32, device=q.device))
-        p.part_out, p.part_lse = parts[0].data_ptr(), parts[1].data_ptr()
     if kv_samples is not None:  # CSR inverse of kv_index: lets the tcgen05 cross-attention kernel stack the samples of an image
         assert kv_offsets.dtype == torch.int32 and kv_samples.dtype == torch.int32
         assert kv_offsets.numel() == Bkv + 1 and kv_samples.numel() == B
         p.kv_offsets, p.kv_samples = kv_offsets.data_ptr(), kv_samples.data_ptr()
+    nb = load().xfm_attention_fwd_parts(C.byref(p))
+    if nb:  # tcgen05 path in key blocks (384 / 480 px): one launch per block + a merge; scratch for the partial results
+        parts = (torch.empty((nb, B * Lq, H * 64), dtype=torch.bfloat16, device=q.device),
+                 torch.empty((nb, B, H, Lq), dtype=torch.float32, device=q.device))
+        p.part_out, p.part_lse = parts[0].data_ptr(), parts[1].data_ptr()
     check(lib().xfm_attention_fwd(C.byref(p), stream_ptr()), "xfm_attention_fwd")
     return out, lse
 
@@ -298,8 +292,9 @@ def vit_attention_tc_ok(n_tokens):
 
 
 def vit_attention_bwd_tc_ok(n_tokens):
-    """Token counts the fused tcgen05 backward handles: the forward's plus 577 (384 px), processed in three key blocks."""
-    return n_tokens in (197, 145, 50, 17, 577)
+    """Token counts the fused tcgen05 backward handles: the forward's plus 577 (384 px) and 901 (480 px), processed in key
+    blocks of about 192 keys (three and five)."""
+    return n_tokens in (197, 145, 50, 17, 577, 901)
 
 
 # ------------------------------------------------------------------------------------------------------
