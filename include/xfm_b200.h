@@ -132,14 +132,12 @@ typedef struct xfm_attn_params {
    * gathers the bias from the table instead of reading `bias`; `bias` must then hold the same values (backward). */
   const float* rel_table;
   int32_t rel_window;
-  int32_t allow_tc;
+  int32_t allow_tc; /* 1: use a tcgen05 / TMEM kernel when the problem fits one; 0: always the mma.sync kernels */
   /* Forward scratch for rows processed in key blocks (577 keys at 384 px: 3 blocks; 901 at 480 px: 5): bf16 [nb, B*Lq, H*64]
    * block-normalised partial outputs and f32 [nb, B, H, Lq] block lse, merged into out / lse by a last kernel, with nb from
    * xfm_attention_fwd_parts.  Without them these forwards run on the mma.sync kernel. */
   void* part_out;
   float* part_lse;
-  float* rel_dtable; /* backward: gradient of rel_table, accumulated (+=) by the tcgen05 dQ kernel; when null or when the
-                      * tcgen05 path is not taken the caller derives it from ds_dump */ /* 1: use the tcgen05 / TMEM kernel when the problem fits it (self-attention, Lk <= 208) */
 } xfm_attn_params;
 
 int xfm_attention_fwd(const xfm_attn_params* p, void* stream);

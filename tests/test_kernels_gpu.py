@@ -501,8 +501,9 @@ def test_vit_attention_tcgen05_forward(lib, B, H, ws, with_table):
 
 @pytest.mark.parametrize("B,H,ws,with_table", [(3, 12, 14, True), (2, 2, 14, False), (2, 2, 4, True), (5, 3, 7, True),
                                                (2, 1, 12, True), (30, 12, 14, True)])
-def test_vit_attention_tcgen05_backward(lib, B, H, ws, with_table):
-    """tcgen05 dQ / dK / dV kernels and the in-kernel relative-position-table gradient against torch autograd."""
+def test_vit_attention_tcgen05_fused_backward(lib, B, H, ws, with_table):
+    """tcgen05 fused dQ / dK / dV kernel, with and without the bf16 dS dump, and the relative-position-table gradient reduced
+    from that dump as the model does it, against torch autograd."""
     from xfm_b200.encoders import closed_form_rel_index
     g = G(ws * 1000 + B)
     L, D = ws * ws + 1, H * 64
@@ -527,19 +528,16 @@ def test_vit_attention_tcgen05_backward(lib, B, H, ws, with_table):
     kw = dict(rel_table=tdev, rel_window=ws if with_table else 0)
     out, lse = lib.attention_fwd(q, k, v, B, H, L, L, 0.125, **kw)
     dqkv = torch.full_like(c, float("nan"))
-    dtab = None if table is None else torch.zeros_like(tdev)
-    lib.attention_bwd(do, q, k, v, out, lse, B, H, L, L, 0.125, dqkv[:, :D], dqkv[:, D:2 * D], dqkv[:, 2 * D:],
-                      rel_dtable=dtab, **kw)
+    n0 = lib.launch_count()
+    lib.attention_bwd(do, q, k, v, out, lse, B, H, L, L, 0.125, dqkv[:, :D], dqkv[:, D:2 * D], dqkv[:, 2 * D:], **kw)
+    assert lib.launch_count() - n0 == 2      # row-delta kernel + one fused launch
     got = dqkv.float().cpu()
     assert torch.isfinite(got).all()
     scale = float(want.abs().max())
     for name, sl in (("dq", slice(0, D)), ("dk", slice(D, 2 * D)), ("dv", slice(2 * D, 3 * D))):
         err = float((got[:, sl] - want[:, sl]).abs().max())
         assert err < 2.5e-2 * max(1.0, scale), (name, err, scale)
-    if table is not None:
-        err = float((dtab.cpu() - table.grad).abs().max())
-        assert err < 2e-2 * max(1.0, float(table.grad.abs().max())), ("dtable", err, float(table.grad.abs().max()))
-    # the fused dQ/dK/dV kernel (taken when the table gradient is NOT accumulated in-kernel) with the bf16 dS dump
+    # the same kernel with the bf16 dS dump
     ld = (L + 7) // 8 * 8
     ds = torch.zeros(B, H, L, ld, dtype=torch.bfloat16, device="cuda")
     dqkv2 = torch.full_like(c, float("nan"))
@@ -548,9 +546,14 @@ def test_vit_attention_tcgen05_backward(lib, B, H, ws, with_table):
     assert torch.isfinite(got2).all()
     for name, sl in (("dq", slice(0, D)), ("dk", slice(D, 2 * D)), ("dv", slice(2 * D, 3 * D))):
         err = float((got2[:, sl] - want[:, sl]).abs().max())
-        assert err < 2.5e-2 * max(1.0, scale), ("fused " + name, err, scale)
+        assert err < 2.5e-2 * max(1.0, scale), ("with dump: " + name, err, scale)
     err = float((ds[..., :L].float().cpu() - s.grad).abs().max())
     assert err < 1e-2 * max(1.0, float(s.grad.abs().max())), ("ds_dump", err)
+    if table is not None:   # the table gradient from the dump, reduced as blocks.vit_block_bwd does
+        dtab = torch.zeros_like(tdev)
+        lib.relpos_bias_bwd(lib.batch_sum_bf16(ds), closed_form_rel_index(ws).cuda(), dtab, L, H, ld)
+        err = float((dtab.cpu() - table.grad).abs().max())
+        assert err < 2e-2 * max(1.0, float(table.grad.abs().max())), ("table grad", err, float(table.grad.abs().max()))
 
 
 @pytest.mark.parametrize("B,H,with_table", [(2, 3, True), (1, 2, False), (5, 12, True), (32, 12, True)])

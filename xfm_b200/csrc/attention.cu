@@ -695,11 +695,8 @@ int attention_bwd(const xfm_attn_params* p, cudaStream_t s) {
     attn_delta_kernel<<<(a.B * a.Lq + 3) / 4, blk, 0, s>>>(a.dout, a.do_stride, a.out, a.o_stride, (float*)p->delta, a.B, a.H, a.Lq);
     count_launch();
   }
-  // tcgen05 path: needs the closed-form table whenever there is a bias; the table gradient either comes out of the bf16
-  // dS dump (reduced by the caller) or is accumulated in-kernel into rel_dtable (shared-memory atomics: slower)
-  if (p->allow_tc && vit_attention_tc_supported(p, true) && (!p->bias || p->rel_table))
-    return vit_attention_bwd_tc(p, s);
-  if (p->allow_tc && cross_attention_tc_supported(p, true) && !p->ds_dump) return cross_attention_bwd_tc(p, s);
+  if (p->allow_tc && vit_attention_tc_supported(p, true)) return vit_attention_bwd_tc(p, s);
+  if (p->allow_tc && cross_attention_tc_supported(p, true)) return cross_attention_bwd_tc(p, s);
   if (p->allow_tc && self_attention_tc_supported(p) && !p->ds_dump) return self_attention_bwd_tc(p, s);
   const bool big_q = a.Lq > 256, big_k = a.Lk > 256;
   const int rq = big_q ? 128 : 64, rk = big_k ? 128 : 64;

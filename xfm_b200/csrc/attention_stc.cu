@@ -46,14 +46,6 @@ XFM_DEVINL void st_ld16(uint32_t taddr, uint32_t (&r)[16]) {
       : "r"(taddr)
       : "memory");
 }
-XFM_DEVINL void st_named_bar(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
-XFM_DEVINL void st_st_bf16x8(uint8_t* dst, const float (&p)[8]) {
-  uint4 u;
-  __nv_bfloat162 t0 = __floats2bfloat162_rn(p[0], p[1]), t1 = __floats2bfloat162_rn(p[2], p[3]);
-  __nv_bfloat162 t2 = __floats2bfloat162_rn(p[4], p[5]), t3 = __floats2bfloat162_rn(p[6], p[7]);
-  u.x = *(uint32_t*)&t0; u.y = *(uint32_t*)&t1; u.z = *(uint32_t*)&t2; u.w = *(uint32_t*)&t3;
-  *(uint4*)dst = u;
-}
 
 // Columns a warp has to look at: the union of the diagonal blocks of its 32 rows.
 XFM_DEVINL void st_union(int quad, int& ulo, int& uhi) {
@@ -200,7 +192,7 @@ sattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
         const int64_t flat = (int64_t)grp * ST_ROWS + r;   // == b * 40 + q for live rows
         mk[r] = (a.kmask && r < ST_ROWS && flat < (int64_t)a.B * ST_L) ? __ldg(a.kmask + flat) * ST_LOG2E : 0.f;
       }
-      st_named_bar(1 + t, 128);
+      named_bar_sync(1 + t, 128);
       const uint64_t pair_base = ((((uint64_t)(valid ? b : 0) * a.H + h) * ST_L + q) * (uint64_t)ST_L) >> 1;
       const uint32_t pb_lo = (uint32_t)pair_base, pb_hi = (uint32_t)(pair_base >> 32);
       mbar_wait(&s_full[t], ph);
@@ -251,7 +243,7 @@ sattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
             p[e] = p0;
             p[e + 1] = p1;
           }
-          st_st_bf16x8(myP + (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4), p);
+          st_bf16x8(myP + (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4), p);
         }
       }
       const float sum = (s4[0] + s4[1]) + (s4[2] + s4[3]);
@@ -280,7 +272,7 @@ sattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
             float vv[8];
 #pragma unroll
             for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[hh][e + k]) * inv;
-            st_st_bf16x8(stg + lane * 128 + (((hh * 4 + (e >> 3)) ^ (lane & 7)) << 4), vv);
+            st_bf16x8(stg + lane * 128 + (((hh * 4 + (e >> 3)) ^ (lane & 7)) << 4), vv);
           }
         if (valid && a.lse) a.lse[((int64_t)b * a.H + h) * ST_L + q] = (m + log2f(sum)) * 0.6931471805599453f;
         __syncwarp();
@@ -455,7 +447,7 @@ sattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
         const int64_t flat = (int64_t)grp * ST_ROWS + r;
         mk[r] = (a.kmask && r < ST_ROWS && flat < (int64_t)a.B * ST_L) ? __ldg(a.kmask + flat) * ST_LOG2E : 0.f;
       }
-      st_named_bar(1, 256);
+      named_bar_sync(1, 256);
       const int64_t st_row = ((int64_t)(valid ? b : 0) * a.H + h) * ST_L + q;
       const float lse2 = valid ? __ldg(a.lse + st_row) * ST_LOG2E : 0.f;
       const float dl = valid ? __ldg(a.delta + st_row) : 0.f;
@@ -501,8 +493,8 @@ sattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
             ds[e + 1] = d1;
           }
           const int off8 = (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4);
-          st_st_bf16x8(myP + off8, pp);
-          st_st_bf16x8(myD + off8, ds);
+          st_bf16x8(myP + off8, pp);
+          st_bf16x8(myD + off8, ds);
         }
       }
       fence_proxy_async();
@@ -546,7 +538,7 @@ sattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
             float vv[8];
 #pragma unroll
             for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[part][e + k]) * mul;
-            st_st_bf16x8(stg + lane * 64 + ((((e >> 3)) ^ ((lane >> 1) & 3)) << 4), vv);
+            st_bf16x8(stg + lane * 64 + ((((e >> 3)) ^ ((lane >> 1) & 3)) << 4), vv);
           }
           __syncwarp();
           const int ch = lane & 3;
@@ -572,20 +564,7 @@ sattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
 
 // ------------------------------------------------------------------------------------------ host
 static int st_encode_rows(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems) {
-  auto fn = get_tensor_map_encoder();
-  if (!fn) return XFM_ERR_NO_DRIVER;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld_elems * 2};
-  cuuint32_t box[2] = {ST_HD, ST_ROWS};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("self attention: cuTensorMapEncodeTiled failed: %d", (int)r);
-    return XFM_ERR_BAD_ARG;
-  }
-  return 0;
+  return encode_rows(map, base, cols, rows, ld_elems, ST_ROWS);
 }
 
 // Instantiated shape: 40-token text / fusion sequences (BASELINE configs[1] max_tokens), optional additive key mask,

@@ -39,23 +39,7 @@ struct VitAttnArgs {
   long long* prof;       // XFM_ATTN_PROF=1: per-phase clock64 totals of CTA 0's first softmax warp (null otherwise)
 };
 
-template <int W>
-struct VitCfg {
-  static constexpr int L = W * W + 1;
-  static constexpr int LPAD = (L + 15) / 16 * 16;
-  static constexpr int NT = (L + 127) / 128;
-  static constexpr int NKB = (LPAD + 63) / 64;
-  static constexpr int T = (2 * W - 1) * (2 * W - 1) + 3;
-  static constexpr int OFFMAX = (W - 1) * (2 * W - 1) + (W - 1);
-  static constexpr int TAB_FLOATS = (OFFMAX + 1 + T + 7) & ~7;  // [OFFMAX+1 copies of table[T-3]] ++ [table]
-  static constexpr int Q_BYTES = NT * 128 * 128;
-  static constexpr int KV_BYTES = LPAD * 128;
-  static constexpr int P_BYTES = NKB * 16384;
-  static constexpr int SMEM_BYTES = Q_BYTES + 2 * KV_BYTES + 2 * P_BYTES + 2 * TAB_FLOATS * 4 + 128;
-  static constexpr int TMEM_O = 2 * LPAD;  // O accumulator columns; S buffers at 0 and LPAD
-  static_assert(2 * LPAD + 64 <= 512, "scores of two tiles + one output tile must fit TMEM");
-};
-// Forward configuration.  Up to 208 keys: an item is one (sample, head) with all its query tiles (== VitCfg).  More (384 px,
+// Forward configuration.  Up to 208 keys: an item is one (sample, head) with all its query tiles.  More (384 px,
 // W = 24, L = 577; 480 px, W = 30, L = 901): one launch per key block (KeyBlocks) writes a block-normalised partial output
 // and the block's lse; the
 // partials are merged afterwards (merge_parts_kernel).  An item is then a PAIR of query tiles of a (sample, head), a CTA
@@ -92,14 +76,6 @@ XFM_DEVINL constexpr int rel_off(int j) {
   return (jj / W) * (2 * W - 1) + jj % W;
 }
 
-XFM_DEVINL void tmem_ld_32x32_16(uint32_t taddr, uint32_t (&r)[32]) {  // 16 columns into r[0..15]
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-}
 XFM_DEVINL void tmem_st_32x32(uint32_t taddr, const uint32_t (&r)[32]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
@@ -420,549 +396,30 @@ vit_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_c
 
 
 // ================================================================================================ backward
-// Both backward kernels keep the forward's structure: two "score-like" MMAs into TMEM (S and dP), an element-wise stage in
-// registers (P = 2^(S*scale2 + bias2 - lse2), dS = P o (dP - delta)), bf16 operands written to shared memory, then the
-// "output-like" MMAs.  The two softmax warpgroups split the COLUMNS of one tile (no row reductions are needed: the
-// forward saved lse, delta = rowsum(dO o O) comes from attn_delta_kernel).
-//   dQ kernel  : rows = queries.  S = Q K^T, dP = dO V^T, dQ = dS K (K read MN-major).  Also accumulates the gradient of
-//                the relative-position table (beit2.py:139-145 backward) with shared-memory atomics through the same
-//                closed-form index, so the [B, H, N, N] dS tensor is never written (the mma.sync path dumps 93 MB/layer).
-//   dK/dV kernel: rows = keys.  S^T = K Q^T, dP^T = V dO^T, dV = P^T dO, dK = dS^T Q (dO / Q read MN-major).
+// One kernel for dQ, dK and dV.  Per query tile S = Q K^T and dP = dO V^T are computed once into TMEM, the element-wise stage
+// (P = 2^(S*scale2 + bias2 - lse2), dS = P o (dP - delta); the forward saved lse, delta = rowsum(dO o O) comes from
+// attn_delta_kernel) writes P and dS to shared memory once, and three products are issued from those buffers — dQ = dS K (dS
+// read K-major), dK = dS^T Q and dV = P^T dO (the same buffers read MN-major: keys become the M dimension, 64-key blocks are
+// 16 KB apart).  The outputs re-use the TMEM columns of S / dP.  The gradient of the relative-position table is not formed
+// here: dS goes to the optional bf16 dump, which the caller reduces (batch_sum_bf16, relpos_bias_bwd).
+// Samples with more than 208 keys (384 px: W = 24, L = 577; 480 px: W = 30, L = 901) are processed one KEY BLOCK per launch
+// (KeyBlocks: 192 / 192 / 193 keys at 577, 4 x 192 + 133 at 901; scores beyond a block's keys are masked): the backward needs no online softmax — P = 2^(S - lse) with the forward's lse — so a
+// key block is just a narrower K / V operand, an offset into the relative-position index, per-block dK / dV rows, and dQ
+// accumulated across the launches (block 0 stores, later blocks TMA-reduce-add; launches of one stream run in order).
 struct VitBwdArgs {
   const float* lse;      // [B, H, L]
   const float* delta;    // [B, H, L]
   const float* table;    // [T, H] or null
-  float* dtable;         // [T, H] accumulated (+=) or null
-  bf16* ds_dump;         // [B, H, L, ds_ld] bf16 dS (natural-logit gradient) or null: cheaper than dtable's smem atomics
+  bf16* ds_dump;         // [B, H, L, ds_ld] bf16 dS (natural-logit gradient) or null
   int64_t ds_ld;
   bf16 *dq, *dk, *dv;
   int64_t dq_stride, dk_stride, dv_stride;
   int B, H;
   float scale;
   int items_per_cta;
-  long long* prof;       // XFM_ATTN_PROF=1 (fused kernel): per-phase clock64 totals of CTA 0, warps 2 and 9
+  long long* prof;       // XFM_ATTN_PROF=1: per-phase clock64 totals of CTA 0, warps 2 and 15
 };
 
-template <int W>
-struct VitBwdCfg : VitCfg<W> {
-  using Base = VitCfg<W>;
-  static constexpr int SPLIT = ((Base::LPAD / 2 + 15) / 16) * 16;  // columns [0, SPLIT) -> warpgroup 0, rest -> warpgroup 1
-  static constexpr int ROWS_BYTES = Base::NT * 128 * 128;          // a 128-row-tiled operand (Q / dO, or K / V)
-  // dQ kernel: Q, dO (row tiles), K, V (LPAD rows), dS operand, table + its gradient
-  static constexpr int DQ_SMEM = 2 * ROWS_BYTES + 2 * Base::KV_BYTES + Base::P_BYTES + 2 * Base::TAB_FLOATS * 4 + 128;
-  // dK/dV kernel: one K and one V tile, Q, dO (LPAD rows), P^T and dS^T operands, lse2 / delta rows, table
-  static constexpr int REP2 = Base::T - 3 - Base::OFFMAX;           // replicated table[T-2] block for the key-0 row
-  static constexpr int TAB2_FLOATS = (REP2 + Base::T + 7) & ~7;
-  static constexpr int DKV_SMEM = 2 * 16384 + 2 * Base::KV_BYTES + 2 * Base::P_BYTES + 2 * Base::LPAD * 4 + TAB2_FLOATS * 4 + 128;
-  static_assert(2 * Base::LPAD + 64 <= 512, "TMEM");
-};
-// row part of the relative-position index of query q >= 1 (beit2.py:104-108)
-template <int W>
-XFM_DEVINL constexpr int rel_base(int q) {
-  const int qq = (q < W * W + 1 ? q : W * W) - 1;
-  return ((qq / W) + W - 1) * (2 * W - 1) + (qq % W) + W - 1;
-}
-
-XFM_DEVINL void st_bf16x8(uint8_t* dst, const float (&p)[8]) {
-  uint4 u;
-  __nv_bfloat162 t0 = __floats2bfloat162_rn(p[0], p[1]), t1 = __floats2bfloat162_rn(p[2], p[3]);
-  __nv_bfloat162 t2 = __floats2bfloat162_rn(p[4], p[5]), t3 = __floats2bfloat162_rn(p[6], p[7]);
-  u.x = *(uint32_t*)&t0; u.y = *(uint32_t*)&t1; u.z = *(uint32_t*)&t2; u.w = *(uint32_t*)&t3;
-  *(uint4*)dst = u;
-}
-
-template <int W>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-vit_attn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_do,
-                          const __grid_constant__ CUtensorMap map_k, const __grid_constant__ CUtensorMap map_v,
-                          const VitBwdArgs a) {
-  using Cfg = VitBwdCfg<W>;
-  constexpr int L = Cfg::L, LPAD = Cfg::LPAD, NT = Cfg::NT, SPLIT = Cfg::SPLIT;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  if (smem_u32(smem) & 1023) __trap();
-  uint8_t* sQ = smem;
-  uint8_t* sdO = sQ + Cfg::ROWS_BYTES;
-  uint8_t* sK = sdO + Cfg::ROWS_BYTES;
-  uint8_t* sV = sK + Cfg::KV_BYTES;
-  uint8_t* sdS = sV + Cfg::KV_BYTES;
-  float* tab = (float*)(sdS + Cfg::P_BYTES);     // [OFFMAX+1 copies of table[T-3]] ++ [table], log2 domain
-  float* gtab = tab + Cfg::TAB_FLOATS;           // gradient accumulator, same layout (natural domain)
-  uint64_t* bars = (uint64_t*)(gtab + Cfg::TAB_FLOATS);
-  uint64_t *in_full = bars, *in_empty = bars + 1, *sd_full = bars + 2, *ds_full = bars + 3, *dq_full = bars + 4,
-           *dq_empty = bars + 5, *k_full = bars + 6, *k_empty = bars + 7;
-  uint32_t* tmem_ptr = (uint32_t*)(bars + 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_do);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    mbar_init(in_full, 1);   // Q, dO, V of an item (dead after its last score MMAs)
-    mbar_init(in_empty, 1);
-    mbar_init(k_full, 1);    // K of an item (also the B operand of dQ)
-    mbar_init(k_empty, 1);
-    mbar_init(sd_full, 1);
-    mbar_init(ds_full, 8);
-    mbar_init(dq_full, 1);
-    mbar_init(dq_empty, 8);
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    tmem_alloc(tmem_ptr, 512);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  constexpr uint32_t TM_S = 0, TM_DP = LPAD, TM_DQ = 2 * LPAD;
-
-  const int n_items = a.B * a.H;
-  const int item0 = blockIdx.x * a.items_per_cta;
-  const int item1 = min(n_items, item0 + a.items_per_cta);
-  const int n_tiles = (item1 - item0) * NT;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      for (int it = item0; it < item1; ++it) {
-        const uint32_t ph = (uint32_t)(it - item0) & 1u;
-        const int h = it / a.B, b = it % a.B;
-        mbar_wait_relaxed(in_empty, ph ^ 1);
-        mbar_arrive_expect_tx(in_full, 2 * Cfg::ROWS_BYTES + Cfg::KV_BYTES);
-        tma_load_2d(sQ, &map_q, in_full, h * TC_HD, b * L);
-        tma_load_2d(sdO, &map_do, in_full, h * TC_HD, b * L);
-        tma_load_2d(sV, &map_v, in_full, h * TC_HD, b * L);
-        mbar_wait_relaxed(k_empty, ph ^ 1);
-        mbar_arrive_expect_tx(k_full, Cfg::KV_BYTES);
-        tma_load_2d(sK, &map_k, k_full, h * TC_HD, b * L);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc_bf16(128, LPAD, 0, 0);
-      constexpr uint32_t idesc_o = make_idesc_bf16(128, TC_HD, 0, 1);
-      const uint32_t aQ = smem_u32(sQ), adO = smem_u32(sdO), aK = smem_u32(sK), aV = smem_u32(sV), adS = smem_u32(sdS);
-      auto issue_scores = [&](int tau) {
-        const int item = tau / NT, t = tau % NT;
-        if (t == 0) {
-          mbar_wait(in_full, (uint32_t)item & 1u);
-          mbar_wait(k_full, (uint32_t)item & 1u);
-          tc_fence_after();
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          umma_bf16(tmem_base + TM_S, make_smem_desc(aQ + t * 16384 + k * 32, 16, 1024), make_smem_desc(aK + k * 32, 16, 1024),
-                    idesc_s, k > 0 ? 1u : 0u);
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          umma_bf16(tmem_base + TM_DP, make_smem_desc(adO + t * 16384 + k * 32, 16, 1024), make_smem_desc(aV + k * 32, 16, 1024),
-                    idesc_s, k > 0 ? 1u : 0u);
-        umma_commit(sd_full);
-        if (t == NT - 1) umma_commit(in_empty);
-      };
-      if (n_tiles > 0) issue_scores(0);
-      for (int tau = 0; tau < n_tiles; ++tau) {
-        const int t = tau % NT;
-        mbar_wait(ds_full, (uint32_t)tau & 1u);             // dS in shared memory, S / dP drained
-        mbar_wait(dq_empty, ((uint32_t)tau & 1u) ^ 1u);     // previous dQ read out
-        tc_fence_after();
-#pragma unroll
-        for (int k = 0; k < LPAD / 16; ++k)
-          umma_bf16(tmem_base + TM_DQ, make_smem_desc(adS + (k >> 2) * 16384 + (k & 3) * 32, 16, 1024),
-                    make_smem_desc(aK + k * 2048, 8192, 1024), idesc_o, k > 0 ? 1u : 0u);
-        umma_commit(dq_full);
-        if (t == NT - 1) umma_commit(k_empty);
-        if (tau + 1 < n_tiles) issue_scores(tau + 1);
-      }
-    }
-    __syncwarp();
-  } else {
-    const int wg = (warp - 2) >> 2;
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const int wgt = threadIdx.x - 64;          // 0..255
-    const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
-    const float scale2 = a.scale * 1.4426950408889634f;
-    uint8_t* myS = sdS + (r >> 3) * 1024 + (r & 7) * 128;
-    const int sw = r & 7;
-    constexpr int C_BEGIN0 = 0, C_END0 = SPLIT, C_END1 = LPAD;
-    int cur_h = -1;
-    auto flush_gtab = [&](int h) {  // gtab -> global dtable (both warpgroups, after a 256-thread barrier)
-      if (!a.dtable) return;
-      for (int i = wgt; i < Cfg::T; i += 256) {
-        float v = gtab[Cfg::OFFMAX + 1 + i];
-        if (i == Cfg::T - 3)
-          for (int k = 0; k <= Cfg::OFFMAX; ++k) v += gtab[k];
-        if (v != 0.f) atomicAdd(a.dtable + (int64_t)i * a.H + h, v);
-      }
-    };
-    for (int tau = 0; tau < n_tiles; ++tau) {
-      const int item = item0 + tau / NT, t = tau % NT;
-      const int h = item / a.B, b = item % a.B;
-      const int qi = t * 128 + r;
-      if (h != cur_h) {
-        named_bar_sync(1, 256);
-        if (cur_h >= 0) flush_gtab(cur_h);
-        named_bar_sync(1, 256);
-        for (int i = wgt; i < Cfg::T; i += 256)
-          tab[Cfg::OFFMAX + 1 + i] = a.table ? __ldg(a.table + (int64_t)i * a.H + h) * 1.4426950408889634f : 0.f;
-        const float row0 = a.table ? __ldg(a.table + (int64_t)(Cfg::T - 3) * a.H + h) * 1.4426950408889634f : 0.f;
-        for (int i = wgt; i <= Cfg::OFFMAX; i += 256) tab[i] = row0;
-        for (int i = wgt; i < Cfg::TAB_FLOATS; i += 256) gtab[i] = 0.f;
-        named_bar_sync(1, 256);
-        cur_h = h;
-      }
-      const int qc = qi < L ? qi : L - 1;
-      const bool row_ok = qi < L;
-      const int rb_off = qc >= 1 ? Cfg::OFFMAX + 1 + (((qc - 1) / W) + W - 1) * (2 * W - 1) + ((qc - 1) % W) + W - 1
-                                 : Cfg::OFFMAX;
-      const float* rb = tab + rb_off;
-      float* gb = gtab + rb_off;
-      const int c0_idx = Cfg::OFFMAX + 1 + (qc >= 1 ? Cfg::T - 2 : Cfg::T - 1);
-      const float bias_c0 = tab[c0_idx];
-      const int64_t st_row = ((int64_t)b * a.H + h) * L + qc;
-      const float lse2 = __ldg(a.lse + st_row) * 1.4426950408889634f;
-      const float dl = __ldg(a.delta + st_row);
-      mbar_wait(sd_full, (uint32_t)tau & 1u);
-      tc_fence_after();
-      const int cb = wg == 0 ? C_BEGIN0 : C_END0, ce = wg == 0 ? C_END0 : C_END1;
-#pragma unroll
-      for (int cc = 0; cc < LPAD; cc += 32) {
-        // warpgroup 0 walks [0, SPLIT), warpgroup 1 [SPLIT, LPAD): same trip structure, compile-time offsets per group
-        if (cc >= (SPLIT > LPAD - SPLIT ? SPLIT : LPAD - SPLIT)) continue;
-        const int c0 = cb + cc;
-        if (c0 >= ce) continue;
-        const bool full = c0 + 32 <= ce;
-        uint32_t vs[32], vp[32];
-        if (full) {
-          tmem_ld_32x32(lane_base + TM_S + c0, vs);
-          tmem_ld_32x32(lane_base + TM_DP + c0, vp);
-        } else {
-          tmem_ld_32x32_16(lane_base + TM_S + c0, vs);
-          tmem_ld_32x32_16(lane_base + TM_DP + c0, vp);
-        }
-        tmem_ld_wait();
-#pragma unroll
-        for (int g8 = 0; g8 < 4; ++g8) {
-          if (!full && g8 >= 2) continue;
-          const int col8 = c0 + g8 * 8;  // SPLIT is a multiple of 16, not 32: a 32-column group may straddle two 64-key blocks
-          uint8_t* dst8 = myS + (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4);
-          float ds[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) {
-            const int j = c0 + g8 * 8 + e;   // wg-dependent, resolved per branch below
-            float bias2;
-            // the column part of the index is an immediate only when j is a compile-time constant: both groups' code paths
-            // are generated (cb is 0 or SPLIT) and selected by the (warp-uniform) wg predicate
-            if (wg == 0) {
-              const int jc = cc + g8 * 8 + e;
-              bias2 = jc == 0 ? bias_c0 : *(rb - rel_off<W>(jc));
-            } else {
-              const int jc = SPLIT + cc + g8 * 8 + e;
-              bias2 = *(rb - rel_off<W>(jc));
-            }
-            const float l2 = fmaf(__uint_as_float(vs[g8 * 8 + e]), scale2, bias2) - lse2;
-            float p = ex2_approx(l2);
-            if (j >= L || !row_ok) p = 0.f;
-            ds[e] = p * (__uint_as_float(vp[g8 * 8 + e]) - dl);
-            if (a.dtable && j < L && row_ok) {
-              if (wg == 0) {
-                const int jc = cc + g8 * 8 + e;
-                atomicAdd(jc == 0 ? gtab + c0_idx : gb - rel_off<W>(jc), ds[e]);
-              } else {
-                const int jc = SPLIT + cc + g8 * 8 + e;
-                atomicAdd(gb - rel_off<W>(jc), ds[e]);
-              }
-            }
-          }
-          st_bf16x8(dst8, ds);
-          if (a.ds_dump && row_ok && col8 < a.ds_ld)   // ds_ld is a multiple of 8: whole 16-byte chunks
-            st_bf16x8((uint8_t*)(a.ds_dump + (st_row * a.ds_ld + col8)), ds);
-        }
-      }
-      fence_proxy_async();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(ds_full);
-      // ---- dQ: this warpgroup stores columns [32 wg, 32 wg + 32)
-      mbar_wait(dq_full, (uint32_t)tau & 1u);
-      tc_fence_after();
-      uint32_t o[32];
-      tmem_ld_32x32(lane_base + TM_DQ + wg * 32, o);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(dq_empty);
-      if (row_ok) {
-        bf16* dst = a.dq + ((int64_t)b * L + qi) * a.dq_stride + h * TC_HD + wg * 32;
-#pragma unroll
-        for (int e = 0; e < 32; e += 8) {
-          float v[8];
-#pragma unroll
-          for (int k = 0; k < 8; ++k) v[k] = __uint_as_float(o[e + k]) * a.scale;
-          st_bf16x8((uint8_t*)(dst + e), v);
-        }
-      }
-    }
-    named_bar_sync(1, 256);
-    if (cur_h >= 0) flush_gtab(cur_h);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
-template <int W>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-vit_attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_do,
-                           const __grid_constant__ CUtensorMap map_k, const __grid_constant__ CUtensorMap map_v,
-                           const VitBwdArgs a) {
-  using Cfg = VitBwdCfg<W>;
-  constexpr int L = Cfg::L, LPAD = Cfg::LPAD, NT = Cfg::NT, SPLIT = Cfg::SPLIT;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  if (smem_u32(smem) & 1023) __trap();
-  uint8_t* sK = smem;                       // one 128-key tile
-  uint8_t* sV = sK + 16384;
-  uint8_t* sQ = sV + 16384;                 // LPAD query rows
-  uint8_t* sdO = sQ + Cfg::KV_BYTES;
-  uint8_t* sPT = sdO + Cfg::KV_BYTES;       // P^T operand  [128 keys x LPAD queries]
-  uint8_t* sdST = sPT + Cfg::P_BYTES;       // dS^T operand
-  float* lse2 = (float*)(sdST + Cfg::P_BYTES);  // [LPAD]
-  float* dlt = lse2 + LPAD;                     // [LPAD]
-  float* tab = dlt + LPAD;                      // [REP2 copies of table[T-2]] ++ [table], log2 domain
-  uint64_t* bars = (uint64_t*)(tab + Cfg::TAB2_FLOATS);
-  uint64_t *qdo_full = bars, *qdo_empty = bars + 1, *kv_full = bars + 2, *kv_empty = bars + 3, *sd_full = bars + 4,
-           *ds_full = bars + 5, *dkv_full = bars + 6, *dkv_empty = bars + 7;
-  uint32_t* tmem_ptr = (uint32_t*)(bars + 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_do);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    mbar_init(qdo_full, 1);
-    mbar_init(qdo_empty, 1);
-    mbar_init(kv_full, 1);
-    mbar_init(kv_empty, 1);
-    mbar_init(sd_full, 1);
-    mbar_init(ds_full, 8);
-    mbar_init(dkv_full, 1);
-    mbar_init(dkv_empty, 8);
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    tmem_alloc(tmem_ptr, 512);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  // dV aliases S^T[0,64); dK starts where dP^T does (or at column 64 when LPAD < 64 so the two outputs do not overlap)
-  constexpr uint32_t TM_S = 0, TM_DP = LPAD, TM_DV = 0, TM_DK = LPAD > 64 ? LPAD : 64;
-
-  const int n_items = a.B * a.H;
-  const int item0 = blockIdx.x * a.items_per_cta;
-  const int item1 = min(n_items, item0 + a.items_per_cta);
-  const int n_tiles = (item1 - item0) * NT;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      for (int tau = 0; tau < n_tiles; ++tau) {
-        const int it = item0 + tau / NT, t = tau % NT;
-        const int h = it / a.B, b = it % a.B;
-        if (t == 0) {
-          mbar_wait_relaxed(qdo_empty, ((uint32_t)(tau / NT) & 1u) ^ 1u);
-          mbar_arrive_expect_tx(qdo_full, 2 * Cfg::KV_BYTES);
-          tma_load_2d(sQ, &map_q, qdo_full, h * TC_HD, b * L);
-          tma_load_2d(sdO, &map_do, qdo_full, h * TC_HD, b * L);
-        }
-        mbar_wait_relaxed(kv_empty, ((uint32_t)tau & 1u) ^ 1u);
-        mbar_arrive_expect_tx(kv_full, 2 * 16384);
-        tma_load_2d(sK, &map_k, kv_full, h * TC_HD, b * L + t * 128);
-        tma_load_2d(sV, &map_v, kv_full, h * TC_HD, b * L + t * 128);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc_bf16(128, LPAD, 0, 0);
-      constexpr uint32_t idesc_o = make_idesc_bf16(128, TC_HD, 0, 1);
-      const uint32_t aQ = smem_u32(sQ), adO = smem_u32(sdO), aK = smem_u32(sK), aV = smem_u32(sV), aPT = smem_u32(sPT),
-                     adST = smem_u32(sdST);
-      for (int tau = 0; tau < n_tiles; ++tau) {
-        const int item = tau / NT, t = tau % NT;
-        if (t == 0) mbar_wait(qdo_full, (uint32_t)item & 1u);
-        mbar_wait(kv_full, (uint32_t)tau & 1u);
-        mbar_wait(dkv_empty, ((uint32_t)tau & 1u) ^ 1u);   // dV / dK of the previous tile read out of the aliased columns
-        tc_fence_after();
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          umma_bf16(tmem_base + TM_S, make_smem_desc(aK + k * 32, 16, 1024), make_smem_desc(aQ + k * 32, 16, 1024), idesc_s,
-                    k > 0 ? 1u : 0u);
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          umma_bf16(tmem_base + TM_DP, make_smem_desc(aV + k * 32, 16, 1024), make_smem_desc(adO + k * 32, 16, 1024), idesc_s,
-                    k > 0 ? 1u : 0u);
-        umma_commit(sd_full);
-        umma_commit(kv_empty);                              // the K / V tile is dead: prefetch the next one
-        mbar_wait(ds_full, (uint32_t)tau & 1u);
-        tc_fence_after();
-#pragma unroll
-        for (int k = 0; k < LPAD / 16; ++k)
-          umma_bf16(tmem_base + TM_DV, make_smem_desc(aPT + (k >> 2) * 16384 + (k & 3) * 32, 16, 1024),
-                    make_smem_desc(adO + k * 2048, 8192, 1024), idesc_o, k > 0 ? 1u : 0u);
-#pragma unroll
-        for (int k = 0; k < LPAD / 16; ++k)
-          umma_bf16(tmem_base + TM_DK, make_smem_desc(adST + (k >> 2) * 16384 + (k & 3) * 32, 16, 1024),
-                    make_smem_desc(aQ + k * 2048, 8192, 1024), idesc_o, k > 0 ? 1u : 0u);
-        umma_commit(dkv_full);
-        if (t == NT - 1) umma_commit(qdo_empty);
-      }
-    }
-    __syncwarp();
-  } else {
-    const int wg = (warp - 2) >> 2;
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const int wgt = threadIdx.x - 64;
-    const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
-    const float scale2 = a.scale * 1.4426950408889634f;
-    uint8_t* myP = sPT + (r >> 3) * 1024 + (r & 7) * 128;
-    uint8_t* myD = sdST + (r >> 3) * 1024 + (r & 7) * 128;
-    const int sw = r & 7;
-    int cur_h = -1, cur_item = -1;
-    for (int tau = 0; tau < n_tiles; ++tau) {
-      const int item = item0 + tau / NT, t = tau % NT;
-      const int h = item / a.B, b = item % a.B;
-      const int key = t * 128 + r;
-      if (item != cur_item) {  // per-item query-side vectors (and, on a head change, the bias table)
-        named_bar_sync(1, 256);
-        const int64_t st = ((int64_t)b * a.H + h) * L;
-        for (int i = wgt; i < LPAD; i += 256) {
-          lse2[i] = i < L ? __ldg(a.lse + st + i) * 1.4426950408889634f : 0.f;
-          dlt[i] = i < L ? __ldg(a.delta + st + i) : 0.f;
-        }
-        if (h != cur_h) {
-          for (int i = wgt; i < Cfg::T; i += 256)
-            tab[Cfg::REP2 + i] = a.table ? __ldg(a.table + (int64_t)i * a.H + h) * 1.4426950408889634f : 0.f;
-          const float k0 = a.table ? __ldg(a.table + (int64_t)(Cfg::T - 2) * a.H + h) * 1.4426950408889634f : 0.f;
-          for (int i = wgt; i < Cfg::REP2; i += 256) tab[i] = k0;
-          cur_h = h;
-        }
-        named_bar_sync(1, 256);
-        cur_item = item;
-      }
-      const int kc = key < L ? key : L - 1;
-      const bool row_ok = key < L;
-      // bias(q, key) = table[base(q) - off(key)]: per-thread pointer, per-column immediate.  key 0 reads the replicated
-      // table[T-2] block through the same immediates; query 0 is the constant table[T-3] (or [T-1] at key 0).
-      const float* kb = kc >= 1 ? tab + Cfg::REP2 - (((kc - 1) / W) * (2 * W - 1) + (kc - 1) % W)
-                                : tab - Cfg::OFFMAX;
-      const float bias_q0 = tab[Cfg::REP2 + (kc >= 1 ? Cfg::T - 3 : Cfg::T - 1)];
-      mbar_wait(sd_full, (uint32_t)tau & 1u);
-      tc_fence_after();
-      const int cb = wg == 0 ? 0 : SPLIT, ce = wg == 0 ? SPLIT : LPAD;
-#pragma unroll
-      for (int cc = 0; cc < LPAD; cc += 32) {
-        if (cc >= (SPLIT > LPAD - SPLIT ? SPLIT : LPAD - SPLIT)) continue;
-        const int c0 = cb + cc;
-        if (c0 >= ce) continue;
-        const bool full = c0 + 32 <= ce;
-        uint32_t vs[32], vp[32];
-        if (full) {
-          tmem_ld_32x32(lane_base + TM_S + c0, vs);
-          tmem_ld_32x32(lane_base + TM_DP + c0, vp);
-        } else {
-          tmem_ld_32x32_16(lane_base + TM_S + c0, vs);
-          tmem_ld_32x32_16(lane_base + TM_DP + c0, vp);
-        }
-        tmem_ld_wait();
-#pragma unroll
-        for (int g8 = 0; g8 < 4; ++g8) {
-          if (!full && g8 >= 2) continue;
-          const int col8 = c0 + g8 * 8;
-          const int off8 = (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4);
-          float pp[8], ds[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) {
-            const int q = c0 + g8 * 8 + e;
-            float bias2, l2q, dq_;
-            if (wg == 0) {
-              const int qc_ = cc + g8 * 8 + e;
-              bias2 = qc_ == 0 ? bias_q0 : *(kb + rel_base<W>(qc_));
-              l2q = lse2[qc_];
-              dq_ = dlt[qc_];
-            } else {
-              const int qc_ = SPLIT + cc + g8 * 8 + e;
-              bias2 = *(kb + rel_base<W>(qc_));
-              l2q = lse2[qc_];
-              dq_ = dlt[qc_];
-            }
-            float p = ex2_approx(fmaf(__uint_as_float(vs[g8 * 8 + e]), scale2, bias2) - l2q);
-            if (q >= L || !row_ok) p = 0.f;
-            pp[e] = p;
-            ds[e] = p * (__uint_as_float(vp[g8 * 8 + e]) - dq_);
-          }
-          st_bf16x8(myP + off8, pp);
-          st_bf16x8(myD + off8, ds);
-        }
-      }
-      fence_proxy_async();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(ds_full);
-      // ---- warpgroup 0 stores dV (aliases S^T[0,64)), warpgroup 1 stores dK * scale (aliases dP^T[0,64))
-      mbar_wait(dkv_full, (uint32_t)tau & 1u);
-      tc_fence_after();
-      uint32_t o[2][32];
-      const uint32_t src = lane_base + (wg == 0 ? TM_DV : TM_DK);
-      tmem_ld_32x32(src, o[0]);
-      tmem_ld_32x32(src + 32, o[1]);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(dkv_empty);
-      if (row_ok) {
-        bf16* dst = wg == 0 ? a.dv + ((int64_t)b * L + key) * a.dv_stride + h * TC_HD
-                            : a.dk + ((int64_t)b * L + key) * a.dk_stride + h * TC_HD;
-        const float mul = wg == 0 ? 1.0f : a.scale;
-#pragma unroll
-        for (int hh = 0; hh < 2; ++hh)
-#pragma unroll
-          for (int e = 0; e < 32; e += 8) {
-            float v[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) v[k] = __uint_as_float(o[hh][e + k]) * mul;
-            st_bf16x8((uint8_t*)(dst + hh * 32 + e), v);
-          }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
-// ================================================================================================ fused backward
-// One kernel for dQ, dK and dV (used when the table gradient comes from the bf16 dS dump, i.e. always in the training step):
-// per query tile S = Q K^T and dP = dO V^T are computed ONCE, the two warpgroups write P and dS to shared memory once, and
-// three products are issued from those buffers — dQ = dS K (dS read K-major), dK = dS^T Q and dV = P^T dO (the same buffers
-// read MN-major: keys become the M dimension, 64-key blocks are 16 KB apart).  The elementwise stage, which bounds these
-// kernels, therefore runs once per (query, key) pair instead of once in a dQ kernel and again in a dK/dV kernel.  The outputs
-// re-use the TMEM columns of S / dP; the second query tile of a (sample, head) adds its dK / dV to the first tile's rows in
-// global memory (same thread, same rows: no synchronisation needed).
-// Samples with more than 208 keys (384 px: W = 24, L = 577; 480 px: W = 30, L = 901) are processed one KEY BLOCK per launch
-// (KeyBlocks: 192 / 192 / 193 keys at 577, 4 x 192 + 133 at 901; scores beyond a block's keys are masked): the backward needs no online softmax — P = 2^(S - lse) with the forward's lse — so a
-// key block is just a narrower K / V operand, an offset into the relative-position index, per-block dK / dV rows, and dQ
-// accumulated across the launches (block 0 stores, later blocks TMA-reduce-add; launches of one stream run in order).
 template <int W>
 struct VitFusedCfg {
   static constexpr int L = W * W + 1;
@@ -1305,7 +762,7 @@ vit_attn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __
 }
 
 // ------------------------------------------------------------------------------------------ host
-static int encode_rows(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems, uint32_t box_rows) {
+int encode_rows(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems, uint32_t box_rows) {
   auto fn = get_tensor_map_encoder();
   if (!fn) return XFM_ERR_NO_DRIVER;
   cuuint64_t dims[2] = {cols, rows};
@@ -1316,15 +773,15 @@ static int encode_rows(CUtensorMap* map, const void* base, uint64_t cols, uint64
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("vit attention: cuTensorMapEncodeTiled failed: %d", (int)r);
+    set_error("attention: cuTensorMapEncodeTiled failed: %d", (int)r);
     return XFM_ERR_BAD_ARG;
   }
   return 0;
 }
 
 // [sample, row, 64-column block] view of a bf16 activation: boxes of 128 rows are clipped at the sample's last row
-static int encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows_per_sample, uint64_t samples,
-                          uint64_t ld_elems, uint64_t sample_stride_rows = 0) {
+int encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows_per_sample, uint64_t samples,
+                   uint64_t ld_elems, uint64_t sample_stride_rows) {
   auto fn = get_tensor_map_encoder();
   if (!fn) return XFM_ERR_NO_DRIVER;
   if (sample_stride_rows == 0) sample_stride_rows = rows_per_sample;   // > rows_per_sample: a row window of every sample
@@ -1336,7 +793,7 @@ static int encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, uin
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("vit attention: cuTensorMapEncodeTiled (3D store map) failed: %d", (int)r);
+    set_error("attention: cuTensorMapEncodeTiled (3D store map) failed: %d", (int)r);
     return XFM_ERR_BAD_ARG;
   }
   return 0;
@@ -1354,7 +811,6 @@ static int window_for(int L, bool bwd = false) {
 
 bool vit_attention_tc_supported(const xfm_attn_params* p, bool bwd) {
   const int w = window_for(p->Lk, bwd || (p->part_out && p->part_lse));   // forward at 24 / 30: needs the key-block scratch
-  if (w * w + 1 > 208 && p->rel_dtable) return false;   // key-blocked shape: fused kernel only (table gradient from the dS dump)
   return p->head_dim == TC_HD && p->Lq == p->Lk && w > 0 && !p->kmask && !p->kv_index &&
          (!p->bias || p->rel_table) && !(p->dropout_p > 0.f) && (p->Bkv == 0 || p->Bkv == p->B) &&
          (p->rel_table == nullptr || p->rel_window == w) &&
@@ -1489,7 +945,7 @@ static int launch_vit_fwd(const xfm_attn_params* p, cudaStream_t s) {
   return launch_merge_parts(Cfg::NB, p->part_out, p->part_lse, p->out, p->o_stride, p->lse, a.B, a.H, Cfg::L, s);
 }
 
-// One fused kernel for dQ, dK and dV (the table gradient, if any, comes from the dS dump); one launch per key block.
+// One launch per key block.
 template <int W, int KB>
 static int launch_vit_bwd_fused_block(const xfm_attn_params* p, const VitBwdArgs& a0, const CUtensorMap& mq1, const CUtensorMap& mdo1,
                                       const CUtensorMap& mk_l, const CUtensorMap& mv_l, const CUtensorMap& m_dq,
@@ -1543,7 +999,7 @@ static int launch_vit_bwd_fused(const xfm_attn_params* p, cudaStream_t s) {
   using FCfg = VitFusedCfg<W>;
   VitBwdArgs a;
   a.prof = nullptr;
-  a.lse = p->lse; a.delta = p->delta; a.table = p->rel_table; a.dtable = nullptr;
+  a.lse = p->lse; a.delta = p->delta; a.table = p->rel_table;
   a.ds_dump = (bf16*)p->ds_dump; a.ds_ld = p->ds_ld;
   a.dq = (bf16*)p->dq; a.dk = (bf16*)p->dk; a.dv = (bf16*)p->dv;
   a.dq_stride = p->dq_stride; a.dk_stride = p->dk_stride; a.dv_stride = p->dv_stride;
@@ -1561,48 +1017,7 @@ static int launch_vit_bwd_fused(const xfm_attn_params* p, cudaStream_t s) {
   return launch_vit_bwd_fused_block<W, 0>(p, a, mq1, mdo1, mk_l, mv_l, m_dq, m_ds, s);
 }
 
-template <int W>
-static int launch_vit_bwd(const xfm_attn_params* p, cudaStream_t s) {
-  using Cfg = VitBwdCfg<W>;
-  VitBwdArgs a;
-  a.prof = nullptr;
-  a.lse = p->lse; a.delta = p->delta; a.table = p->rel_table; a.dtable = p->rel_dtable;
-  a.ds_dump = (bf16*)p->ds_dump; a.ds_ld = p->ds_ld;
-  a.dq = (bf16*)p->dq; a.dk = (bf16*)p->dk; a.dv = (bf16*)p->dv;
-  a.dq_stride = p->dq_stride; a.dk_stride = p->dk_stride; a.dv_stride = p->dv_stride;
-  a.B = p->B; a.H = p->H; a.scale = p->scale;
-  const uint64_t rows = (uint64_t)a.B * Cfg::L, cols = (uint64_t)a.H * TC_HD;
-  CUtensorMap mq_t, mdo_t, mk_l, mv_l, mq_l, mdo_l, mk_t, mv_t;   // _t: 128-row tiles, _l: LPAD rows
-  int rc = encode_rows(&mq_t, p->q, cols, rows, p->q_stride, Cfg::NT * 128);
-  if (!rc) rc = encode_rows(&mdo_t, p->dout, cols, rows, p->do_stride, Cfg::NT * 128);
-  if (!rc) rc = encode_rows(&mk_l, p->k, cols, rows, p->k_stride, Cfg::LPAD);
-  if (!rc) rc = encode_rows(&mv_l, p->v, cols, rows, p->v_stride, Cfg::LPAD);
-  if (!rc) rc = encode_rows(&mq_l, p->q, cols, rows, p->q_stride, Cfg::LPAD);
-  if (!rc) rc = encode_rows(&mdo_l, p->dout, cols, rows, p->do_stride, Cfg::LPAD);
-  if (!rc) rc = encode_rows(&mk_t, p->k, cols, rows, p->k_stride, 128);
-  if (!rc) rc = encode_rows(&mv_t, p->v, cols, rows, p->v_stride, 128);
-  if (rc) return rc;
-  if (!a.dtable) return launch_vit_bwd_fused<W>(p, s);   // table gradient (if any) comes from the dS dump
-  static bool attr = false;
-  if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(vit_attn_bwd_dq_tc_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::DQ_SMEM);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(vit_attn_bwd_dkv_tc_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::DKV_SMEM);
-    if (e != cudaSuccess) return (int)e;
-    attr = true;
-  }
-  const int n_items = a.B * a.H;
-  const int ctas = n_items < num_sms() ? n_items : num_sms();
-  a.items_per_cta = (n_items + ctas - 1) / ctas;
-  const int grid = (n_items + a.items_per_cta - 1) / a.items_per_cta;
-  vit_attn_bwd_dq_tc_kernel<W><<<grid, TC_THREADS, Cfg::DQ_SMEM, s>>>(mq_t, mdo_t, mk_l, mv_l, a);
-  count_launch();
-  vit_attn_bwd_dkv_tc_kernel<W><<<grid, TC_THREADS, Cfg::DKV_SMEM, s>>>(mq_l, mdo_l, mk_t, mv_t, a);
-  count_launch();
-  return (int)cudaGetLastError();
-}
-
-// delta must already be in p->delta (attn_delta_kernel); dq / dk / dv are written, rel_dtable accumulated.
+// delta must already be in p->delta (attn_delta_kernel); dq / dk / dv are written, and dS to ds_dump when it is given.
 int vit_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s) {
   if ((((uintptr_t)p->dout) & 15) || (p->do_stride & 7) || ((p->dq_stride | p->dk_stride | p->dv_stride) & 7) ||
       (((uintptr_t)p->dq | (uintptr_t)p->dk | (uintptr_t)p->dv) & 15)) {
@@ -1612,10 +1027,10 @@ int vit_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s) {
   switch (window_for(p->Lk, true)) {
     case 30: return launch_vit_bwd_fused<30>(p, s);
     case 24: return launch_vit_bwd_fused<24>(p, s);
-    case 14: return launch_vit_bwd<14>(p, s);
-    case 12: return launch_vit_bwd<12>(p, s);
-    case 7: return launch_vit_bwd<7>(p, s);
-    case 4: return launch_vit_bwd<4>(p, s);
+    case 14: return launch_vit_bwd_fused<14>(p, s);
+    case 12: return launch_vit_bwd_fused<12>(p, s);
+    case 7: return launch_vit_bwd_fused<7>(p, s);
+    case 4: return launch_vit_bwd_fused<4>(p, s);
   }
   set_error("vit attention: no tcgen05 instantiation for %d tokens", p->Lk);
   return XFM_ERR_BAD_ARG;

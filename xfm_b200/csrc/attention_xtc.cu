@@ -59,22 +59,6 @@ struct XCfg {
 };
 
 XFM_DEVINL void xt_ld32(uint32_t taddr, uint32_t (&r)[32]) { tmem_ld_32x32(taddr, r); }
-XFM_DEVINL void xt_ld16(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-}
-XFM_DEVINL void xt_named_bar(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
-XFM_DEVINL void xt_st_bf16x8(uint8_t* dst, const float (&p)[8]) {
-  uint4 u;
-  __nv_bfloat162 t0 = __floats2bfloat162_rn(p[0], p[1]), t1 = __floats2bfloat162_rn(p[2], p[3]);
-  __nv_bfloat162 t2 = __floats2bfloat162_rn(p[4], p[5]), t3 = __floats2bfloat162_rn(p[6], p[7]);
-  u.x = *(uint32_t*)&t0; u.y = *(uint32_t*)&t1; u.z = *(uint32_t*)&t2; u.w = *(uint32_t*)&t3;
-  *(uint4*)dst = u;
-}
 
 // One "unit" = (K/V row, head, chunk of <= GMAX samples).  Every role walks the same unit sequence.
 struct XUnit {
@@ -245,7 +229,7 @@ xattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
         for (int c0 = 0; c0 < LPAD; c0 += 32) {
           uint32_t v[32];
           if (c0 + 32 <= LPAD) xt_ld32(t_s + c0, v);
-          else xt_ld16(t_s + c0, v);
+          else tmem_ld_32x32_16(t_s + c0, v);
           tmem_ld_wait();
 #pragma unroll
           for (int e = 0; e < 32; ++e)
@@ -259,7 +243,7 @@ xattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
         uint32_t v[32];
         if (wv) {
           if (c0 + 32 <= LPAD) xt_ld32(t_s + c0, v);
-          else xt_ld16(t_s + c0, v);
+          else tmem_ld_32x32_16(t_s + c0, v);
           tmem_ld_wait();
         }
 #pragma unroll
@@ -286,7 +270,7 @@ xattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
               p[e + 1] = p1;
             }
             const int col8 = c0 + g8 * 8;
-            xt_st_bf16x8(myP + (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4), p);
+            st_bf16x8(myP + (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4), p);
           }
         }
       }
@@ -316,7 +300,7 @@ xattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
             float vv[8];
 #pragma unroll
             for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[hh][e + k]) * inv;
-            xt_st_bf16x8((uint8_t*)(orow + hh * 32 + e), vv);
+            st_bf16x8((uint8_t*)(orow + hh * 32 + e), vv);
           }
         if (a.lse) a.lse[((int64_t)b * a.H + u.h) * LQS + q] = (m + log2f(sum)) * 0.6931471805599453f;
       }
@@ -332,519 +316,13 @@ xattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
 }
 
 
-// ================================================================================================ backward
-// dQ kernel: rows = stacked queries (same slot layout as the forward), one 128-row tile at a time: S = Q K^T and
-// dP = dO V^T into TMEM, the two warpgroups split the key columns, dS = P o (keep * dP / (1-p) - delta) -> shared memory,
-// dQ = dS K (K read MN-major) -> global.
-template <int LQS, int LK, int GMAX>
-__global__ void __launch_bounds__(XT_THREADS, 1)
-xattn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_do,
-                       const __grid_constant__ CUtensorMap map_k, const __grid_constant__ CUtensorMap map_v, const XAttnArgs a) {
-  using Cfg = XCfg<LQS, LK, GMAX>;
-  constexpr int LPAD = Cfg::LPAD, PER_TILE = Cfg::PER_TILE;
-  constexpr int SPLIT = ((LPAD / 2 + 15) / 16) * 16;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  if (smem_u32(smem) & 1023) __trap();
-  uint8_t* sQ = smem;
-  uint8_t* sdO = sQ + Cfg::Q_BYTES;
-  uint8_t* sK = sdO + Cfg::Q_BYTES;
-  uint8_t* sV = sK + Cfg::KV_BYTES;
-  uint8_t* sdS = sV + Cfg::KV_BYTES;
-  uint64_t* bars = (uint64_t*)(sdS + Cfg::P_BYTES);
-  uint64_t *in_full = bars, *in_empty = bars + 1, *k_full = bars + 2, *k_empty = bars + 3, *sd_full = bars + 4,
-           *ds_full = bars + 5, *dq_full = bars + 6, *dq_empty = bars + 7;
-  uint32_t* tmem_ptr = (uint32_t*)(bars + 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < 2 * Cfg::Q_BYTES / 16; i += blockDim.x) ((uint4*)sQ)[i] = make_uint4(0u, 0u, 0u, 0u);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_do);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    mbar_init(in_full, 1);
-    mbar_init(in_empty, 1);
-    mbar_init(k_full, 1);
-    mbar_init(k_empty, 1);
-    mbar_init(sd_full, 1);
-    mbar_init(ds_full, 8);
-    mbar_init(dq_full, 1);
-    mbar_init(dq_empty, 8);
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    tmem_alloc(tmem_ptr, 512);
-    tmem_relinquish();
-  }
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  constexpr uint32_t TM_S = 0, TM_DP = LPAD, TM_DQ = 2 * LPAD;
-
-  const int n_items = a.Bkv * a.H;
-  const int item0 = blockIdx.x * a.items_per_cta;
-  const int item1 = min(n_items, item0 + a.items_per_cta);
-
-  if (warp == 0) {
-    if (lane == 0) {
-      XWalker<GMAX> w(a, item0, item1);
-      XUnit u;
-      uint32_t ph = 0;
-      while (w.next(u)) {
-        mbar_wait_relaxed(in_empty, ph ^ 1);
-        mbar_arrive_expect_tx(in_full, 2 * u.ns * LQS * 128 + Cfg::KV_BYTES);
-        for (int g = 0; g < u.ns; ++g) {
-          const int b = a.kv_samples[u.first + g];
-          const int o = (g & 1) * 16384 + (g >> 1) * (LQS * 128);
-          tma_load_2d(sQ + o, &map_q, in_full, u.h * XT_HD, b * LQS);
-          tma_load_2d(sdO + o, &map_do, in_full, u.h * XT_HD, b * LQS);
-        }
-        tma_load_2d(sV, &map_v, in_full, u.h * XT_HD, u.r * LK);
-        mbar_wait_relaxed(k_empty, ph ^ 1);
-        mbar_arrive_expect_tx(k_full, Cfg::KV_BYTES);
-        tma_load_2d(sK, &map_k, k_full, u.h * XT_HD, u.r * LK);
-        ph ^= 1;
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc_bf16(128, LPAD, 0, 0);
-      constexpr uint32_t idesc_o = make_idesc_bf16(128, XT_HD, 0, 1);
-      const uint32_t aQ = smem_u32(sQ), adO = smem_u32(sdO), aK = smem_u32(sK), aV = smem_u32(sV), adS = smem_u32(sdS);
-      XWalker<GMAX> w(a, item0, item1);
-      XUnit u;
-      uint32_t ph = 0, tp = 0;   // unit parity; tile parity (sd_full / ds_full / dq_full / dq_empty complete once per tile)
-      while (w.next(u)) {
-        mbar_wait(in_full, ph);
-        mbar_wait(k_full, ph);
-        for (int t = 0; t < 2; ++t) {
-          tc_fence_after();
-          // S / dP of the previous tile were drained before its dS was published (ds_full waited below)
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_base + TM_S, make_smem_desc(aQ + t * 16384 + k * 32, 16, 1024), make_smem_desc(aK + k * 32, 16, 1024),
-                      idesc_s, k > 0 ? 1u : 0u);
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_base + TM_DP, make_smem_desc(adO + t * 16384 + k * 32, 16, 1024), make_smem_desc(aV + k * 32, 16, 1024),
-                      idesc_s, k > 0 ? 1u : 0u);
-          umma_commit(sd_full);
-          if (t == 1) umma_commit(in_empty);
-          mbar_wait(ds_full, tp);
-          mbar_wait(dq_empty, tp ^ 1);
-          tc_fence_after();
-#pragma unroll
-          for (int k = 0; k < LPAD / 16; ++k)
-            umma_bf16(tmem_base + TM_DQ, make_smem_desc(adS + (k >> 2) * 16384 + (k & 3) * 32, 16, 1024),
-                      make_smem_desc(aK + k * 2048, 8192, 1024), idesc_o, k > 0 ? 1u : 0u);
-          umma_commit(dq_full);
-          if (t == 1) umma_commit(k_empty);
-          tp ^= 1;
-        }
-        ph ^= 1;
-      }
-    }
-    __syncwarp();
-  } else {
-    const int wg = (warp - 2) >> 2;
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const int slot_in_tile = r / LQS, q = r % LQS;
-    const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
-    const float scale2 = a.scale * 1.4426950408889634f;
-    const bool drop_on = a.dropout_p > 0.f;
-    const float inv_keep = drop_on ? 1.0f / (1.0f - a.dropout_p) : 1.0f;
-    const uint32_t seed_mix = drop_seed_mix(a.seed + *a.salt), thr = drop_threshold(a.dropout_p);
-    uint8_t* myS = sdS + (r >> 3) * 1024 + (r & 7) * 128;
-    const int sw = r & 7;
-    const int cb = wg == 0 ? 0 : SPLIT, ce = wg == 0 ? SPLIT : LPAD;
-    constexpr int LKE = (LK + 1) & ~1;
-    XWalker<GMAX> w(a, item0, item1);
-    XUnit u;
-    uint32_t tp = 0;
-    while (w.next(u)) {
-#pragma unroll 1
-      for (int t = 0; t < 2; ++t) {
-        const int g = 2 * slot_in_tile + t;
-        const bool valid = slot_in_tile < PER_TILE && g < u.ns;
-        const bool wv = __any_sync(0xffffffffu, valid);
-        const int b = valid ? a.kv_samples[u.first + g] : 0;
-        const int64_t st_row = ((int64_t)b * a.H + u.h) * LQS + q;
-        const float lse2 = valid ? __ldg(a.lse + st_row) * 1.4426950408889634f : 0.f;
-        const float dl = valid ? __ldg(a.delta + st_row) : 0.f;
-        const uint64_t pair_base = ((uint64_t)st_row * (uint64_t)LKE) >> 1;
-        const uint32_t pb_lo = (uint32_t)pair_base, pb_hi = (uint32_t)(pair_base >> 32);
-        mbar_wait(sd_full, tp);
-        tc_fence_after();
-#pragma unroll 1
-        for (int c0 = cb; c0 < ce; c0 += 32) {
-          const bool full = c0 + 32 <= ce;
-          uint32_t vs[32], vp[32];
-          if (wv) {
-            if (full) {
-              xt_ld32(lane_base + TM_S + c0, vs);
-              xt_ld32(lane_base + TM_DP + c0, vp);
-            } else {
-              xt_ld16(lane_base + TM_S + c0, vs);
-              xt_ld16(lane_base + TM_DP + c0, vp);
-            }
-            tmem_ld_wait();
-          }
-#pragma unroll
-          for (int g8 = 0; g8 < 4; ++g8) {
-            if (!full && g8 >= 2) continue;
-            float ds[8];
-#pragma unroll
-            for (int e = 0; e < 8; e += 2) {
-              const int j = c0 + g8 * 8 + e;   // even
-              float d0 = 0.f, d1 = 0.f;
-              if (valid && j < LK) {
-                const float p0 = ex2_approx(fmaf(__uint_as_float(vs[g8 * 8 + e]), scale2, -lse2));
-                const float p1 = j + 1 < LK ? ex2_approx(fmaf(__uint_as_float(vs[g8 * 8 + e + 1]), scale2, -lse2)) : 0.f;
-                float dp0 = __uint_as_float(vp[g8 * 8 + e]), dp1 = __uint_as_float(vp[g8 * 8 + e + 1]);
-                if (drop_on) {
-                  const uint32_t lo = pb_lo + (uint32_t)(j >> 1);
-                  const uint32_t keep = drop_keep_pair(seed_mix, lo, pb_hi + (lo < pb_lo ? 1u : 0u), thr);
-                  dp0 = (keep & 1u) ? dp0 * inv_keep : 0.f;
-                  dp1 = (keep & 2u) ? dp1 * inv_keep : 0.f;
-                }
-                d0 = p0 * (dp0 - dl);
-                d1 = p1 * (dp1 - dl);
-              }
-              ds[e] = d0;
-              ds[e + 1] = d1;
-            }
-            const int col8 = c0 + g8 * 8;
-            xt_st_bf16x8(myS + (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4), ds);
-          }
-        }
-        fence_proxy_async();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(ds_full);
-        mbar_wait(dq_full, tp);
-        tc_fence_after();
-        uint32_t o[32];
-        if (wv) {
-          tmem_ld_32x32(lane_base + TM_DQ + wg * 32, o);
-          tmem_ld_wait();
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(dq_empty);
-        if (valid) {
-          bf16* dst = a.dq + ((int64_t)b * LQS + q) * a.dq_stride + u.h * XT_HD + wg * 32;
-#pragma unroll
-          for (int e = 0; e < 32; e += 8) {
-            float vv[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[e + k]) * a.scale;
-            xt_st_bf16x8((uint8_t*)(dst + e), vv);
-          }
-        }
-        tp ^= 1;
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
-// dK / dV kernel: rows = keys (two 128-key tiles per image), columns = the stacked queries of the chunk (slot g -> columns
-// [g LQS, (g+1) LQS)).  S^T = K Q^T, dP^T = V dO^T; P^T (with the dropout mask and 1/(1-p)) and dS^T go to shared memory as
-// the A operands of dV = P^T dO and dK = dS^T Q, which sum over ALL samples that reference the image in one MMA chain.
-template <int LQS, int LK, int GMAX>
-struct XDkvCfg : XCfg<LQS, LK, GMAX> {
-  static constexpr int NQ = GMAX * LQS;                     // stacked query columns (multiple of 16)
-  static_assert(NQ % 16 == 0 && NQ <= 256, "stacked queries must form a legal MMA N");
-  static constexpr int QC_BYTES = NQ * 128;
-  static constexpr int NQB = (NQ + 63) / 64;
-  static constexpr int PT_BYTES = NQB * 16384;
-  static constexpr int SMEM = 2 * 16384 + 2 * QC_BYTES + 2 * PT_BYTES + 4 * NQ * 4 + 128;
-  static_assert(2 * NQ <= 512, "TMEM");
-};
-
-template <int LQS, int LK, int GMAX>
-__global__ void __launch_bounds__(XT_THREADS, 1)
-xattn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_do,
-                        const __grid_constant__ CUtensorMap map_k, const __grid_constant__ CUtensorMap map_v, const XAttnArgs a) {
-  using Cfg = XDkvCfg<LQS, LK, GMAX>;
-  constexpr int NQ = Cfg::NQ;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  if (smem_u32(smem) & 1023) __trap();
-  uint8_t* sK = smem;
-  uint8_t* sV = sK + 16384;
-  uint8_t* sQ = sV + 16384;                  // NQ stacked query rows
-  uint8_t* sdO = sQ + Cfg::QC_BYTES;
-  uint8_t* sPT = sdO + Cfg::QC_BYTES;
-  uint8_t* sdST = sPT + Cfg::PT_BYTES;
-  float* lse2 = (float*)(sdST + Cfg::PT_BYTES);   // per stacked query column
-  float* dlt = lse2 + NQ;
-  uint32_t* pbl = (uint32_t*)(dlt + NQ);          // dropout pair base of the column's (b, h, q) row, low / high words
-  uint32_t* pbh = pbl + NQ;
-  uint64_t* bars = (uint64_t*)(pbh + NQ);
-  uint64_t *qdo_full = bars, *qdo_empty = bars + 1, *kv_full = bars + 2, *kv_empty = bars + 3, *sd_full = bars + 4,
-           *ds_full = bars + 5, *dkv_full = bars + 6, *dkv_empty = bars + 7;
-  uint32_t* tmem_ptr = (uint32_t*)(bars + 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < 2 * Cfg::QC_BYTES / 16; i += blockDim.x) ((uint4*)sQ)[i] = make_uint4(0u, 0u, 0u, 0u);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_do);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    mbar_init(qdo_full, 1);
-    mbar_init(qdo_empty, 1);
-    mbar_init(kv_full, 1);
-    mbar_init(kv_empty, 1);
-    mbar_init(sd_full, 1);
-    mbar_init(ds_full, 8);
-    mbar_init(dkv_full, 1);
-    mbar_init(dkv_empty, 8);
-    fence_barrier_init();
-  }
-  if (warp == 1) {
-    tmem_alloc(tmem_ptr, 512);
-    tmem_relinquish();
-  }
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  constexpr uint32_t TM_S = 0, TM_DP = NQ, TM_DV = 0, TM_DK = NQ > 64 ? NQ : 64;
-
-  const int n_items = a.Bkv * a.H;
-  const int item0 = blockIdx.x * a.items_per_cta;
-  const int item1 = min(n_items, item0 + a.items_per_cta);
-
-  if (warp == 0) {
-    if (lane == 0) {
-      XWalker<GMAX> w(a, item0, item1);
-      XUnit u;
-      uint32_t ph = 0, tp = 0;
-      while (w.next(u)) {
-        mbar_wait_relaxed(qdo_empty, ph ^ 1);
-        mbar_arrive_expect_tx(qdo_full, 2 * u.ns * LQS * 128);
-        for (int g = 0; g < u.ns; ++g) {
-          const int b = a.kv_samples[u.first + g];
-          tma_load_2d(sQ + g * (LQS * 128), &map_q, qdo_full, u.h * XT_HD, b * LQS);
-          tma_load_2d(sdO + g * (LQS * 128), &map_do, qdo_full, u.h * XT_HD, b * LQS);
-        }
-        for (int t = 0; t < 2; ++t) {
-          mbar_wait_relaxed(kv_empty, tp ^ 1);
-          mbar_arrive_expect_tx(kv_full, 2 * 16384);
-          tma_load_2d(sK, &map_k, kv_full, u.h * XT_HD, u.r * LK + t * 128);
-          tma_load_2d(sV, &map_v, kv_full, u.h * XT_HD, u.r * LK + t * 128);
-          tp ^= 1;
-        }
-        ph ^= 1;
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc_bf16(128, NQ, 0, 0);
-      constexpr uint32_t idesc_o = make_idesc_bf16(128, XT_HD, 0, 1);
-      const uint32_t aQ = smem_u32(sQ), adO = smem_u32(sdO), aK = smem_u32(sK), aV = smem_u32(sV), aPT = smem_u32(sPT),
-                     adST = smem_u32(sdST);
-      XWalker<GMAX> w(a, item0, item1);
-      XUnit u;
-      uint32_t ph = 0, tp = 0;
-      while (w.next(u)) {
-        const int nk = (u.ns * LQS + 15) / 16;   // k-steps of the output MMAs: only the valid stacked queries
-        mbar_wait(qdo_full, ph);
-        for (int t = 0; t < 2; ++t) {
-          mbar_wait(kv_full, tp);
-          mbar_wait(dkv_empty, tp ^ 1);
-          tc_fence_after();
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_base + TM_S, make_smem_desc(aK + k * 32, 16, 1024), make_smem_desc(aQ + k * 32, 16, 1024), idesc_s,
-                      k > 0 ? 1u : 0u);
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_base + TM_DP, make_smem_desc(aV + k * 32, 16, 1024), make_smem_desc(adO + k * 32, 16, 1024), idesc_s,
-                      k > 0 ? 1u : 0u);
-          umma_commit(sd_full);
-          umma_commit(kv_empty);
-          mbar_wait(ds_full, tp);
-          tc_fence_after();
-          for (int k = 0; k < nk; ++k)
-            umma_bf16(tmem_base + TM_DV, make_smem_desc(aPT + (k >> 2) * 16384 + (k & 3) * 32, 16, 1024),
-                      make_smem_desc(adO + k * 2048, 8192, 1024), idesc_o, k > 0 ? 1u : 0u);
-          for (int k = 0; k < nk; ++k)
-            umma_bf16(tmem_base + TM_DK, make_smem_desc(adST + (k >> 2) * 16384 + (k & 3) * 32, 16, 1024),
-                      make_smem_desc(aQ + k * 2048, 8192, 1024), idesc_o, k > 0 ? 1u : 0u);
-          umma_commit(dkv_full);
-          if (t == 1) umma_commit(qdo_empty);
-          tp ^= 1;
-        }
-        ph ^= 1;
-      }
-    }
-    __syncwarp();
-  } else {
-    const int wg = (warp - 2) >> 2;
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const int wgt = threadIdx.x - 64;
-    const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
-    const float scale2 = a.scale * 1.4426950408889634f;
-    const bool drop_on = a.dropout_p > 0.f;
-    const float inv_keep = drop_on ? 1.0f / (1.0f - a.dropout_p) : 1.0f;
-    const uint32_t seed_mix = drop_seed_mix(a.seed + *a.salt), thr = drop_threshold(a.dropout_p);
-    uint8_t* myP = sPT + (r >> 3) * 1024 + (r & 7) * 128;
-    uint8_t* myD = sdST + (r >> 3) * 1024 + (r & 7) * 128;
-    const int sw = r & 7;
-    constexpr int LKE = (LK + 1) & ~1;
-    XWalker<GMAX> w(a, item0, item1);
-    XUnit u;
-    uint32_t tp = 0;
-    int chunk_of_item = 0, cur_it = -1;
-    while (w.next(u)) {
-      const int it_id = u.h * a.Bkv + u.r;
-      chunk_of_item = (it_id == cur_it) ? chunk_of_item + 1 : 0;
-      cur_it = it_id;
-      const int ncols = u.ns * LQS;
-      const int nkc = (ncols + 15) / 16 * 16;                 // columns read by the output MMAs
-      const int half = ((nkc / 2 + 15) / 16) * 16;
-      const int cb = wg == 0 ? 0 : half, ce = wg == 0 ? half : nkc;
-      // per-column vectors of this unit (both warpgroups; the previous unit's readers are all past their last tile)
-      xt_named_bar(1, 256);
-      for (int c = wgt; c < NQ; c += 256) {
-        const int g = c / LQS, qq = c % LQS;
-        float l = 0.f, d = 0.f;
-        uint64_t pb = 0;
-        if (g < u.ns) {
-          const int b = a.kv_samples[u.first + g];
-          const int64_t st = ((int64_t)b * a.H + u.h) * LQS + qq;
-          l = __ldg(a.lse + st) * 1.4426950408889634f;
-          d = __ldg(a.delta + st);
-          pb = (uint64_t)st * (uint64_t)LKE;   // element index of key 0 in that (b, h, q) row (even)
-        }
-        lse2[c] = l;
-        dlt[c] = d;
-        pbl[c] = (uint32_t)pb;
-        pbh[c] = (uint32_t)(pb >> 32);
-      }
-      xt_named_bar(1, 256);
-#pragma unroll 1
-      for (int t = 0; t < 2; ++t) {
-        const int key = t * 128 + r;
-        const bool row_ok = key < LK;
-        mbar_wait(sd_full, tp);
-        tc_fence_after();
-#pragma unroll 1
-        for (int c0 = cb; c0 < ce; c0 += 32) {
-          const bool full = c0 + 32 <= ce;
-          uint32_t vs[32], vp[32];
-          if (full) {
-            xt_ld32(lane_base + TM_S + c0, vs);
-            xt_ld32(lane_base + TM_DP + c0, vp);
-          } else {
-            xt_ld16(lane_base + TM_S + c0, vs);
-            xt_ld16(lane_base + TM_DP + c0, vp);
-          }
-          tmem_ld_wait();
-#pragma unroll
-          for (int g8 = 0; g8 < 4; ++g8) {
-            if (!full && g8 >= 2) continue;
-            float pp[8], ds[8];
-#pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              const int c = c0 + g8 * 8 + e;
-              float p = 0.f, dpe = __uint_as_float(vp[g8 * 8 + e]);
-              if (row_ok && c < ncols) {
-                p = ex2_approx(fmaf(__uint_as_float(vs[g8 * 8 + e]), scale2, -lse2[c]));
-                if (drop_on) {
-                  // element index = row base (even) + key: pair = (base + key) >> 1, half selected by the key's parity
-                  const uint32_t lo0 = pbl[c];
-                  const uint32_t lo1 = lo0 + (uint32_t)key;
-                  const uint32_t hi1 = pbh[c] + (lo1 < lo0 ? 1u : 0u);
-                  const uint32_t keep = drop_keep_pair(seed_mix, (lo1 >> 1) | (hi1 << 31), hi1 >> 1, thr);
-                  const bool k1 = (key & 1) ? (keep & 2u) != 0u : (keep & 1u) != 0u;
-                  const float km = k1 ? inv_keep : 0.f;
-                  dpe *= km;
-                  pp[e] = p * km;
-                } else {
-                  pp[e] = p;
-                }
-                ds[e] = p * (dpe - dlt[c]);
-              } else {
-                pp[e] = 0.f;
-                ds[e] = 0.f;
-              }
-            }
-            const int col8 = c0 + g8 * 8;
-            const int off8 = (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4);
-            xt_st_bf16x8(myP + off8, pp);
-            xt_st_bf16x8(myD + off8, ds);
-          }
-        }
-        fence_proxy_async();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(ds_full);
-        mbar_wait(dkv_full, tp);
-        tc_fence_after();
-        uint32_t o[2][32];
-        const uint32_t src = lane_base + (wg == 0 ? TM_DV : TM_DK);
-        tmem_ld_32x32(src, o[0]);
-        tmem_ld_32x32(src + 32, o[1]);
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(dkv_empty);
-        if (row_ok) {
-          bf16* dst = wg == 0 ? a.dv + ((int64_t)u.r * LK + key) * a.dv_stride + u.h * XT_HD
-                              : a.dk + ((int64_t)u.r * LK + key) * a.dk_stride + u.h * XT_HD;
-          const float mul = wg == 0 ? 1.0f : a.scale;
-#pragma unroll
-          for (int hh = 0; hh < 2; ++hh)
-#pragma unroll
-            for (int e = 0; e < 32; e += 8) {
-              float vv[8];
-#pragma unroll
-              for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[hh][e + k]) * mul;
-              if (chunk_of_item > 0) {   // image referenced by more than GMAX samples: add to the earlier chunks' result
-                const uint4 prev = *(const uint4*)(dst + hh * 32 + e);
-                const __nv_bfloat162* ph2 = (const __nv_bfloat162*)&prev;
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const float2 f = __bfloat1622float2(ph2[k]);
-                  vv[2 * k] += f.x;
-                  vv[2 * k + 1] += f.y;
-                }
-              }
-              xt_st_bf16x8((uint8_t*)(dst + hh * 32 + e), vv);
-            }
-        }
-        tp ^= 1;
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
 // ================================================================================================ fused backward
 // One kernel for dQ, dK and dV.  A unit is (image, head, chunk of <= 3 samples): ONE 128-row query tile (three 40-row slots).
 // S = Q K^T and dP = dO V^T are computed once, P~ (dropout mask and 1/(1-p) applied) and dS are written to shared memory
 // once, and dQ = dS K (dS read K-major), dK = dS^T Q, dV = P~^T dO (the same buffers read MN-major, keys as the M dimension
-// in two 128-key tiles) are issued from them into the TMEM columns S / dP occupied.  The elementwise stage runs once per
-// (query, key) pair instead of once in a dQ and once more in a dK/dV kernel.  Later chunks of the same image add their
-// dK / dV to the rows the first chunk stored (same CTA, same thread per row: ordered without synchronisation).
+// in two 128-key tiles) are issued from them into the TMEM columns S / dP occupied, so the elementwise stage runs once per
+// (query, key) pair.  Later chunks of the same image add their dK / dV to the rows the first chunk stored (same CTA, same
+// thread per row: ordered without synchronisation).
 template <int LQS, int LK>
 struct XFusedCfg {
   static constexpr int GMAX = 3;
@@ -1057,8 +535,8 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
         const int c0 = ch * 16;
         uint32_t vs[32], vp[32];                 // [0..15] used
         if (wv) {   // tcgen05.ld is warp-collective: decide per warp, mask per thread
-          xt_ld16(lane_base + TM_S + c0, vs);
-          xt_ld16(lane_base + TM_DP + c0, vp);
+          tmem_ld_32x32_16(lane_base + TM_S + c0, vs);
+          tmem_ld_32x32_16(lane_base + TM_DP + c0, vp);
           tmem_ld_wait();
         }
 #pragma unroll
@@ -1090,8 +568,8 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
           }
           const int col8 = c0 + g8 * 8;
           const int off8 = (col8 >> 6) * 16384 + ((((col8 & 63) >> 3) ^ sw) << 4);
-          xt_st_bf16x8(myS + off8, ds);
-          xt_st_bf16x8(myP + off8, pp);
+          st_bf16x8(myS + off8, ds);
+          st_bf16x8(myP + off8, pp);
         }
       }
       fence_proxy_async();
@@ -1133,7 +611,7 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
           float vv[8];
 #pragma unroll
           for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[e + k]) * mul;
-          xt_st_bf16x8(row + (((half * 4 + (e >> 3)) ^ sw) << 4), vv);
+          st_bf16x8(row + (((half * 4 + (e >> 3)) ^ sw) << 4), vv);
         }
       }
       tc_fence_before();                         // every TMEM read of this warp is complete (tcgen05.wait::ld above)
@@ -1175,48 +653,13 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
 }
 
 // ------------------------------------------------------------------------------------------ host
-static int xt_encode_rows(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems, uint32_t box_rows) {
-  auto fn = get_tensor_map_encoder();
-  if (!fn) return XFM_ERR_NO_DRIVER;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld_elems * 2};
-  cuuint32_t box[2] = {XT_HD, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cross attention: cuTensorMapEncodeTiled failed: %d", (int)r);
-    return XFM_ERR_BAD_ARG;
-  }
-  return 0;
-}
-
-// [image, key, 64-column block] view of dK / dV: boxes of 128 keys are clipped at the image's last key
-static int xt_encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows_per_sample, uint64_t samples,
-                             uint64_t ld_elems, uint64_t sample_stride_rows = 0) {
-  auto fn = get_tensor_map_encoder();
-  if (!fn) return XFM_ERR_NO_DRIVER;
-  if (sample_stride_rows == 0) sample_stride_rows = rows_per_sample;   // > rows_per_sample: a row window of every image
-  cuuint64_t dims[3] = {cols, rows_per_sample, samples};
-  cuuint64_t strides[2] = {ld_elems * 2, sample_stride_rows * ld_elems * 2};
-  cuuint32_t box[3] = {XT_HD, 128, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cross attention: cuTensorMapEncodeTiled (3D store map) failed: %d", (int)r);
-    return XFM_ERR_BAD_ARG;
-  }
-  return 0;
-}
-
 // Instantiated shapes: 40 text tokens attending to 197 image tokens (BASELINE configs[1]), up to 6 samples per chunk; and
-// to 577 / 901 image tokens (384 / 480 px) in key blocks: the forward needs the part scratch, the backward has no dS dump.
+// to 577 / 901 image tokens (384 / 480 px) in key blocks, where the forward needs the part scratch.  The backward writes no
+// dS dump.
 bool cross_attention_tc_supported(const xfm_attn_params* p, bool bwd) {
   const bool blocked = p->Lk == 577 || p->Lk == 901;
-  return p->head_dim == XT_HD && p->Lq == 40 && (p->Lk == 197 || (blocked && (bwd ? !p->ds_dump : (p->part_out && p->part_lse)))) && !p->kmask && !p->bias && p->kv_offsets && p->kv_samples &&
+  return p->head_dim == XT_HD && p->Lq == 40 && (p->Lk == 197 || blocked) &&
+         (bwd ? !p->ds_dump : (!blocked || (p->part_out && p->part_lse))) && !p->kmask && !p->bias && p->kv_offsets && p->kv_samples &&
          p->Bkv > 0 && ((uintptr_t)p->q & 15) == 0 && ((uintptr_t)p->k & 15) == 0 && ((uintptr_t)p->v & 15) == 0 &&
          ((p->q_stride | p->k_stride | p->v_stride | p->o_stride) & 7) == 0;
 }
@@ -1267,9 +710,9 @@ static int xt_launch_fwd(const xfm_attn_params* p, cudaStream_t s) {
   xt_fill(p, a);
   const uint64_t cols = (uint64_t)a.H * XT_HD;
   CUtensorMap mq, mk, mv;
-  int rc = xt_encode_rows(&mq, p->q, cols, (uint64_t)a.B * LQS, p->q_stride, LQS);
-  if (!rc) rc = xt_encode_rows(&mk, p->k, cols, (uint64_t)a.Bkv * LK, p->k_stride, Cfg::LPAD);
-  if (!rc) rc = xt_encode_rows(&mv, p->v, cols, (uint64_t)a.Bkv * LK, p->v_stride, Cfg::LPAD);
+  int rc = encode_rows(&mq, p->q, cols, (uint64_t)a.B * LQS, p->q_stride, LQS);
+  if (!rc) rc = encode_rows(&mk, p->k, cols, (uint64_t)a.Bkv * LK, p->k_stride, Cfg::LPAD);
+  if (!rc) rc = encode_rows(&mv, p->v, cols, (uint64_t)a.Bkv * LK, p->v_stride, Cfg::LPAD);
   if (rc) return rc;
   rc = xt_launch_fwd_block<LQS, LK, GMAX, 0>(p, a, mq, mk, mv, s);
   if (rc || !Cfg::BLOCKED) return rc;
@@ -1299,8 +742,8 @@ static int xt_launch_fused_block(const xfm_attn_params* p, const XAttnArgs& a, c
   }
   const uint64_t cols = (uint64_t)a.H * XT_HD;
   CUtensorMap m_dk, m_dv;   // this block's key rows of every image
-  int rc = xt_encode_rows_3d(&m_dk, (const bf16*)p->dk + (int64_t)K0 * p->dk_stride, cols, KLEN, a.Bkv, p->dk_stride, LK);
-  if (!rc) rc = xt_encode_rows_3d(&m_dv, (const bf16*)p->dv + (int64_t)K0 * p->dv_stride, cols, KLEN, a.Bkv, p->dv_stride, LK);
+  int rc = encode_rows_3d(&m_dk, (const bf16*)p->dk + (int64_t)K0 * p->dk_stride, cols, KLEN, a.Bkv, p->dk_stride, LK);
+  if (!rc) rc = encode_rows_3d(&m_dv, (const bf16*)p->dv + (int64_t)K0 * p->dv_stride, cols, KLEN, a.Bkv, p->dv_stride, LK);
   if (rc) return rc;
   const int n_items_f = a.Bkv * a.H;
   const int grid_f = (n_items_f + a.items_per_cta - 1) / a.items_per_cta;
@@ -1319,59 +762,26 @@ static int xt_launch_fused(const xfm_attn_params* p, cudaStream_t s) {
   xt_fill(p, a);
   const uint64_t cols = (uint64_t)a.H * XT_HD;
   CUtensorMap mq, mdo, mk_l, mv_l, m_dq;
-  int rc = xt_encode_rows(&mq, p->q, cols, (uint64_t)a.B * LQS, p->q_stride, LQS);
-  if (!rc) rc = xt_encode_rows(&mdo, p->dout, cols, (uint64_t)a.B * LQS, p->do_stride, LQS);
-  if (!rc) rc = xt_encode_rows(&mk_l, p->k, cols, (uint64_t)a.Bkv * LK, p->k_stride, FCfg::LPAD);
-  if (!rc) rc = xt_encode_rows(&mv_l, p->v, cols, (uint64_t)a.Bkv * LK, p->v_stride, FCfg::LPAD);
-  if (!rc) rc = xt_encode_rows(&m_dq, p->dq, cols, (uint64_t)a.B * LQS, p->dq_stride, LQS);
+  int rc = encode_rows(&mq, p->q, cols, (uint64_t)a.B * LQS, p->q_stride, LQS);
+  if (!rc) rc = encode_rows(&mdo, p->dout, cols, (uint64_t)a.B * LQS, p->do_stride, LQS);
+  if (!rc) rc = encode_rows(&mk_l, p->k, cols, (uint64_t)a.Bkv * LK, p->k_stride, FCfg::LPAD);
+  if (!rc) rc = encode_rows(&mv_l, p->v, cols, (uint64_t)a.Bkv * LK, p->v_stride, FCfg::LPAD);
+  if (!rc) rc = encode_rows(&m_dq, p->dq, cols, (uint64_t)a.B * LQS, p->dq_stride, LQS);
   if (rc) return rc;
   return xt_launch_fused_block<LQS, LK, 0>(p, a, mq, mdo, mk_l, mv_l, m_dq, s);
 }
 
 int cross_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s) {
-  constexpr int LQS = 40, LK = 197, GMAX = 6;
-  using Cfg = XCfg<LQS, LK, GMAX>;
-  using DCfg = XDkvCfg<LQS, LK, GMAX>;
   if ((((uintptr_t)p->dout | (uintptr_t)p->dq | (uintptr_t)p->dk | (uintptr_t)p->dv) & 15) ||
       ((p->do_stride | p->dq_stride | p->dk_stride | p->dv_stride) & 7)) {
     set_error("cross attention bwd: operands must be 16-byte aligned with row strides that are multiples of 8");
     return XFM_ERR_BAD_ARG;
   }
-  if (!p->ds_dump) {   // one fused kernel
-    switch (p->Lk) {
-      case 577: return xt_launch_fused<LQS, 577>(p, s);
-      case 901: return xt_launch_fused<LQS, 901>(p, s);
-    }
-    return xt_launch_fused<LQS, LK>(p, s);
+  switch (p->Lk) {
+    case 577: return xt_launch_fused<40, 577>(p, s);
+    case 901: return xt_launch_fused<40, 901>(p, s);
   }
-  XAttnArgs a;
-  xt_fill(p, a);
-  const uint64_t cols = (uint64_t)a.H * XT_HD;
-  CUtensorMap mq, mdo, mk_l, mv_l, mk_t, mv_t;
-  int rc = xt_encode_rows(&mq, p->q, cols, (uint64_t)a.B * LQS, p->q_stride, LQS);
-  if (!rc) rc = xt_encode_rows(&mdo, p->dout, cols, (uint64_t)a.B * LQS, p->do_stride, LQS);
-  if (!rc) rc = xt_encode_rows(&mk_l, p->k, cols, (uint64_t)a.Bkv * LK, p->k_stride, Cfg::LPAD);
-  if (!rc) rc = xt_encode_rows(&mv_l, p->v, cols, (uint64_t)a.Bkv * LK, p->v_stride, Cfg::LPAD);
-  if (!rc) rc = xt_encode_rows(&mk_t, p->k, cols, (uint64_t)a.Bkv * LK, p->k_stride, 128);
-  if (!rc) rc = xt_encode_rows(&mv_t, p->v, cols, (uint64_t)a.Bkv * LK, p->v_stride, 128);
-  if (rc) return rc;
-  constexpr int DQ_SMEM = 2 * Cfg::Q_BYTES + 2 * Cfg::KV_BYTES + Cfg::P_BYTES + 128;
-  auto kdq = xattn_bwd_dq_tc_kernel<LQS, LK, GMAX>;
-  auto kdkv = xattn_bwd_dkv_tc_kernel<LQS, LK, GMAX>;
-  static bool attr = false;
-  if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(kdq, cudaFuncAttributeMaxDynamicSharedMemorySize, DQ_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(kdkv, cudaFuncAttributeMaxDynamicSharedMemorySize, DCfg::SMEM);
-    if (e != cudaSuccess) return (int)e;
-    attr = true;
-  }
-  const int n_items = a.Bkv * a.H;
-  const int grid = (n_items + a.items_per_cta - 1) / a.items_per_cta;
-  kdq<<<grid, XT_THREADS, DQ_SMEM, s>>>(mq, mdo, mk_l, mv_l, a);
-  count_launch();
-  kdkv<<<grid, XT_THREADS, DCfg::SMEM, s>>>(mq, mdo, mk_t, mv_t, a);
-  count_launch();
-  return (int)cudaGetLastError();
+  return xt_launch_fused<40, 197>(p, s);
 }
 
 }  // namespace xfm

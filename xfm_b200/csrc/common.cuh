@@ -146,7 +146,24 @@ XFM_DEVINL void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32]) {
       : "r"(taddr)
       : "memory");
 }
+XFM_DEVINL void tmem_ld_32x32_16(uint32_t taddr, uint32_t (&r)[32]) {  // 16 columns into r[0..15]
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr)
+      : "memory");
+}
 XFM_DEVINL void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+
+// eight fp32 values -> bf16 (round to nearest), one 16-byte store
+XFM_DEVINL void st_bf16x8(uint8_t* dst, const float (&p)[8]) {
+  uint4 u;
+  __nv_bfloat162 t0 = __floats2bfloat162_rn(p[0], p[1]), t1 = __floats2bfloat162_rn(p[2], p[3]);
+  __nv_bfloat162 t2 = __floats2bfloat162_rn(p[4], p[5]), t3 = __floats2bfloat162_rn(p[6], p[7]);
+  u.x = *(uint32_t*)&t0; u.y = *(uint32_t*)&t1; u.z = *(uint32_t*)&t2; u.w = *(uint32_t*)&t3;
+  *(uint4*)dst = u;
+}
 
 // Shared-memory matrix descriptor (sm_100 "version 1"), SWIZZLE_128B.
 //  K-major  operand: rows of 128 B (64 bf16 along K); 8-row groups 1024 B apart  -> SBO = 1024, LBO unused.

@@ -27,6 +27,12 @@ int attention_bwd(const xfm_attn_params* p, cudaStream_t s);
 bool vit_attention_tc_supported(const xfm_attn_params* p, bool bwd = false);
 int vit_attention_fwd_tc(const xfm_attn_params* p, cudaStream_t s);
 int vit_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s);
+// TMA maps of the tcgen05 attention kernels (attention_tc.cu): a bf16 activation of `cols` columns with a row stride of ld_elems
+// elements, SWIZZLE_128B boxes of 64 columns.  2D: [rows] rows, boxes of box_rows rows.  3D: [samples][rows_per_sample] rows
+// (samples sample_stride_rows rows apart, default rows_per_sample), boxes of 128 rows that clip at a sample's last row.
+int encode_rows(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems, uint32_t box_rows);
+int encode_rows_3d(CUtensorMap* map, const void* base, uint64_t cols, uint64_t rows_per_sample, uint64_t samples,
+                   uint64_t ld_elems, uint64_t sample_stride_rows = 0);
 // out / lse from nb key-block partials (bf16 [nb, B*L, H*64], f32 [nb, B, H, L]); attention_tc.cu
 int launch_merge_parts(int nb, const void* part_out, const float* part_lse, void* out, int64_t o_stride, float* lse, int B, int H,
                        int L, cudaStream_t s);

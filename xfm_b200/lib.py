@@ -197,7 +197,7 @@ class AttnParams(C.Structure):
         ("ds_ld", C.c_int64),
         ("kv_offsets", C.c_void_p), ("kv_samples", C.c_void_p),
         ("rel_table", C.c_void_p), ("rel_window", C.c_int32), ("allow_tc", C.c_int32),
-        ("part_out", C.c_void_p), ("part_lse", C.c_void_p), ("rel_dtable", C.c_void_p),
+        ("part_out", C.c_void_p), ("part_lse", C.c_void_p),
     ]
 
 
@@ -253,11 +253,10 @@ def attention_fwd(q, k, v, B, H, Lq, Lk, scale, *, Bkv=None, bias=None, kmask=No
 
 def attention_bwd(dout, q, k, v, out, lse, B, H, Lq, Lk, scale, dq, dk, dv, *, Bkv=None, bias=None, kmask=None,
                   kv_index=None, kv_offsets=None, kv_samples=None, dropout_p=0.0, dropout_seed=0, ds_dump=None,
-                  rel_table=None, rel_window=0, rel_dtable=None, allow_tc=True):
-    """Writes bf16 dq [B*Lq, ...], dk / dv [Bkv*Lk, ...] (views with row strides).  ds_dump: bf16 [B,H,Lq,ld] (mma.sync path:
-    the caller reduces it into the bias-table gradient).  rel_table / rel_window / rel_dtable: closed-form relative-position
-    bias and (optionally) its f32 gradient accumulator [(2W-1)^2+3, H] (tcgen05 path; ds_dump + the caller's reduction is
-    the faster way to get the table gradient)."""
+                  rel_table=None, rel_window=0, allow_tc=True):
+    """Writes bf16 dq [B*Lq, ...], dk / dv [Bkv*Lk, ...] (views with row strides).  ds_dump: bf16 [B,H,Lq,ld] receives dS;
+    the caller reduces it into the bias-table gradient (batch_sum_bf16, relpos_bias_bwd).  rel_table / rel_window:
+    closed-form relative-position bias [(2W-1)^2+3, H] f32 whose gather equals `bias` (tcgen05 path)."""
     Bkv = B if Bkv is None else Bkv
     p = AttnParams()
     _attn_common(p, q, k, v, B, H, Lq, Lk, Bkv, scale, bias, kmask, kv_index, dropout_p, dropout_seed)
@@ -280,15 +279,7 @@ def attention_bwd(dout, q, k, v, out, lse, B, H, Lq, Lk, scale, dq, dk, dv, *, B
         assert rel_table.dtype == torch.float32 and rel_table.is_contiguous() and rel_table.shape[1] == H
         assert rel_table.shape[0] == (2 * rel_window - 1) ** 2 + 3
         p.rel_table, p.rel_window = rel_table.data_ptr(), rel_window
-        if rel_dtable is not None:
-            assert rel_dtable.dtype == torch.float32 and rel_dtable.is_contiguous() and rel_dtable.shape == rel_table.shape
-            p.rel_dtable = rel_dtable.data_ptr()
     check(lib().xfm_attention_bwd(C.byref(p), stream_ptr()), "xfm_attention_bwd")
-
-
-def vit_attention_tc_ok(n_tokens):
-    """Token counts (W*W + 1) with an instantiated tcgen05 self-attention kernel (attention_tc.cu::window_for)."""
-    return n_tokens in (197, 145, 50, 17)
 
 
 def vit_attention_bwd_tc_ok(n_tokens):
