@@ -308,6 +308,33 @@ int xfm_resize_taps(const int64_t* desc, int32_t* hb, int32_t* hk, int KH, int32
 int xfm_resize_bicubic_u8(const uint8_t* src, const int64_t* desc, const int32_t* hb, const int32_t* hk, int KH, const int32_t* vb,
                           const int32_t* vk, int KV, uint8_t* tmp, uint8_t* out, int B, int max_rows, int OH, int OW, void* stream);
 
+/* Baseline JPEG decode of the batch feeder (csrc/jpeg.cu): file bytes -> RGB, bit-identical to Pillow's
+ * Image.open(f).convert("RGB") over libjpeg-turbo (jdhuff.c decode_mcu, jidctint.c ISLOW as its SIMD code computes it,
+ * jdsample.c h2v1 / h2v2 fancy upsampling, jdcolor.c ycc_rgb_convert) for the device subset: SOF0 / SOF1 8-bit, one
+ * sequential Huffman scan, grayscale or YCbCr (libjpeg's default_decompress_parms rule), sampling 4:4:4 / 4:2:2 / 4:2:0,
+ * with or without DRI.  Every other stream gets a non-zero status and is decoded by the caller (feed.py: Pillow).
+ * Two host-only calls (no CUDA call; all pointers HOST pointers, images spread over up to `threads` threads):
+ *   xfm_jpeg_plan    info int64 [n, XFM_JPEG_INFO] = {status (0 = device path), width, height, restart intervals,
+ *                    coefficient blocks, component plane bytes, 0, 0}; width / height are 0 when the header was not read.
+ *   xfm_jpeg_tables  offs int64 [n, 4] = {byte offset of the blob in the device byte buffer, first coefficient block, first
+ *                    plane byte (multiple of 8), byte offset of the image in out}; fills desc (n * xfm_jpeg_desc_bytes(),
+ *                    16-byte aligned: Huffman look-up tables, natural-order quantisation tables, geometry) and intervals
+ *                    int64 [sum of info[:, 3], 2] (byte range of every restart interval in the device byte buffer).
+ * xfm_jpeg_decode (device pointers; three launches on `stream`, graph-capturable):
+ *   bytes    u8 packed blobs           coef   int16 [sum blocks, 64] scratch (16-byte aligned)
+ *   planes   u8 scratch, sum plane bytes                out  u8: image b is [height, width, 3] at byte offs[b][3]
+ *   status   int32 [n]: 0 on entry for device-path images; the entropy stage ORs in a code (invalid Huffman code 16, run
+ *            past coefficient 63 32, data ending before the interval's last MCU 64, unexpected marker 128) — such an image
+ *            must be decoded again by the caller.  Images with info status != 0 are not touched (out included).
+ *   max_blocks / max_w / max_h: the largest coefficient block count, width and height of a device-path image. */
+#define XFM_JPEG_INFO 8
+int xfm_jpeg_plan(const void* const* blobs, const int64_t* nbytes, int n, int64_t* info, int threads);
+size_t xfm_jpeg_desc_bytes(void);
+int xfm_jpeg_tables(const void* const* blobs, const int64_t* nbytes, int n, const int64_t* info, const int64_t* offs, void* desc,
+                    int64_t* intervals, int threads);
+int xfm_jpeg_decode(const uint8_t* bytes, const void* desc, const int64_t* intervals, int n, int16_t* coef, uint8_t* planes,
+                    uint8_t* out, int32_t* status, int64_t max_blocks, int max_w, int max_h, void* stream);
+
 /* Flat-buffer optimizer step (accelerators/ddp_accelerator.py:89-98 clip_grad_norm_ + optimizer.step with the
  * transformers AdamW of optim.py:4-50).  P/G/M/V: f32 buffers of nchunks*64 elements, S: bf16 shadow (may be null).
  *   chunk_seg[nchunks] int32  static: parameter segment of every 64-element chunk, -1 = frozen / padding (never touched)

@@ -256,6 +256,19 @@ int xfm_host_pack(const void* const* srcs, const int64_t* nbytes, int n, void* d
   for (auto& th : pool) th.join();
   return 0;
 }
+// Host-side JPEG plan (two calls: sizes, then tables into caller buffers) and the device decode; csrc/jpeg.cu.
+int xfm_jpeg_plan(const void* const* blobs, const int64_t* nbytes, int n, int64_t* info, int threads) {
+  return jpeg_plan(blobs, nbytes, n, info, threads);
+}
+size_t xfm_jpeg_desc_bytes(void) { return jpeg_desc_bytes(); }
+int xfm_jpeg_tables(const void* const* blobs, const int64_t* nbytes, int n, const int64_t* info, const int64_t* offs, void* desc,
+                    int64_t* intervals, int threads) {
+  return jpeg_tables(blobs, nbytes, n, info, offs, desc, intervals, threads);
+}
+int xfm_jpeg_decode(const uint8_t* bytes, const void* desc, const int64_t* intervals, int n, int16_t* coef, uint8_t* planes,
+                    uint8_t* out, int32_t* status, int64_t max_blocks, int max_w, int max_h, void* stream) {
+  return jpeg_decode(bytes, desc, intervals, n, coef, planes, out, status, max_blocks, max_w, max_h, ST);
+}
 int xfm_resize_taps(const int64_t* desc, int32_t* hb, int32_t* hk, int KH, int32_t* vb, int32_t* vk, int KV, int B, int OH, int OW,
                     void* stream) {
   return resize_taps(desc, hb, hk, KH, vb, vk, KV, B, OH, OW, ST);

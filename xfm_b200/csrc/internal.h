@@ -128,6 +128,12 @@ int resize_bicubic_u8(const uint8_t* src, const int64_t* desc, const int32_t* hb
                       const int32_t* vk, int KV, uint8_t* tmp, uint8_t* out, int B, int max_rows, int OH, int OW, cudaStream_t s);
 int resize_taps(const int64_t* desc, int32_t* hb, int32_t* hk, int KH, int32_t* vb, int32_t* vk, int KV, int B, int OH, int OW,
                 cudaStream_t s);
+int jpeg_plan(const void* const* blobs, const int64_t* nbytes, int n, int64_t* info, int threads);
+size_t jpeg_desc_bytes();
+int jpeg_tables(const void* const* blobs, const int64_t* nbytes, int n, const int64_t* info, const int64_t* offs, void* desc,
+                int64_t* intervals, int threads);
+int jpeg_decode(const uint8_t* bytes, const void* desc, const int64_t* intervals, int n, int16_t* coef, uint8_t* planes, uint8_t* out,
+                int32_t* status, int64_t max_blocks, int max_w, int max_h, cudaStream_t s);
 int image_u8_to_f32(const uint8_t* in, float* out, const uint8_t* flip, int B, int H, int W, const float* mean, const float* stdv,
                     cudaStream_t s);
 int grad_sumsq(const float* g, const int32_t* chunk_seg, const uint8_t* seg_group, size_t nchunks, int32_t* seg_step,

@@ -38,8 +38,14 @@ Device half:
                               transform (decode -> resize -> normalize); the training Compose keeps RandAugment (cv2, on the
                               host) between crop and ToTensor, so there it is an option for loaders that augment after it.
 
-JPEG decode and RandAugment stay CPU work in the DataLoader workers (DESIGN §7).  There is no CPU path for
-the device half: `DeviceFeeder` raises without a CUDA device.
+  * `decode_jpeg`, `decode_crop_resize`  baseline JPEG decode on the GPU (`xfm_jpeg_plan` on the host, `xfm_jpeg_decode`:
+                              Huffman, ISLOW IDCT, fancy upsampling, YCbCr -> RGB), bit-identical to
+                              `Image.open(f).convert("RGB")`; other files (progressive, CMYK, PNG, ...) are decoded by Pillow
+                              into the same buffer.  With `crop_resize`'s device half, the evaluation transform runs from file
+                              bytes to the normalized tensor on the GPU.  `jpeg_size` reads a file's size from its header.
+
+RandAugment stays CPU work in the DataLoader workers (DESIGN §7).  There is no CPU path for the device half:
+`DeviceFeeder`, `crop_resize` and `decode_jpeg` raise without a CUDA device.
 """
 import math
 import random as _random
@@ -930,13 +936,123 @@ def crop_resize(images, boxes, out_h, out_w, device=None, taps="device", flips=N
         return out
     packed = torch.empty(plan["src_bytes"], dtype=torch.uint8, pin_memory=True)
     lib.host_pack([im.contiguous() for im in images], packed)      # multi-threaded gather into the staging buffer
-    desc = plan["desc"].pin_memory().to(device, non_blocking=True)
+    return _resize_on_device(packed.to(device, non_blocking=True), plan, out, taps)
+
+
+def _resize_on_device(src, plan, out, taps="device"):
+    """Device half of `crop_resize` / `decode_crop_resize`: src = the packed images on the device, in the layout of
+    `crop_resize_plan` (image b at byte desc[b, 0]); taps as in `crop_resize`."""
+    from . import lib
+    B, out_h, out_w, _ = out.shape
+    desc = plan["desc"].pin_memory().to(out.device, non_blocking=True)
     if taps == "host":
-        hb, hk, vb, vk = (plan[k].pin_memory().to(device, non_blocking=True) for k in ("hb", "hk", "vb", "vk"))
+        hb, hk, vb, vk = (plan[k].pin_memory().to(out.device, non_blocking=True) for k in ("hb", "hk", "vb", "vk"))
     else:
         hb, hk, vb, vk = lib.resize_taps(desc, out_h, out_w, plan["KH"], plan["KV"])
-    tmp = torch.empty(plan["tmp_bytes"], dtype=torch.uint8, device=device)
-    return lib.resize_bicubic_u8(packed.to(device, non_blocking=True), desc, hb, hk, vb, vk, tmp, out, plan["max_rows"])
+    tmp = torch.empty(plan["tmp_bytes"], dtype=torch.uint8, device=out.device)
+    return lib.resize_bicubic_u8(src, desc, hb, hk, vb, vk, tmp, out, plan["max_rows"])
+
+
+# --------------------------------------------------------------------------------------------------- baseline JPEG decode
+def _pil_rgb(blob):
+    """What the evaluation loaders do to a file: `Image.open(f).convert("RGB")`, as uint8 [h, w, 3]."""
+    import io
+    import numpy as np
+    from PIL import Image
+    with Image.open(io.BytesIO(blob)) as im:
+        return torch.from_numpy(np.array(im.convert("RGB")))
+
+
+def jpeg_size(blob):
+    """(width, height) of an image file's bytes, read from its header (for `random_resized_crop_box` before decoding):
+    the marker walk of `xfm_jpeg_plan` for the device subset, Pillow's header parser for anything else."""
+    import io
+    from PIL import Image
+    from . import lib
+    st, w, h = (int(v) for v in lib.jpeg_plan([bytes(blob)], threads=1)[0, :3])
+    if st == 0:
+        return w, h
+    with Image.open(io.BytesIO(blob)) as im:
+        return im.size
+
+
+def decode_jpeg(blobs, device=None, threads=8):
+    """Decode a batch of image files (a list of `bytes`) on the GPU: returns (out, meta, n_fallback) with out = uint8 on the
+    device, image b = out[meta[b, 0] : + meta[b, 1] * meta[b, 2] * 3] viewed as [meta[b, 2] (height), meta[b, 1] (width), 3],
+    packed back to back in order (the source layout of `crop_resize_plan`), and meta int64 [B, 3] (offset, width, height) on
+    the host.  Every image equals `Image.open(BytesIO(b)).convert("RGB")` byte for byte (or the call raises what Pillow
+    raises): baseline Huffman JPEGs (grayscale or YCbCr, 4:4:4 / 4:2:2 / 4:2:0, with or without restart markers) are decoded
+    by `xfm_jpeg_decode` (csrc/jpeg.cu); every other file, and every file the device decoder flags (invalid code, data
+    ending early, unexpected marker), is decoded by Pillow into the same place.  n_fallback counts those.
+    One synchronisation per call: the device->host read of the per-image status words that decides the second group."""
+    import numpy as np
+    from PIL import Image
+    from . import lib
+    if not torch.cuda.is_available():
+        raise RuntimeError("xfm_b200.feed.decode_jpeg needs a CUDA device (sm_100a); there is no CPU path")
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    blobs = [b if isinstance(b, bytes) else bytes(b) for b in blobs]
+    B = len(blobs)
+    info = lib.jpeg_plan(blobs, threads)
+    limit = Image.MAX_IMAGE_PIXELS
+    host = {}
+    for i in range(B):
+        if info[i, 0] == 0 and limit is not None and info[i, 1] * info[i, 2] > limit:
+            info[i, 0] = -1                                  # Pillow's decompression-bomb check decides (warning or error)
+        if info[i, 0] != 0:
+            host[i] = _pil_rgb(blobs[i])
+            info[i, 1], info[i, 2] = host[i].shape[1], host[i].shape[0]
+    dev = info[:, 0] == 0
+    nbytes = info[:, 1] * info[:, 2] * 3
+    offs = np.zeros((B, 4), np.int64)
+    for col, size in ((0, np.array([len(b) for b in blobs], np.int64)), (1, info[:, 4]), (2, info[:, 5]), (3, nbytes)):
+        size = size if col == 3 else np.where(dev, size, 0)
+        offs[:, col] = np.cumsum(size) - size
+    meta = torch.from_numpy(np.stack([offs[:, 3], info[:, 1], info[:, 2]], 1) if B else np.zeros((0, 3), np.int64))
+    out = torch.empty(max(int(nbytes.sum()), 1), dtype=torch.uint8, device=device)
+    if dev.any():
+        desc, intervals = lib.jpeg_tables(blobs, info, offs, threads)
+        data = torch.empty(int(sum(len(blobs[i]) for i in np.nonzero(dev)[0])), dtype=torch.uint8, pin_memory=True)
+        lib.host_pack([blobs[i] for i in np.nonzero(dev)[0]], data, threads)
+        status_h = torch.from_numpy(np.where(dev, 0, 1).astype(np.int32)).pin_memory()
+        nb = lambda n: torch.empty(max(int(n), 1), dtype=torch.uint8, device=device)  # noqa: E731
+        coef = torch.empty((max(int(info[dev, 4].sum()), 1), 64), dtype=torch.int16, device=device)
+        planes, status = nb(info[dev, 5].sum()), status_h.to(device, non_blocking=True)
+        lib.jpeg_decode(data.to(device, non_blocking=True), desc.to(device, non_blocking=True),
+                        intervals.to(device, non_blocking=True), B, coef, planes, out, status,
+                        int(info[dev, 4].max()), int(info[dev, 1].max()), int(info[dev, 2].max()))
+    for i, img in host.items():
+        out[offs[i, 3]:offs[i, 3] + nbytes[i]].copy_(img.reshape(-1))
+    n_fallback = len(host)
+    if dev.any():
+        flagged = torch.nonzero(status.cpu() != 0).flatten().tolist()     # the one synchronisation of the call
+        for i in flagged:
+            if i in host:
+                continue
+            img = _pil_rgb(blobs[i])
+            if tuple(img.shape) != (int(info[i, 2]), int(info[i, 1]), 3):
+                raise RuntimeError(f"decode_jpeg: image {i}: Pillow returned {tuple(img.shape)}, the header says "
+                                   f"{int(info[i, 1])} x {int(info[i, 2])}")
+            out[offs[i, 3]:offs[i, 3] + nbytes[i]].copy_(img.reshape(-1))
+            n_fallback += 1
+    return out, meta, n_fallback
+
+
+def decode_crop_resize(blobs, boxes, out_h, out_w, device=None):
+    """Decode + crop + bicubic resize of image files on the GPU: uint8 [B, out_h, out_w, 3] on the device equal to
+    `Image.open(BytesIO(b)).convert("RGB").crop(box).resize((out_w, out_h), BICUBIC)`; boxes entries (x0, y0, x1, y1) or
+    None = the whole image.  `decode_jpeg` -> `xfm_resize_taps` -> `xfm_resize_bicubic_u8` reading the decoded batch in
+    place (no copy in between); `lib.image_u8_to_f32` finishes the evaluation transform."""
+    src, meta, _ = decode_jpeg(blobs, device)
+    sizes = [(int(h), int(w)) for _, w, h in meta.tolist()]
+    boxes = [(0, 0, w, h) if bx is None else tuple(int(v) for v in bx) for bx, (h, w) in zip(boxes, sizes)]
+    if len(boxes) != len(sizes):
+        raise ValueError("decode_crop_resize: one box (or None) per image")
+    plan = crop_resize_plan(sizes, boxes, out_h, out_w, taps=False)
+    out = torch.empty((len(sizes), out_h, out_w, 3), dtype=torch.uint8, device=src.device)
+    if not sizes:
+        return out
+    return _resize_on_device(src, plan, out)
 
 
 def _is_u8_image(t):

@@ -651,15 +651,65 @@ def image_u8_to_f32(img_u8, mean, std, flip=None, out=None):
 
 
 def host_pack(tensors, out, threads=8):
-    """Copy the bytes of the (contiguous, host) tensors back to back into `out` (uint8, host; normally pinned) with several
+    """Copy the bytes of the (contiguous, host) tensors or `bytes` objects back to back into `out` (uint8, host; normally pinned) with several
     threads.  Host-only: works without a CUDA device."""
     n = len(tensors)
     assert out.device.type == "cpu" and out.dtype == torch.uint8 and out.is_contiguous()
-    sizes = [t.numel() * t.element_size() for t in tensors]
-    assert all(t.device.type == "cpu" and t.is_contiguous() for t in tensors) and sum(sizes) <= out.numel()
-    srcs = (C.c_void_p * max(n, 1))(*[t.data_ptr() for t in tensors])
-    nb = (C.c_int64 * max(n, 1))(*sizes)
+    assert all(isinstance(t, bytes) or (t.device.type == "cpu" and t.is_contiguous()) for t in tensors)
+    srcs, nb = _host_segments(tensors)
+    assert sum(nb) <= out.numel()
     check(load().xfm_host_pack(srcs, nb, n, C.c_void_p(out.data_ptr()), int(threads)), "xfm_host_pack")
+    return out
+
+
+def _host_segments(parts):
+    """ctypes (void* [n], int64 [n]) of host tensors or `bytes` objects (their buffers, not copies; the caller keeps `parts`
+    alive for the duration of the C call)."""
+    n = len(parts)
+    ptrs = [C.cast(C.c_char_p(p), C.c_void_p).value if isinstance(p, bytes) else p.data_ptr() for p in parts]
+    sizes = [len(p) if isinstance(p, bytes) else p.numel() * p.element_size() for p in parts]
+    return (C.c_void_p * max(n, 1))(*ptrs), (C.c_int64 * max(n, 1))(*sizes)
+
+
+JPEG_INFO = 8      # XFM_JPEG_INFO: columns of xfm_jpeg_plan's per-image row
+
+
+def jpeg_plan(blobs, threads=8):
+    """Host-only marker walk of each `bytes` blob (xfm_jpeg_plan): int64 [n, 8] {status (0 = device path), width, height,
+    restart intervals, coefficient blocks, plane bytes, 0, 0}.  Works without a CUDA device."""
+    import numpy as np
+    info = np.zeros((len(blobs), JPEG_INFO), np.int64)
+    srcs, nb = _host_segments(blobs)
+    check(load().xfm_jpeg_plan(srcs, nb, len(blobs), C.c_void_p(info.ctypes.data), int(threads)), "xfm_jpeg_plan")
+    return info
+
+
+def jpeg_tables(blobs, info, offs, threads=8):
+    """Second host call (xfm_jpeg_tables): offs int64 [n, 4] {blob offset in the device byte buffer, first coefficient block,
+    first plane byte, output byte offset}.  Returns (desc u8 [n * desc bytes], intervals int64 [sum info[:, 3], 2]) as host
+    tensors, pinned when CUDA is there."""
+    import numpy as np
+    l = load()
+    l.xfm_jpeg_desc_bytes.restype = C.c_size_t
+    n = len(blobs)
+    info, offs = np.ascontiguousarray(info, np.int64), np.ascontiguousarray(offs, np.int64)
+    assert info.shape == (n, JPEG_INFO) and offs.shape == (n, 4)
+    pin = torch.cuda.is_available()
+    desc = torch.empty(max(n, 1) * l.xfm_jpeg_desc_bytes(), dtype=torch.uint8, pin_memory=pin)
+    n_int = int(info[info[:, 0] == 0, 3].sum())
+    intervals = torch.empty((max(n_int, 1), 2), dtype=torch.int64, pin_memory=pin)
+    srcs, nb = _host_segments(blobs)
+    check(l.xfm_jpeg_tables(srcs, nb, n, C.c_void_p(info.ctypes.data), C.c_void_p(offs.ctypes.data), C.c_void_p(desc.data_ptr()),
+                            C.c_void_p(intervals.data_ptr()), int(threads)), "xfm_jpeg_tables")
+    return desc, intervals
+
+
+def jpeg_decode(data, desc, intervals, n, coef, planes, out, status, max_blocks, max_w, max_h):
+    """The three decode launches (xfm_jpeg_decode) on the current stream; every tensor on the device (include/xfm_b200.h)."""
+    assert data.dtype == torch.uint8 and desc.dtype == torch.uint8 and intervals.dtype == torch.int64 and coef.dtype == torch.int16
+    assert planes.dtype == torch.uint8 and out.dtype == torch.uint8 and status.dtype == torch.int32 and status.numel() >= n
+    check(lib().xfm_jpeg_decode(_p(data), _p(desc), _p(intervals), int(n), _p(coef), _p(planes), _p(out), _p(status),
+                                C.c_int64(int(max_blocks)), int(max_w), int(max_h), stream_ptr()), "xfm_jpeg_decode")
     return out
 
 
