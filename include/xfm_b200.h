@@ -107,7 +107,8 @@ int xfm_gemm_bf16(const xfm_gemm_params* p, void* stream);
  *   logits = scale * q.k + bias[h,i,j] + kmask[b,j]
  * Backward needs lse (saved by the forward), a [B,H,Lq] f32 scratch `delta`, and writes bf16 dq/dk/dv.
  * ds_dump (optional, bf16 [B,H,Lq,ds_ld]) receives dS for the relative-position-bias gradient.
- * kv_offsets/kv_samples: CSR inverse of kv_index over the Bkv K/V rows (null = identity).
+ * kv_offsets/kv_samples: CSR inverse of kv_index over the Bkv K/V rows (null = identity); the backward requires them
+ * whenever kv_index is given.  K/V rows that no sample references get zero dk/dv.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct xfm_attn_params {
   const void *q, *k, *v;

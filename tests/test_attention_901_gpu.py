@@ -1,10 +1,10 @@
 """Attention at 480 px (W = 30, 901 image tokens): the tcgen05 kernels in five key blocks (4 x 192 + 133) for ViT
 self-attention and for 40-token cross-attention, and the streaming mma.sync kernels that serve every shape whose K / V
 (or Q / dO) do not fit shared memory.  End to end: XFMForVQA at image_res 480 against the CPU oracle."""
-import numpy as np
 import pytest
 import torch
 
+from oracle import dropout_mask as D
 from oracle import xfm_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -29,25 +29,9 @@ def bf(x):
     return x.to(torch.bfloat16)
 
 
-def _mix32(x):
-    x = x ^ (x >> np.uint32(16))
-    x = x * np.uint32(0x7FEB352D)
-    x = x ^ (x >> np.uint32(15))
-    x = x * np.uint32(0x846CA68B)
-    return x ^ (x >> np.uint32(16))
-
-
 def attn_keep_mask(B, H, Lq, Lk, seed, p):
-    """attention.cu::drop_keep: element ((b*H + h)*Lq + q) * ((Lk+1) & ~1) + key of common.cuh's hash, as [B, H, Lq, Lk]."""
-    lke = (Lk + 1) & ~1
-    thr = np.uint32(np.float32(p) * np.float32(65536.0) + np.float32(0.5))
-    s = np.uint32((seed & 0xFFFFFFFF) ^ (((seed >> 32) * 0x85EBCA6B) & 0xFFFFFFFF))
-    idx = (np.arange(B * H * Lq, dtype=np.uint64)[:, None] * np.uint64(lke) + np.arange(Lk, dtype=np.uint64)[None, :])
-    pair = idx >> np.uint64(1)
-    lo, hi = (pair & np.uint64(0xFFFFFFFF)).astype(np.uint32), (pair >> np.uint64(32)).astype(np.uint32)
-    x = _mix32((lo + hi * np.uint32(0x9E3779B1)) ^ s)
-    bits = np.where((idx & np.uint64(1)) == 1, x >> np.uint32(16), x & np.uint32(0xFFFF))
-    return torch.from_numpy((bits >= thr).reshape(B, H, Lq, Lk))
+    """attention.cu::drop_keep as [B, H, Lq, Lk]."""
+    return torch.from_numpy(D.keep(seed, D.attention_index(B, H, Lq, Lk), p))
 
 
 def kernel_names(fn):

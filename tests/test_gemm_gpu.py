@@ -15,6 +15,9 @@ from dataclasses import dataclass
 import numpy as np
 import pytest
 import torch
+from canary import Buf
+
+from oracle.dropout_mask import keep
 
 pytestmark = pytest.mark.gpu
 
@@ -40,55 +43,9 @@ def _r8(x):
     return (x + 7) // 8 * 8
 
 
-# ------------------------------------------------------------------------------------------------ canary buffers
-_BITS = {torch.float32: torch.int32, torch.bfloat16: torch.int16}
-_CANARY = {torch.float32: 0x7FC00000, torch.bfloat16: 0x7FA5}   # an f32 NaN and a bf16 NaN with payload
-
-
-class Buf:
-    """[rows, cols] view with row stride ld inside a canary-filled buffer: `off` elements and one full row before it, two
-    rows after it, ld - cols columns beside every row."""
-
-    def __init__(self, rows, cols, ld, dtype, off=0):
-        self.buf = torch.empty(off + (rows + 3) * ld, dtype=dtype, device="cuda")
-        self.buf.view(_BITS[dtype]).fill_(_CANARY[dtype])
-        self.shape, self.stride, self.start = (rows, cols), (ld, 1), off + ld
-        self.view = torch.as_strided(self.buf, self.shape, self.stride, self.start)
-        self.before = None
-
-    def snapshot(self):
-        self.before = self.buf.view(_BITS[self.buf.dtype]).clone()
-
-    def outside_unchanged(self):
-        now = self.buf.view(_BITS[self.buf.dtype]).clone()
-        before = self.before.clone()
-        for t in (now, before):
-            torch.as_strided(t, self.shape, self.stride, self.start).zero_()
-        return torch.equal(now, before)
-
-    def unchanged(self):
-        return torch.equal(self.buf.view(_BITS[self.buf.dtype]), self.before)
-
-
-# ------------------------------------------------------------------------------------------------ dropout mask (common.cuh)
-def _mix32(x):
-    x = x ^ (x >> np.uint32(16))
-    x = x * np.uint32(0x7FEB352D)
-    x = x ^ (x >> np.uint32(15))
-    x = x * np.uint32(0x846CA68B)
-    return x ^ (x >> np.uint32(16))
-
-
 def keep_mask(M, N, seed, p):
-    """drop_keep_idx(seed, row * N + col, p) for every element of an [M, N] output (numpy uint32 arithmetic)."""
-    thr = np.uint32(np.float32(p) * np.float32(65536.0) + np.float32(0.5))
-    s = np.uint32((seed & 0xFFFFFFFF) ^ (((seed >> 32) * 0x85EBCA6B) & 0xFFFFFFFF))
-    idx = np.arange(M * N, dtype=np.uint64)
-    pair = idx >> np.uint64(1)
-    lo, hi = (pair & np.uint64(0xFFFFFFFF)).astype(np.uint32), (pair >> np.uint64(32)).astype(np.uint32)
-    x = _mix32((lo + hi * np.uint32(0x9E3779B1)) ^ s)
-    bits = np.where((idx & np.uint64(1)) == 1, x >> np.uint32(16), x & np.uint32(0xFFFF))
-    return torch.from_numpy((bits >= thr).reshape(M, N))
+    """The dropout mask of an [M, N] epilogue: element row * N + col of common.cuh's hash."""
+    return torch.from_numpy(keep(seed, np.arange(M * N), p).reshape(M, N))
 
 
 # ------------------------------------------------------------------------------------------------ the case matrix

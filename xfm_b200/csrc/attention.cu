@@ -681,6 +681,10 @@ int attention_bwd(const xfm_attn_params* p, cudaStream_t s) {
     set_error("attention_bwd: missing pointer");
     return XFM_ERR_BAD_ARG;
   }
+  if (p->kv_index && (!p->kv_offsets || !p->kv_samples)) {   // dK / dV sum over the samples of each K/V row: the CSR lists them
+    set_error("attention_bwd: kv_index needs kv_offsets and kv_samples");
+    return XFM_ERR_BAD_ARG;
+  }
   if (p->ds_dump && ((p->ds_ld & 7) || p->ds_ld < p->Lk)) {
     set_error("attention_bwd: ds_ld must be a multiple of 8 and >= Lk");
     return XFM_ERR_BAD_ARG;

@@ -60,11 +60,12 @@ struct XCfg {
 
 XFM_DEVINL void xt_ld32(uint32_t taddr, uint32_t (&r)[32]) { tmem_ld_32x32(taddr, r); }
 
-// One "unit" = (K/V row, head, chunk of <= GMAX samples).  Every role walks the same unit sequence.
+// One "unit" = (K/V row, head, chunk of <= GMAX samples).  Every role walks the same unit sequence.  With EMPTY, an image
+// that no sample references is one unit with ns = 0 (the backward stores zero dK / dV for it); without, it is skipped.
 struct XUnit {
   int r, h, first, ns;   // K/V row, head, index of the chunk's first entry in kv_samples, samples in the chunk
 };
-template <int GMAX>
+template <int GMAX, bool EMPTY = false>
 struct XWalker {
   const XAttnArgs& a;
   int it, it_end, chunk, nchunks, off0, cnt;
@@ -77,6 +78,7 @@ struct XWalker {
       off0 = a.kv_offsets[r];
       cnt = a.kv_offsets[r + 1] - off0;
       nchunks = (cnt + GMAX - 1) / GMAX;
+      if (EMPTY && nchunks == 0) nchunks = 1;
       chunk = 0;
     }
     u.r = it % a.Bkv;
@@ -409,7 +411,7 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
   // Every role walks the same unit sequence; K / V are loaded once per item (image, head), Q / dO once per unit.
   if (warp == 0) {
     if (lane == 0) {
-      XWalker<GMAX> w(a, item0, item1);
+      XWalker<GMAX, true> w(a, item0, item1);
       XUnit u;
       uint32_t up = 0, ip = 0;   // unit parity, item parity
       int cur = -1;
@@ -440,7 +442,7 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
       constexpr uint32_t idesc_dkv = make_idesc_bf16(128, XT_HD, 1, 1);
       const uint32_t aQ = smem_u32(sQ), adO = smem_u32(sdO), aK = smem_u32(sK), aV = smem_u32(sV), adS = smem_u32(sdS),
                      aP = smem_u32(sP);
-      XWalker<GMAX> w(a, item0, item1);
+      XWalker<GMAX, true> w(a, item0, item1);
       XUnit u;
       uint32_t up = 0, ip = 1;
       int cur = -1;
@@ -509,7 +511,7 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
     const int ch_lo = (wg * N16) / 4, ch_hi = ((wg + 1) * N16) / 4;
     constexpr int LKE = (LK + 1) & ~1;
     const bool elected = threadIdx.x == 64;   // issues every TMA store of this CTA (bulk groups are per thread)
-    XWalker<GMAX> w(a, item0, item1);
+    XWalker<GMAX, true> w(a, item0, item1);
     XUnit u;
     uint32_t up = 0;
     int cur = -1, chunk_of_item = 0;
@@ -610,7 +612,7 @@ xattn_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
         for (int e = 0; e < 32; e += 8) {
           float vv[8];
 #pragma unroll
-          for (int k = 0; k < 8; ++k) vv[k] = __uint_as_float(o[e + k]) * mul;
+          for (int k = 0; k < 8; ++k) vv[k] = u.ns > 0 ? __uint_as_float(o[e + k]) * mul : 0.f;   // no samples: accumulators never written
           st_bf16x8(row + (((half * 4 + (e >> 3)) ^ sw) << 4), vv);
         }
       }
