@@ -148,6 +148,41 @@ int xfm_attention_bwd(const xfm_attn_params* p, void* stream);
 int xfm_attention_fwd_parts(const xfm_attn_params* p);
 
 /* ------------------------------------------------------------------------------------------------
+ * K4v — packed variable-length self-attention, head_dim 64 (RoBERTa sequence classification over GLUE batches, whose
+ * sentences are padded to max_seq_length but mostly much shorter).  n sequences of 1..128 tokens are packed back to back,
+ * with no padding rows: sequence s occupies rows [cu_seqlens[s], cu_seqlens[s+1]) of the q / k / v / out column slices
+ * (T = cu_seqlens[n] rows); a query sees exactly the keys of its own sequence.
+ *   logits = scale * q.k;  lse / delta f32 [H, T]
+ * Tiles: a tile is a maximal run of consecutive sequences of at most 128 rows in total; tiles int32 [n_tiles + 1] holds
+ * the first sequence of every tile, then n.  xfm_attention_varlen_plan computes cu_seqlens and tiles from the lengths
+ * (host-only, no device; HOST pointers, cu_seqlens [n + 1], tiles room for n + 1 entries) and rejects lengths outside
+ * 1..128.  The fwd / bwd entry points read DEVICE copies of both.
+ * Dropout: element (s, h, query i, key j) is numbered ((s H + h) Lpad + i) ((Lpad + 1) & ~1) + j, the index the
+ * xfm_attention_* kernels give it in the padded [n, Lpad] layout, so both draw the same mask for the same seed.
+ * The backward writes delta itself (bf16 dq / dk / dv; every row is written exactly once: no accumulation).
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct xfm_varlen_params {
+  const void *q, *k, *v;
+  void* out;
+  float* lse;
+  int64_t q_stride, k_stride, v_stride, o_stride;
+  const int32_t* cu_seqlens;
+  const int32_t* tiles;
+  int32_t n, n_tiles, H, Lpad, T;
+  float scale, dropout_p;
+  uint64_t dropout_seed;
+  /* backward */
+  const void* dout;
+  float* delta;
+  void *dq, *dk, *dv;
+  int64_t do_stride, dq_stride, dk_stride, dv_stride;
+} xfm_varlen_params;
+
+int xfm_attention_varlen_plan(const int32_t* lengths, int n, int32_t* cu_seqlens, int32_t* tiles, int32_t* n_tiles);
+int xfm_attention_varlen_fwd(const xfm_varlen_params* p, void* stream);
+int xfm_attention_varlen_bwd(const xfm_varlen_params* p, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * K6 — LayerNorm (torch layer_norm at beit2.py:201-205,458; xroberta.py:135,303,384,1328; xfm.py:118).
  * dtype codes: 0 = bf16, 1 = f32.  stats = [M,2] f32 (mean, rstd).  y2_f32: optional second f32 copy.
  * bwd: dx = LN'(dy) (+ add_in); dw/db accumulate (+=) with f32 atomics.

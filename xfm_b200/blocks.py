@@ -141,8 +141,10 @@ def _attn_out_fwd(ctx, w, pre, resid, eps, drop, s, tag):
 
 
 def roberta_layer_fwd(h, w, Bt, Lt, H, eps, kmask, enc=None, Benc=0, Lenc=0, kv_index=None, drop=NO_DROP, save=True,
-                      h32=None, kv_offsets=None, kv_samples=None, self_bias=None, enc_kmask=None, kvc=None):
+                      h32=None, kv_offsets=None, kv_samples=None, self_bias=None, enc_kmask=None, kvc=None, varlen=None):
     """h: bf16 [Bt*Lt, D] (h32: the same hidden state in f32, used as the residual when given).
+    varlen: encoders.Varlen of a packed variable-length batch (h holds its T rows; Bt, Lt and kmask are unused): the
+    self-attention runs on the packed kernels, everything else is row-wise anyway.
     enc: bf16 [Benc*Lenc, Denc] image tokens (cross-attention) or None.  Returns (h_out bf16, h_out f32, saved).
     self_bias: f32 [H, Lt, ld] additive self-attention term (the decoder's causal mask, xroberta.py:771-806);
     enc_kmask: f32 [Bt, Lenc] additive key mask of the cross-attention (xroberta.py:903-909).
@@ -153,8 +155,12 @@ def roberta_layer_fwd(h, w, Bt, Lt, H, eps, kmask, enc=None, Benc=0, Lenc=0, kv_
     scale = 1.0 / math.sqrt(64)
     qkv = L.gemm(h, w["qkv_w16"], bias=w["qkv_b"])
     seed_a = drop.next_seed() if drop.p_attn > 0 else 0
-    ctx, lse = L.attention_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], Bt, H, Lt, Lt, scale, kmask=kmask, bias=self_bias,
-                               dropout_p=drop.p_attn, dropout_seed=seed_a)
+    if varlen is not None:
+        ctx, lse = L.attention_varlen_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], varlen.cu, varlen.tiles, H, varlen.Lpad,
+                                          scale, dropout_p=drop.p_attn, dropout_seed=seed_a)
+    else:
+        ctx, lse = L.attention_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], Bt, H, Lt, Lt, scale, kmask=kmask,
+                                   bias=self_bias, dropout_p=drop.p_attn, dropout_seed=seed_a)
     h1, h1_32 = _attn_out_fwd(ctx, w, "a_", h if h32 is None else h32, eps, drop, s, "a")
     if save:
         s.h, s.qkv, s.ctx, s.lse, s.seed_a, s.h1 = h, qkv, ctx, lse, seed_a, h1
@@ -202,7 +208,7 @@ def _attn_out_bwd(dh, s, w, g, pre, tag, ctx):
 
 
 def roberta_layer_bwd(dh3, s, w, g, Bt, Lt, H, kmask, Benc=0, Lenc=0, kv_index=None, kv_offsets=None, kv_samples=None,
-                      d_enc=None, need_dh=True, self_bias=None, enc_kmask=None, dkvc_out=None):
+                      d_enc=None, need_dh=True, self_bias=None, enc_kmask=None, dkvc_out=None, varlen=None):
     """dh3: bf16 or fp32 [Bt*Lt, D].  d_enc: fp32 [Benc*Lenc, Denc] accumulator for the image-token gradient.
     dkvc_out: where this layer's K | V gradient goes when the caller back-propagates all layers' K / V projections in one
     GEMM afterwards (the per-layer d_enc GEMM is then skipped).  Returns the fp32 gradient wrt the layer input (or None)."""
@@ -237,8 +243,14 @@ def roberta_layer_bwd(dh3, s, w, g, Bt, Lt, H, kmask, Benc=0, Lenc=0, kv_index=N
     # ---- self-attention
     d_res, d_ctx = _attn_out_bwd(dh1, s, w, g, "a_", "a", s.ctx)
     dqkv = torch.empty_like(s.qkv)
-    L.attention_bwd(d_ctx, s.qkv[:, :D], s.qkv[:, D:2 * D], s.qkv[:, 2 * D:], s.ctx, s.lse, Bt, H, Lt, Lt, scale, dqkv[:, :D],
-                    dqkv[:, D:2 * D], dqkv[:, 2 * D:], kmask=kmask, bias=self_bias, dropout_p=s.p_attn, dropout_seed=s.seed_a)
+    if varlen is not None:
+        L.attention_varlen_bwd(d_ctx, s.qkv[:, :D], s.qkv[:, D:2 * D], s.qkv[:, 2 * D:], s.ctx, s.lse, varlen.cu, varlen.tiles, H,
+                               varlen.Lpad, scale, dqkv[:, :D], dqkv[:, D:2 * D], dqkv[:, 2 * D:], dropout_p=s.p_attn,
+                               dropout_seed=s.seed_a)
+    else:
+        L.attention_bwd(d_ctx, s.qkv[:, :D], s.qkv[:, D:2 * D], s.qkv[:, 2 * D:], s.ctx, s.lse, Bt, H, Lt, Lt, scale,
+                        dqkv[:, :D], dqkv[:, D:2 * D], dqkv[:, 2 * D:], kmask=kmask, bias=self_bias, dropout_p=s.p_attn,
+                        dropout_seed=s.seed_a)
     L.colsum_into(dqkv, g("qkv_b"))
     wgrad(g("qkv_w"), dqkv, s.h)
     if not need_dh:

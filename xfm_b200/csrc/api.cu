@@ -92,6 +92,11 @@ int xfm_gemm_bf16(const xfm_gemm_params* p, void* stream) { return gemm_bf16(p, 
 int xfm_attention_fwd(const xfm_attn_params* p, void* stream) { return attention_fwd(p, ST); }
 int xfm_attention_bwd(const xfm_attn_params* p, void* stream) { return attention_bwd(p, ST); }
 int xfm_attention_fwd_parts(const xfm_attn_params* p) { return attention_fwd_parts(p); }
+int xfm_attention_varlen_plan(const int32_t* lengths, int n, int32_t* cu_seqlens, int32_t* tiles, int32_t* n_tiles) {
+  return varlen_plan(lengths, n, cu_seqlens, tiles, n_tiles);
+}
+int xfm_attention_varlen_fwd(const xfm_varlen_params* p, void* stream) { return varlen_attention_fwd(p, ST); }
+int xfm_attention_varlen_bwd(const xfm_varlen_params* p, void* stream) { return varlen_attention_bwd(p, ST); }
 
 int xfm_layernorm_fwd(const void* x, int x_dtype, const float* w, const float* b, void* y, int y_dtype, float* y2_f32,
                       float* stats, int M, int D, float eps, void* stream) {

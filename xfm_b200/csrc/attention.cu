@@ -359,6 +359,14 @@ __global__ void attn_delta_kernel(const bf16* __restrict__ dout, int64_t do_stri
   }
 }
 
+int launch_attn_delta(const bf16* dout, int64_t do_stride, const bf16* out, int64_t o_stride, float* delta, int B, int H, int Lq,
+                      cudaStream_t s) {
+  if (8 * H * 4 > 1024) { set_error("attention_bwd: too many heads"); return XFM_ERR_BAD_ARG; }
+  attn_delta_kernel<<<(B * Lq + 3) / 4, dim3(8 * H, 4), 0, s>>>(dout, do_stride, out, o_stride, delta, B, H, Lq);
+  count_launch();
+  return 0;
+}
+
 // Kernel A: dQ (+ optional bf16 dS dump).  Same tiling as the forward; STREAM: K / V in chunks, as there.
 template <int WARPS, bool STREAM>
 __global__ void __launch_bounds__(WARPS * 32)
@@ -694,10 +702,8 @@ int attention_bwd(const xfm_attn_params* p, cudaStream_t s) {
   const int LkP = (a.Lk + AT_TILE - 1) / AT_TILE * AT_TILE;
   const int LqP = (a.Lq + AT_TILE - 1) / AT_TILE * AT_TILE;
   {
-    dim3 blk(8 * a.H, 4);
-    if (8 * a.H * 4 > 1024) { set_error("attention_bwd: too many heads"); return XFM_ERR_BAD_ARG; }
-    attn_delta_kernel<<<(a.B * a.Lq + 3) / 4, blk, 0, s>>>(a.dout, a.do_stride, a.out, a.o_stride, (float*)p->delta, a.B, a.H, a.Lq);
-    count_launch();
+    const int rc = launch_attn_delta(a.dout, a.do_stride, a.out, a.o_stride, (float*)p->delta, a.B, a.H, a.Lq, s);
+    if (rc) return rc;
   }
   if (p->allow_tc && vit_attention_tc_supported(p, true)) return vit_attention_bwd_tc(p, s);
   if (p->allow_tc && cross_attention_tc_supported(p, true)) return cross_attention_bwd_tc(p, s);

@@ -60,8 +60,15 @@ int cross_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s);
 bool self_attention_tc_supported(const xfm_attn_params* p);
 int self_attention_fwd_tc(const xfm_attn_params* p, cudaStream_t s);
 int self_attention_bwd_tc(const xfm_attn_params* p, cudaStream_t s);
+// Packed variable-length self-attention (attention_vtc.cu): host tile planner, forward, backward (delta kernel included).
+int varlen_plan(const int32_t* lengths, int n, int32_t* cu_seqlens, int32_t* tiles, int32_t* n_tiles);
+int varlen_attention_fwd(const xfm_varlen_params* p, cudaStream_t s);
+int varlen_attention_bwd(const xfm_varlen_params* p, cudaStream_t s);
 
 typedef __nv_bfloat16 bf16_t;
+// delta[b, h, i] = rowsum(dO o O) of the attention backward (attention.cu)
+int launch_attn_delta(const bf16_t* dout, int64_t do_stride, const bf16_t* out, int64_t o_stride, float* delta, int B, int H,
+                      int Lq, cudaStream_t s);
 int layernorm_fwd(const void* x, int x_dtype, const float* w, const float* b, void* y, int y_dtype, float* y2, float* stats,
                   int M, int D, float eps, cudaStream_t s);
 int layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* stats, const float* w,

@@ -394,11 +394,14 @@ class RobertaStack:
                             pos_pad=-1 if self.names.arch == "bert" else self.pad)   # xbert.py:172-174 vs xroberta.py:92-102
 
     def layers_fwd(self, h, Bt, Lt, kmask, enc=None, Benc=0, Lenc=0, kv_index=None, drop=BK.NO_DROP, save=True, h32=None,
-                   self_bias=None, enc_kmask=None):
-        """Returns (h bf16 [Bt*Lt, D], h f32 same shape, state).  self_bias / enc_kmask: see blocks.roberta_layer_fwd."""
+                   self_bias=None, enc_kmask=None, varlen=None):
+        """Returns (h bf16 [Bt*Lt, D], h f32 same shape, state).  self_bias / enc_kmask: see blocks.roberta_layer_fwd.
+        varlen: a Varlen batch packed into h's rows (Bt = 1, Lt = T, no kmask, no cross-attention)."""
         if self.w is None:
             self.refresh()
+        assert varlen is None or (enc is None and kmask is None and self_bias is None and Bt == 1 and Lt == varlen.T)
         st = State()
+        st.varlen = varlen
         st.layers, st.Bt, st.Lt, st.kmask, st.Benc, st.Lenc, st.kv_index = [], Bt, Lt, kmask, Benc, Lenc, kv_index
         st.kv_offsets = st.kv_samples = None
         st.self_bias, st.enc_kmask = self_bias, enc_kmask
@@ -423,7 +426,7 @@ class RobertaStack:
             h, h32, s = BK.roberta_layer_fwd(h, self.w[i], Bt, Lt, self.H, self.eps, kmask, enc=enc, Benc=Benc, Lenc=Lenc,
                                              kv_index=kv_index, drop=drop, save=save, h32=h32, kv_offsets=st.kv_offsets,
                                              kv_samples=st.kv_samples, self_bias=self_bias, enc_kmask=enc_kmask,
-                                             kvc=st.kvc_all[:, i * D2:(i + 1) * D2] if merged else None)
+                                             kvc=st.kvc_all[:, i * D2:(i + 1) * D2] if merged else None, varlen=varlen)
             st.layers.append(s)
             if self.collect is not None:
                 self.collect.append(h32.view(Bt, Lt, -1).clone())
@@ -469,12 +472,24 @@ class RobertaStack:
                                       Lenc=st.Lenc, kv_index=st.kv_index, kv_offsets=kv_offsets, kv_samples=kv_samples,
                                       d_enc=d_enc, need_dh=(need_dh or not last), self_bias=st.self_bias,
                                       enc_kmask=st.enc_kmask,
-                                      dkvc_out=dkvc_all[:, i * D2:(i + 1) * D2] if dkvc_all is not None else None)
+                                      dkvc_out=dkvc_all[:, i * D2:(i + 1) * D2] if dkvc_all is not None else None,
+                                      varlen=getattr(st, "varlen", None))
             st.layers[i] = None
         if dkvc_all is not None and d_enc is not None:   # gradient wrt the image tokens: all layers in one long-K GEMM
             L.gemm(dkvc_all, st.kv_wall, b_t=True, out=d_enc, accumulate=not d_enc_fresh)
         st.kvc_all = st.kv_wall = None
         return dh
+
+
+class Varlen:
+    """A packed variable-length batch: n sequences of 1..128 tokens back to back in T rows.  cu / tiles: int32 device copies
+    of lib.varlen_plan (row offsets, tiles of the packed attention kernels); Lpad: the padded length the batch arrived in,
+    which numbers the attention dropout mask as in the padded layout."""
+
+    def __init__(self, lengths, Lpad, device):
+        cu, tiles = L.varlen_plan(lengths)
+        self.n, self.T, self.Lpad = cu.numel() - 1, int(cu[-1]), int(Lpad)
+        self.cu, self.tiles = cu.to(device, non_blocking=True), tiles.to(device, non_blocking=True)
 
 
 MERGE_CROSS_KV = __import__("os").environ.get("XFM_MERGE_CROSS_KV", "1") != "0"   # A/B switch for measurements

@@ -282,6 +282,78 @@ def attention_bwd(dout, q, k, v, out, lse, B, H, Lq, Lk, scale, dq, dk, dv, *, B
     check(lib().xfm_attention_bwd(C.byref(p), stream_ptr()), "xfm_attention_bwd")
 
 
+class VarlenParams(C.Structure):
+    _fields_ = [
+        ("q", C.c_void_p), ("k", C.c_void_p), ("v", C.c_void_p), ("out", C.c_void_p), ("lse", C.c_void_p),
+        ("q_stride", C.c_int64), ("k_stride", C.c_int64), ("v_stride", C.c_int64), ("o_stride", C.c_int64),
+        ("cu_seqlens", C.c_void_p), ("tiles", C.c_void_p),
+        ("n", C.c_int32), ("n_tiles", C.c_int32), ("H", C.c_int32), ("Lpad", C.c_int32), ("T", C.c_int32),
+        ("scale", C.c_float), ("dropout_p", C.c_float), ("dropout_seed", C.c_uint64),
+        ("dout", C.c_void_p), ("delta", C.c_void_p),
+        ("dq", C.c_void_p), ("dk", C.c_void_p), ("dv", C.c_void_p),
+        ("do_stride", C.c_int64), ("dq_stride", C.c_int64), ("dk_stride", C.c_int64), ("dv_stride", C.c_int64),
+    ]
+
+
+def varlen_plan(lengths):
+    """Sequence lengths (1..128 each) -> (cu_seqlens int32 [n+1], tiles int32 [n_tiles+1]) on the host: the packed row
+    offsets and the tiles of xfm_attention_varlen_plan (first sequence of every tile, then n).  Needs no device."""
+    ln = torch.as_tensor(lengths, dtype=torch.int32).reshape(-1).contiguous()
+    n = ln.numel()
+    cu = torch.empty(n + 1, dtype=torch.int32)
+    tiles = torch.empty(n + 1, dtype=torch.int32)
+    nt = C.c_int32(0)
+    check(load().xfm_attention_varlen_plan(C.c_void_p(ln.data_ptr()), n, C.c_void_p(cu.data_ptr()),
+                                           C.c_void_p(tiles.data_ptr()), C.byref(nt)), "xfm_attention_varlen_plan")
+    return cu, tiles[:nt.value + 1].clone()
+
+
+def _varlen_common(p, q, k, v, cu_seqlens, tiles, H, Lpad, scale, dropout_p, dropout_seed):
+    for t in (q, k, v):
+        assert t.dtype == torch.bfloat16 and t.dim() == 2 and t.stride(1) == 1 and t.shape[1] == H * 64
+    assert q.shape[0] == k.shape[0] == v.shape[0]
+    for t in (cu_seqlens, tiles):
+        assert t.dtype == torch.int32 and t.is_contiguous() and t.device == q.device
+    p.q, p.k, p.v = q.data_ptr(), k.data_ptr(), v.data_ptr()
+    p.q_stride, p.k_stride, p.v_stride = q.stride(0), k.stride(0), v.stride(0)
+    p.cu_seqlens, p.tiles = cu_seqlens.data_ptr(), tiles.data_ptr()
+    p.n, p.n_tiles, p.H, p.Lpad, p.T = cu_seqlens.numel() - 1, tiles.numel() - 1, H, Lpad, q.shape[0]
+    p.scale, p.dropout_p, p.dropout_seed = scale, dropout_p, dropout_seed
+
+
+def attention_varlen_fwd(q, k, v, cu_seqlens, tiles, H, Lpad, scale, *, dropout_p=0.0, dropout_seed=0, out=None):
+    """Packed variable-length self-attention.  q, k, v: bf16 [T, H*64] views (row strides allowed); cu_seqlens / tiles:
+    int32 device copies of varlen_plan's output; Lpad: the padded length the batch arrived in (numbers the dropout mask as
+    the padded layout does).  Returns (out bf16 [T, H*64], lse f32 [H, T])."""
+    T = q.shape[0]
+    if out is None:
+        out = torch.empty((T, H * 64), dtype=torch.bfloat16, device=q.device)
+    lse = torch.empty((H, T), dtype=torch.float32, device=q.device)
+    p = VarlenParams()
+    _varlen_common(p, q, k, v, cu_seqlens, tiles, H, Lpad, scale, dropout_p, dropout_seed)
+    assert out.shape == (T, H * 64) and out.stride(1) == 1
+    p.out, p.o_stride, p.lse = out.data_ptr(), out.stride(0), lse.data_ptr()
+    check(lib().xfm_attention_varlen_fwd(C.byref(p), stream_ptr()), "xfm_attention_varlen_fwd")
+    return out, lse
+
+
+def attention_varlen_bwd(dout, q, k, v, out, lse, cu_seqlens, tiles, H, Lpad, scale, dq, dk, dv, *, dropout_p=0.0,
+                         dropout_seed=0):
+    """Writes bf16 dq / dk / dv [T, H*64] (views with row strides) of attention_varlen_fwd."""
+    p = VarlenParams()
+    _varlen_common(p, q, k, v, cu_seqlens, tiles, H, Lpad, scale, dropout_p, dropout_seed)
+    T = q.shape[0]
+    assert lse.shape == (H, T) and lse.dtype == torch.float32 and lse.is_contiguous()
+    delta = torch.empty((H, T), dtype=torch.float32, device=q.device)
+    for t in (dout, out, dq, dk, dv):
+        assert t.dtype == torch.bfloat16 and t.stride(1) == 1 and t.shape == (T, H * 64)
+    p.out, p.o_stride, p.lse = out.data_ptr(), out.stride(0), lse.data_ptr()
+    p.dout, p.do_stride, p.delta = dout.data_ptr(), dout.stride(0), delta.data_ptr()
+    p.dq, p.dk, p.dv = dq.data_ptr(), dk.data_ptr(), dv.data_ptr()
+    p.dq_stride, p.dk_stride, p.dv_stride = dq.stride(0), dk.stride(0), dv.stride(0)
+    check(lib().xfm_attention_varlen_bwd(C.byref(p), stream_ptr()), "xfm_attention_varlen_bwd")
+
+
 def vit_attention_bwd_tc_ok(n_tokens):
     """Token counts the fused tcgen05 backward handles: the forward's plus 577 (384 px) and 901 (480 px), processed in key
     blocks of about 192 keys (three and five)."""
